@@ -14,14 +14,15 @@ the headline (C4 greedy: `value` device-resident, `e2e` through host buffers), i
 `gpu_library_baseline`, a `vp` block at N>1 (the 1 M-item catalog sharded vocab-parallel, strong scaling) and, at
 N=1, an `also` array with the sampled / C2 / C1 / training sub-results.  See DESIGN.md "Measurement".
 
-Timing: the K steps form one PASS (per-step CUDA-event pairs, L2 flushed between steps, summed); the pass is
-replayed `reps` times so that the timed window is >= --window seconds, each pass bracketed by barrier +
-synchronize, max over ranks per pass, and the MEDIAN pass is reported.
+Timing: after W warm-up steps, exactly K timed steps (per-step CUDA-event pairs, L2 flushed between steps, summed),
+bracketed by barrier + synchronize, max over ranks.  K defaults to the workload's `steps`, about 0.5 s of timed work.
+
+--dump-outputs DIR writes what the timed path returned in its last timed step as DIR/<name>.npy (float32 / float64).
+Weights, inputs and noise seeds are fixed, so two builds run with the same arguments can be compared output for output.
 """
 import argparse
 import gc
 import json
-import math
 import os
 import subprocess
 import sys
@@ -36,18 +37,22 @@ if ROOT not in sys.path:
     sys.path.insert(0, ROOT)
 
 WORKLOADS = {
-    "c1": dict(n_items=3707, n_users=6041, L=5, D=8, Z=16, H=256, PH=128, no_user=False, B=64,
+    "c1": dict(n_items=3707, n_users=6041, L=5, D=8, Z=16, H=256, PH=128, no_user=False, B=64, steps=4500,
                desc="C1 ML-1M shape: 3707 items, 6041 users, slate 5, dim 8, with user, B=64"),
-    "c2": dict(n_items=50000, n_users=1, L=10, D=8, Z=16, H=256, PH=128, no_user=True, B=1024,
+    "c2": dict(n_items=50000, n_users=1, L=10, D=8, Z=16, H=256, PH=128, no_user=True, B=1024, steps=3500,
                desc="C2 Yoochoose shape: 50k items, slate 10, dim 8, nouser, B=1024"),
-    "c3": dict(n_items=100000, n_users=6041, L=5, D=8, Z=16, H=256, PH=128, no_user=False, B=4096,
+    "c3": dict(n_items=100000, n_users=6041, L=5, D=8, Z=16, H=256, PH=128, no_user=False, B=4096, steps=400,
                desc="C3: PivotCVAE gt training, fused full-catalog soft-max CE + KL, 100k items, slate 5, dim 8, B=4096"),
-    "c4": dict(n_items=1000000, n_users=6041, L=5, D=8, Z=16, H=256, PH=128, no_user=False, B=4096,
+    "c4": dict(n_items=1000000, n_users=6041, L=5, D=8, Z=16, H=256, PH=128, no_user=False, B=4096, steps=400,
                desc="C4: 1M items, slate 5, dim 8, with user, B=4096, PivotCVAE + response MLP"),
-    "c5": dict(n_items=10000000, n_users=1024, L=5, D=8, Z=16, H=256, PH=128, no_user=False, B=65536, samples_per_user=64,
+    "c5": dict(n_items=10000000, n_users=1024, L=5, D=8, Z=16, H=256, PH=128, no_user=False, B=65536, samples_per_user=64, steps=4,
                desc="C5 variation-control sweep: 10M items, slate 5, dim 8, 1024 users x 64 sampled slates = 65536 rows "
                     "(gt_spi: sampled pivot + fresh z per sample), coverage + ILS of the result"),
 }
+# steps: the default --steps of a workload, about 0.5 s of timed steps on one B200 (C4: 1.55 ms per step, C2: 0.13-0.17 ms,
+# C1: 0.12 ms, C3 training: 1.3 ms, C5: 176 ms); the `also` sub-results of the default run time half of that.
+# The CPU reference arm (--impl reference) defaults to REFERENCE_STEPS: at C4 one of its steps takes about 0.5 s.
+REFERENCE_STEPS = 20
 MODEL_OF_MODE = {"greedy": "PivotCVAE gt_pi", "sampled": "PivotCVAE gt_spi (sampled pivot)", "list": "ListCVAE", "train": "PivotCVAE gt"}
 
 
@@ -243,29 +248,46 @@ class Dist:
             self.started = False
 
 
-def timed_passes(D, step, K, W, window_s, flush, max_reps=400):
-    """W warm-up steps, then `reps` passes of exactly K steps; step(i) runs step i of a pass on the current
-    stream.  Per-step CUDA-event pairs (L2 flushed outside the pairs) are summed per pass; every pass is
-    bracketed by barrier + synchronize; per pass the MAX over ranks is taken.  -> (median pass ms, reps, all passes)."""
+def timed_steps(D, step, K, W, flush):
+    """W warm-up steps, then exactly K timed steps; step(i) runs step i on the current stream.  Per-step CUDA-event
+    pairs (L2 flushed outside the pairs) are summed; the K steps are bracketed by barrier + synchronize and the MAX
+    over ranks is taken.  -> ms of the K steps."""
     for i in range(W):
         step(i % K)
     D.barrier()
     ev = [(torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)) for _ in range(K)]
+    for i in range(K):
+        flush.zero_()
+        ev[i][0].record()
+        step(i)
+        ev[i][1].record()
+    D.barrier()
+    return D.max_([sum(a.elapsed_time(b) for a, b in ev)])[0]
 
-    def one_pass():
-        D.barrier()
-        for i in range(K):
-            flush.zero_()
-            ev[i][0].record()
-            step(i)
-            ev[i][1].record()
-        D.barrier()
-        return D.max_([sum(a.elapsed_time(b) for a, b in ev)])[0]
 
-    first = one_pass()
-    reps = int(min(max_reps, max(3, math.ceil(window_s * 1e3 / max(first, 1e-3)))))
-    passes = [first] + [one_pass() for _ in range(reps - 1)]
-    return float(np.median(passes)), reps, passes
+DUMP_LIMIT = 64 * 10 ** 6      # bytes of all files written by dump_outputs
+NPY_HEADER = 256               # bytes allowed per .npy header (numpy writes 128 for these shapes)
+
+
+def dump_outputs(path, arrays):
+    """Write {name: tensor} as path/<name>.npy: floats of 32 bits or fewer as float32, everything else (item ids,
+    float64) as float64.  When the files would exceed DUMP_LIMIT bytes in all, every array keeps the same fraction of
+    its rows, a sorted sample drawn with a fixed seed, and the kept row indices go to <name>.rows.npy."""
+    os.makedirs(path, exist_ok=True)
+    out = {}
+    for k, v in arrays.items():
+        a = v.detach().cpu().numpy()
+        out[k] = a.astype(np.float32 if a.dtype.kind == "f" and a.itemsize <= 4 else np.float64)
+    budget = DUMP_LIMIT - 2 * NPY_HEADER * len(out)      # an array and its row indices: two files, two headers
+    total = sum(a.nbytes + 8 * len(a) for a in out.values() if a.ndim)
+    fixed = sum(a.nbytes for a in out.values() if not a.ndim)
+    for k, a in out.items():
+        if a.ndim and total + fixed > budget:
+            keep = int(len(a) * (budget - fixed) / total)
+            rows = np.sort(np.random.default_rng(0).choice(len(a), keep, replace=False))
+            np.save(os.path.join(path, k + ".rows.npy"), rows.astype(np.float64))
+            a = a[rows]
+        np.save(os.path.join(path, k + ".npy"), a)
 
 
 # ------------------------------------------------------------------ CPU arms
@@ -393,13 +415,15 @@ def parity_check(w, sd, env_sd, mode, model, env, device):
 
 
 # ------------------------------------------------------------------ generation measurement
-def measure_generate(D, args, wname, mode, window_s, vp=False, full=True, cpu_seconds=0.0):
-    """One (workload, mode) measurement -> dict with value / e2e / roofline (/ cpu_baseline when cpu_seconds > 0)."""
+def measure_generate(D, args, wname, mode, vp=False, full=True, cpu_seconds=0.0, dump=None, steps=None):
+    """One (workload, mode) measurement -> dict with value / e2e / roofline (/ cpu_baseline when cpu_seconds > 0).
+    dump: directory for rank 0's slates, z_mu and response scores of the last timed step.  steps: timed steps
+    (default --steps)."""
     from pivotcvae_b200 import ops
     from pivotcvae_b200.graphs import GraphedSlateGenerator
     w = WORKLOADS[wname]
     device, world, rank = D.device, D.world, D.rank
-    B, K, W = (args.batch or w["B"]), args.steps, args.warmup
+    B, K, W = (args.batch or w["B"]), (steps or args.steps), args.warmup
     sd, env_sd = make_weights(w, "list" if mode == "list" else "pivot")
     model, env = build_gpu(w, sd, env_sd, mode, device)
     model.noise.reseed(1234 + (0 if vp else rank))   # vocab-parallel ranks replicate inputs AND noise
@@ -433,21 +457,23 @@ def measure_generate(D, args, wname, mode, window_s, vp=False, full=True, cpu_se
     # lives on the device, so every replay draws fresh noise.  Vocab-parallel: the NCCL all-reduces are captured too.
     gen = GraphedSlateGenerator(model, env, B, warmup=3)
 
-    ms, reps, passes = timed_passes(D, lambda i: gen(ctx_d[i], usr_d[i]), K, W, window_s, flush)
+    ms = timed_steps(D, lambda i: gen(ctx_d[i], usr_d[i]), K, W, flush)
+    if dump and rank == 0:
+        dump_outputs(dump, {"items": gen.items, "z_mu": gen.z_mu, "resp": gen.resp})
 
     def e2e_step(i):
         items, resp = gen(ctx_h[i], usr_h[i])      # pinned host -> static device buffers
         items_h.copy_(items, non_blocking=True)
         resp_h.copy_(resp, non_blocking=True)
-    ms_e2e, reps_e2e, _ = timed_passes(D, e2e_step, K, min(W, 3), window_s, flush)
+    ms_e2e = timed_steps(D, e2e_step, K, min(W, 3), flush)
 
     total = B * (1 if vp else world) * K      # vocab-parallel: all ranks work on the SAME batch (strong scaling)
     out = {"workload": wname, "mode": mode, "model": MODEL_OF_MODE[mode], "metric": "generated slates/sec (%s)" % mode,
-           "value": total / (ms / 1e3), "unit": "slates/s", "ms_per_step": ms / K, "batch_per_gpu": B, "reps": reps,
-           "timed_region_s": sum(passes) / 1e3,
+           "value": total / (ms / 1e3), "unit": "slates/s", "ms_per_step": ms / K, "batch_per_gpu": B, "steps": K,
+           "timed_region_s": ms / 1e3,
            "e2e": {"value": total / (ms_e2e / 1e3), "unit": "slates/s", "h2d_bytes_per_step": int(B * w["L"] * 4 + B * 8),
-                   "d2h_bytes_per_step": int(B * w["L"] * 8 + B * w["L"] * 4), "ms_per_step": ms_e2e / K, "reps": reps_e2e},
-           "launches_per_step": gen.launches_per_step, "gpu_launches": int(gen.launches_per_step * K * reps)}
+                   "d2h_bytes_per_step": int(B * w["L"] * 8 + B * w["L"] * 4), "ms_per_step": ms_e2e / K},
+           "launches_per_step": gen.launches_per_step, "gpu_launches": int(gen.launches_per_step * K)}
     if parity is not None:
         out["parity_check"] = parity
         out["parity_detail"] = parity_detail
@@ -553,14 +579,16 @@ def traffic_of(wname, M, N):
 
 
 # ------------------------------------------------------------------ training measurement
-def measure_train(D, args, wname, n_neg_arg, ce_engine, window_s, cpu_seconds=0.0):
-    """train samples/sec: get_gen_loss (prior + encoder + decoder + fused catalog CE + KL) -> backward -> Adam.step."""
+def measure_train(D, args, wname, n_neg_arg, ce_engine, cpu_seconds=0.0, dump=None, steps=None):
+    """train samples/sec: get_gen_loss (prior + encoder + decoder + fused catalog CE + KL) -> backward -> Adam.step.
+    dump: directory for rank 0's loss, recLoss, KLD and trained parameters after the last timed step.  steps: timed
+    steps (default --steps)."""
     import torch.distributed as dist
     from pivotcvae_b200 import ops
     from pivotcvae_b200.train_generative import get_gen_loss
     w = WORKLOADS[wname]
     device, world, rank = D.device, D.world, D.rank
-    B, K, W = (args.batch or w["B"]), args.steps, args.warmup
+    B, K, W = (args.batch or w["B"]), (steps or args.steps), args.warmup
     sd, env_sd = make_weights(w, "pivot")
     model, _ = build_gpu(w, sd, env_sd, "greedy", device)
     model.noise.reseed(99 + rank)
@@ -595,26 +623,36 @@ def measure_train(D, args, wname, n_neg_arg, ce_engine, window_s, cpu_seconds=0.
                     p.grad.copy_(flat[o:o + n].view_as(p.grad))
                     o += n
         opt.step()
-        return loss
+        return loss, rec, kld
 
     graphed = None
     if world == 1:     # single GPU: the whole step is one CUDA graph (the DP arm keeps the eager NCCL all-reduce)
         from pivotcvae_b200.graphs import GraphedTrainStep
         graphed = GraphedTrainStep(model, opt, B, 0.001, n_neg)
-        run = lambda b: graphed(b)[0]
+        run = graphed
     else:
         run = eager_step
-    l0 = ops.launch_count()
-    ms, reps, passes = timed_passes(D, lambda i: run(dev_batches[i]), K, W, window_s, flush)
-    launches = graphed.launches_per_step * K * reps if graphed else ops.launch_count() - l0
+    last, step_launches = {}, []
+
+    def step(i):
+        l0 = ops.launch_count()
+        last["out"] = run(dev_batches[i])
+        step_launches.append(ops.launch_count() - l0)
+    ms = timed_steps(D, step, K, W, flush)
+    # a graph replay launches no kernel from the host: its count is the one taken at capture
+    launches = graphed.launches_per_step * K if graphed else sum(step_launches[-K:])
+    if dump and rank == 0:
+        loss, rec, kld = last.pop("out")
+        dump_outputs(dump, dict({"loss": loss, "rec_loss": rec, "kld": kld},
+                                **{"param." + k: v for k, v in model.named_parameters() if v.requires_grad}))
 
     def e2e_step(i):
         if graphed:
-            loss = run(pin_batches[i])
+            loss = run(pin_batches[i])[0]
         else:
-            loss = run({k: v.to(device, non_blocking=True) for k, v in pin_batches[i].items()})
+            loss = run({k: v.to(device, non_blocking=True) for k, v in pin_batches[i].items()})[0]
         loss_h.copy_(loss.detach(), non_blocking=True)
-    ms_e2e, reps_e2e, _ = timed_passes(D, e2e_step, K, min(W, 3), window_s, flush)
+    ms_e2e = timed_steps(D, e2e_step, K, min(W, 3), flush)
 
     # per-kernel CUDA-event timing of the same step launched eagerly (roofline of the dominant kernel)
     with ops.KernelTimer() as kt:
@@ -637,7 +675,7 @@ def measure_train(D, args, wname, n_neg_arg, ce_engine, window_s, cpu_seconds=0.
     ach = flops / (dom["ms_avg"] * 1e-3) / 1e12
     out = {"workload": wname, "mode": "train", "model": MODEL_OF_MODE["train"],
            "metric": "train samples/sec (PivotCVAE gt, fused catalog CE + KL, fwd+bwd+Adam)", "value": total / (ms / 1e3),
-           "unit": "samples/s", "ms_per_step": ms / K, "batch_per_gpu": B, "reps": reps, "timed_region_s": sum(passes) / 1e3,
+           "unit": "samples/s", "ms_per_step": ms / K, "batch_per_gpu": B, "steps": K, "timed_region_s": ms / 1e3,
            "dtype": ("tf32 operands (logits, MLP gradient GEMMs), f32 accumulate" if tf32 else "f32"),
            "n_neg": n_neg, "beta": 0.001, "ce_engine": ce_engine,
            "e2e": {"value": total / (ms_e2e / 1e3), "unit": "samples/s",
@@ -737,19 +775,19 @@ def run_ours(args, w):
         clocks.start()
     is_default = not args.no_also and args.mode == "greedy" and args.workload == "c4" and not args.batch
     if args.mode == "train":
-        main = measure_train(D, args, args.workload, args.n_neg, args.ce_engine, args.window,
-                             cpu_seconds=0 if args.no_cpu else 8.0)
+        main = measure_train(D, args, args.workload, args.n_neg, args.ce_engine,
+                             cpu_seconds=0 if args.no_cpu else 8.0, dump=args.dump_outputs)
         wsd = None
     else:
-        main, wsd = measure_generate(D, args, args.workload, args.mode, args.window, vp=(args.parallel == "vp" and D.world > 1),
-                                     cpu_seconds=0 if (args.no_cpu or D.world > 1) else 12.0)
+        main, wsd = measure_generate(D, args, args.workload, args.mode, vp=(args.parallel == "vp" and D.world > 1),
+                                     cpu_seconds=0 if (args.no_cpu or D.world > 1) else 12.0, dump=args.dump_outputs)
     clk = clocks.stop() if D.rank == 0 else None
     extra = {}
     if args.mode != "train" and args.parallel != "vp":
         if D.world > 1 and not args.no_vp:
             # the 1 M-item catalog sharded vocab-parallel over the same N GPUs (strong scaling on ONE batch)
-            vpres, _ = measure_generate(D, args, args.workload, args.mode, args.window / 2, vp=True, full=False)
-            extra["vp"] = {k: vpres[k] for k in ("value", "unit", "ms_per_step", "batch_per_gpu", "reps", "e2e", "slates_equal_1gpu",
+            vpres, _ = measure_generate(D, args, args.workload, args.mode, vp=True, full=False)
+            extra["vp"] = {k: vpres[k] for k in ("value", "unit", "ms_per_step", "batch_per_gpu", "e2e", "slates_equal_1gpu",
                                                  "scaling", "parallelism", "launches_per_step") if k in vpres}
             if "roofline" in vpres:
                 extra["vp"]["per_call_ms"] = vpres["roofline"]["per_call_ms"]
@@ -759,7 +797,7 @@ def run_ours(args, w):
             also = []
             for wn, md in ALSO_GENERATE:
                 try:
-                    r, s = measure_generate(D, args, wn, md, 0.25, cpu_seconds=0 if args.no_cpu else 4.0)
+                    r, s = measure_generate(D, args, wn, md, cpu_seconds=0 if args.no_cpu else 4.0, steps=WORKLOADS[wn]["steps"] // 2)
                     r["config"] = {"workload": WORKLOADS[wn]["desc"], "batch": WORKLOADS[wn]["B"], "mode": md, "model": MODEL_OF_MODE[md]}
                     if (wn, md) == ("c2", "greedy") and not args.no_cpu:
                         r["gpu_library_baseline"] = gpu_library_baseline(s[0], s[1], s[2], md, D.device, 2.0)
@@ -768,7 +806,7 @@ def run_ours(args, w):
                     also.append({"workload": wn, "mode": md, "error": "%s: %s" % (type(e).__name__, str(e)[:300])})
             for wn, nn, eng in ALSO_TRAIN:
                 try:
-                    r = measure_train(D, args, wn, nn, eng, 0.25, cpu_seconds=0 if args.no_cpu else 4.0)
+                    r = measure_train(D, args, wn, nn, eng, cpu_seconds=0 if args.no_cpu else 4.0, steps=WORKLOADS[wn]["steps"] // 2)
                     r["config"] = {"workload": WORKLOADS[wn]["desc"], "batch": WORKLOADS[wn]["B"], "mode": "train", "n_neg": r["n_neg"]}
                     also.append(r)
                 except Exception as e:     # noqa: BLE001
@@ -779,9 +817,9 @@ def run_ours(args, w):
             saved_engine = args.mlp_engine
             try:
                 args.mlp_engine = other
-                r, _ = measure_generate(D, args, args.workload, args.mode, 0.25, cpu_seconds=0)
+                r, _ = measure_generate(D, args, args.workload, args.mode, cpu_seconds=0, steps=w["steps"] // 2)
                 also.append({"workload": args.workload, "mode": args.mode, "mlp_engine": other, "value": r["value"], "unit": r["unit"],
-                             "ms_per_step": r["ms_per_step"], "parity_check": r.get("parity_check"),
+                             "ms_per_step": r["ms_per_step"], "steps": r["steps"], "parity_check": r.get("parity_check"),
                              "parity_detail": r.get("parity_detail"), "per_call_ms": r.get("roofline", {}).get("per_call_ms")})
             except Exception as e:     # noqa: BLE001
                 also.append({"workload": args.workload, "mode": args.mode, "mlp_engine": other, "error": "%s: %s" % (type(e).__name__, str(e)[:300])})
@@ -799,11 +837,11 @@ def run_ours(args, w):
                                    "auto": "tcgen05 3xTF32 (csrc/mlp_tc.cu) for batches >= 2048 rows, FFMA chain below"}[args.mlp_engine])
                                  if args.mode != "train" else "training engine (saves activations)",
                    "l2": "flushed between steps (256 MiB write, outside the event pairs)",
-                   "timing": "per-step CUDA-event pairs summed over the K steps of a pass; %d passes (window >= %.2f s), max over "
-                             "ranks per pass, median pass reported" % (main["reps"], args.window),
+                   "timing": "per-step CUDA-event pairs summed over the %d timed steps after %d warm-up steps, max over ranks"
+                             % (args.steps, args.warmup),
                    "launch": "one CUDA graph replay per step (%s kernels of libpcv_b200)" % main.get("launches_per_step")})
     line = {"metric": main["metric"], "value": main["value"], "unit": main["unit"], "n_gpus": D.world, "steps": args.steps,
-            "warmup": args.warmup, "ms_per_step": main["ms_per_step"], "reps": main["reps"], "timed_region_s": main["timed_region_s"],
+            "warmup": args.warmup, "ms_per_step": main["ms_per_step"], "timed_region_s": main["timed_region_s"],
             "higher_is_better": True, "scaling": "strong" if vp_main else "weak", "vs_baseline": None,
             "dtype": main.get("dtype", "f32"), "data": "synthetic", "config": config, "e2e": main["e2e"],
             "gpu_launches": main["gpu_launches"], "roofline": main.get("roofline"), "cpu_baseline": main.get("cpu_baseline"),
@@ -818,7 +856,8 @@ def run_ours(args, w):
 def main():
     ap = argparse.ArgumentParser()
     ap.add_argument("--gpus", type=int, default=1)
-    ap.add_argument("--steps", type=int, default=20)
+    ap.add_argument("--steps", type=int, default=None,
+                    help="timed steps (default: the workload's, about 0.5 s on one B200; --impl reference: %d)" % REFERENCE_STEPS)
     ap.add_argument("--warmup", type=int, default=5)
     ap.add_argument("--impl", default="ours", choices=["ours", "reference"])
     ap.add_argument("--workload", default="c4", choices=sorted(WORKLOADS))
@@ -833,17 +872,25 @@ def main():
                          "auto = tc for batches of >= 2048 rows")
     ap.add_argument("--batch", type=int, default=0)
     ap.add_argument("--parallel", default="dp", choices=["dp", "vp"], help="N>1 headline: batch data-parallel (default) or vocab-parallel")
-    ap.add_argument("--window", type=float, default=0.6, help="minimum timed window in seconds (the K-step pass is repeated)")
     ap.add_argument("--no-cpu", action="store_true", help="skip the CPU / GPU-library baselines")
     ap.add_argument("--no-also", action="store_true", help="skip the sub-results of the default run")
     ap.add_argument("--no-vp", action="store_true", help="N>1: skip the vocab-parallel block")
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="write the slates, z_mu and response scores (train: loss terms and parameters) of the last timed step "
+                         "of the headline measurement as DIR/<name>.npy")
     args = ap.parse_args()
+    if args.steps is not None and args.steps < 1:
+        ap.error("--steps must be >= 1")
+    if args.dump_outputs and args.impl != "ours":
+        ap.error("--dump-outputs applies to --impl ours")
     args.warmup = max(args.warmup, 3) if args.impl == "ours" else args.warmup
     w = WORKLOADS[args.workload]
     if args.workload == "c5" and args.mode == "greedy":
         args.mode = "sampled"      # C5 is the sampled-slates sweep
     if args.workload == "c3" and args.mode != "train":
         args.mode = "train"
+    if args.steps is None:
+        args.steps = REFERENCE_STEPS if args.impl == "reference" else w["steps"]
     if args.impl == "reference":
         run_reference(args, w)
     else:

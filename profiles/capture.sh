@@ -9,7 +9,7 @@ OUT=gpurun_out
 mkdir -p $OUT
 python profiles/probe_kernels.py > $OUT/${TAG}_probe.txt 2>&1
 ncu --metrics gpu__time_duration.sum --clock-control none --cache-control none -c 600 --csv \
-    --log-file $OUT/${TAG}_launches_c4.csv python bench.py --steps 3 --warmup 3 --window 0.01 --no-cpu --no-also \
+    --log-file $OUT/${TAG}_launches_c4.csv python bench.py --steps 3 --warmup 3 --no-cpu --no-also \
     > $OUT/${TAG}_bench_under_ncu.log 2>&1
 KERNELS='score_select_tc_kernel|tc_refine_kernel|mlp_cluster_kernel|mlp_tc_kernel|sigmoid_categorical|urm_kernel|slate_metrics_kernel|ce_tc2_kernel|ce_sparse_kernel|cand_ce_kernel|ce_kernel|score_select_kernel|gemm_tn_tc_kernel|topk_kernel'
 PROBE_WARM=0 PROBE_ITERS=1 ncu --set full --clock-control none -k "regex:$KERNELS" -o $OUT/${TAG}_kernels -f \
@@ -18,7 +18,7 @@ ncu -i $OUT/${TAG}_kernels.ncu-rep --page raw --csv > $OUT/${TAG}_kernels_raw.cs
 ls -la $OUT/${TAG}_kernels.ncu-rep; [ $(stat -c %s $OUT/${TAG}_kernels.ncu-rep) -gt 40000000 ] && rm -f $OUT/${TAG}_kernels.ncu-rep
 # launch list of the C3 training step (own backward GEMMs, tensor-core CE)
 ncu --metrics gpu__time_duration.sum --clock-control none --cache-control none -c 1500 --csv \
-    --log-file $OUT/${TAG}_launches_c3_train.csv python bench.py --workload c3 --mode train --steps 3 --warmup 3 --window 0.01 \
+    --log-file $OUT/${TAG}_launches_c3_train.csv python bench.py --workload c3 --mode train --steps 3 --warmup 3 \
     --no-cpu --no-also > /dev/null 2>&1
 # tensor-pipe evidence of the generalised filter: D = 128 at the C4 shape
 PROBE_WARM=1 PROBE_ITERS=1 ncu --set full --clock-control none -k "regex:score_select_tc_kernel" -s 1 -c 1 \

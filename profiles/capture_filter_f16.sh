@@ -13,7 +13,7 @@ PROBE_WARM=0 PROBE_ITERS=1 ncu --set full --clock-control none -k "regex:score_s
 ncu -i $OUT/${TAG}_filter.ncu-rep --page raw --csv > $OUT/${TAG}_filter_raw.csv 2>/dev/null
 ls -la $OUT/${TAG}_filter.ncu-rep
 ncu --metrics gpu__time_duration.sum --clock-control none --cache-control none -c 600 --csv \
-    --log-file $OUT/${TAG}_launches_c4.csv python bench.py --steps 3 --warmup 3 --window 0.01 --no-cpu --no-also \
+    --log-file $OUT/${TAG}_launches_c4.csv python bench.py --steps 3 --warmup 3 --no-cpu --no-also \
     > $OUT/${TAG}_bench_under_ncu.log 2>&1
 timeout 600 compute-sanitizer --tool memcheck --error-exitcode 1 python -m pytest tests/test_gpu_tcgen05.py \
     -x -q -m gpu -k "not full_size and not max_size" > $OUT/${TAG}_memcheck.txt 2>&1

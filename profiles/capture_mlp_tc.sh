@@ -10,7 +10,7 @@ mkdir -p $OUT
 python profiles/probe_kernels.py mlp_engines mlp_tc > $OUT/${TAG}_probe_mlp.txt 2>&1
 python profiles/probe_tc_accum.py > $OUT/${TAG}_tc_accum.txt 2>&1
 ncu --metrics gpu__time_duration.sum --clock-control none --cache-control none -c 600 --csv \
-    --log-file $OUT/${TAG}_launches_c4.csv python bench.py --steps 3 --warmup 3 --window 0.01 --no-cpu --no-also \
+    --log-file $OUT/${TAG}_launches_c4.csv python bench.py --steps 3 --warmup 3 --no-cpu --no-also \
     > $OUT/${TAG}_bench_under_ncu.log 2>&1
 PROBE_WARM=1 PROBE_ITERS=1 ncu --set full --clock-control none --import-source on -k "regex:mlp_tc_kernel" -s 3 -c 3 \
     -o $OUT/${TAG}_mlp_tc -f python profiles/probe_kernels.py mlp_tc > $OUT/${TAG}_probe_under_ncu.txt 2>&1

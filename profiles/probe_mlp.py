@@ -1,5 +1,5 @@
-import sys, torch
-sys.path.insert(0, "/root/repo")
+import os, sys, torch
+sys.path.insert(0, os.path.dirname(os.path.dirname(os.path.abspath(__file__))))
 from pivotcvae_b200 import ops
 B=1024
 g=torch.Generator(device="cuda").manual_seed(0)

@@ -8,8 +8,8 @@ Tables, MLP weights, the Exp(1) race noise and the Bernoulli mask are regenerate
 Slate parity is audited, not just asserted: the MLP blocks here are a sequential-k FMA chain, within ~1e-6 of
 torch's addmm but not bit-identical to it, so a query row can differ from the reference's by |dq| ~ 1e-6 and an
 arg-max whose reference top-1/top-2 gap is below 2*|dq| may legitimately flip (table rows have unit norm, so a
-logit moves by at most |dq|).  Every mismatch must be such a near-tie; anything else fails.  The counts go to
-gpurun_out/parity_big.json (copied to profiles/ and quoted in DESIGN.md).
+logit moves by at most |dq|).  Every mismatch must be such a near-tie; anything else fails.  The counts go to the
+JSON file named by $PCV_PARITY_REPORT when it is set (profiles/*_parity_big.json, quoted in DESIGN.md).
 
 CPU legs (-m "not gpu") run the same audit on the oracle; GPU legs (-m gpu) on the drop-in classes through the C ABI.
 """
@@ -27,8 +27,7 @@ import synth  # noqa: E402
 
 import oracle  # noqa: E402
 
-ROOT = os.path.dirname(HERE)
-REPORT = os.path.join(ROOT, "gpurun_out", "parity_big.json")
+REPORT = os.environ.get("PCV_PARITY_REPORT")
 
 _fx_cache, _w_cache = {}, {}
 
@@ -50,7 +49,9 @@ def weights(workload, kind, fx, prefix=""):
 
 
 def report(key, entry):
-    os.makedirs(os.path.dirname(REPORT), exist_ok=True)
+    if not REPORT:
+        return
+    os.makedirs(os.path.dirname(os.path.abspath(REPORT)), exist_ok=True)
     data = {}
     if os.path.exists(REPORT):
         try:

@@ -243,6 +243,76 @@ def test_bench_reference_arm_runs_on_cpu():
     assert line["e2e"]["h2d_bytes_per_step"] == 0 and line["unit"] == "slates/s"
 
 
+def test_bench_dump_outputs_dtypes_and_size_limit(tmp_path, monkeypatch):
+    """bench.dump_outputs: item ids as float64, scores as float32, scalars whole; past DUMP_LIMIT every array keeps the
+    same fixed sample of its rows, stored beside it as <name>.rows.npy."""
+    import bench
+    arrays = {"items": torch.arange(5000, dtype=torch.int64).view(1000, 5) * 977, "resp": torch.randn(1000, 5),
+              "loss": torch.tensor(0.25, dtype=torch.float64)}
+    bench.dump_outputs(str(tmp_path / "all"), arrays)
+    items, resp, loss = (np.load(tmp_path / "all" / (k + ".npy")) for k in ("items", "resp", "loss"))
+    assert items.dtype == np.float64 and np.array_equal(items, arrays["items"].numpy())
+    assert resp.dtype == np.float32 and np.array_equal(resp, arrays["resp"].numpy())
+    assert loss.dtype == np.float64 and loss == 0.25
+    assert sorted(os.listdir(tmp_path / "all")) == ["items.npy", "loss.npy", "resp.npy"]
+    monkeypatch.setattr(bench, "DUMP_LIMIT", 30000)
+    for run in ("cut", "cut_again"):
+        bench.dump_outputs(str(tmp_path / run), arrays)
+    for k in ("items", "resp"):
+        rows = np.load(tmp_path / "cut" / (k + ".rows.npy"))
+        got = np.load(tmp_path / "cut" / (k + ".npy"))
+        assert 0 < len(rows) < 1000 and (np.diff(rows) > 0).all()
+        assert np.array_equal(got, arrays[k].numpy()[rows.astype(np.int64)].astype(got.dtype))
+        assert np.array_equal(rows, np.load(tmp_path / "cut_again" / (k + ".rows.npy")))
+    assert sum(f.stat().st_size for f in (tmp_path / "cut").iterdir()) <= 30000
+    assert np.load(tmp_path / "cut" / "loss.npy") == 0.25
+
+
+def test_bench_times_exactly_k_steps(monkeypatch):
+    """bench.timed_steps: the W warm-up steps run before the first event; then exactly K steps, each alone between the
+    two events of its pair, and the result is the sum of the K pairs."""
+    import bench
+    log = []
+
+    class Event:
+        def __init__(self, enable_timing=False):
+            self.id = len([e for e in log if e[0] == "new"])
+            log.append(("new", self.id))
+
+        def record(self):
+            log.append(("record", self.id))
+
+        def elapsed_time(self, end):
+            return 1.5
+
+    class Dist:
+        def barrier(self):
+            log.append(("barrier",))
+
+        def max_(self, values):
+            return values
+
+    class Flush:
+        def zero_(self):
+            log.append(("flush",))
+
+    monkeypatch.setattr(torch.cuda, "Event", Event)
+    K, W = 7, 3
+    ms = bench.timed_steps(Dist(), lambda i: log.append(("step", i)), K, W, Flush())
+    assert ms == 1.5 * K
+    first = log.index(next(e for e in log if e[0] == "record"))
+    assert [e for e in log[:first] if e[0] == "step"] == [("step", i % K) for i in range(W)]
+    timed = [e for e in log[first:] if e[0] != "flush"]
+    assert timed[:-1] == [x for i in range(K) for x in (("record", 2 * i), ("step", i), ("record", 2 * i + 1))]
+    assert timed[-1] == ("barrier",)
+
+
+@pytest.mark.parametrize("argv", [["--steps", "0"], ["--impl", "reference", "--dump-outputs", "x"]])
+def test_bench_rejects_bad_arguments(argv):
+    out = subprocess.run([sys.executable, os.path.join(ROOT, "bench.py")] + argv, capture_output=True, text=True, timeout=300)
+    assert out.returncode == 2 and "error" in out.stderr
+
+
 def test_mlp_engine_policy_is_validated_and_scoped():
     """ops.mlp_engine: context manager over the process default; unknown names are rejected; the library default is the
     bit-exact FFMA engine and the model classes default to it (mlp_engine = None)."""
