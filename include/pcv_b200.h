@@ -30,7 +30,7 @@
 extern "C" {
 #endif
 
-#define PCV_ABI_VERSION 1
+#define PCV_ABI_VERSION 2
 
 #define PCV_OK 0
 #define PCV_ERR_ARG (-1)
@@ -166,14 +166,11 @@ typedef struct {
   const float *W; /* [n_out, n_in] row-major == nn.Linear.weight */
   const float *b; /* [n_out]                                     */
   int n_in, n_out, act;
-  /* optional: the same weights pre-tiled by pcv_mlp_pack (NULL = stream W as is).  When EVERY layer
-   * of a launch carries one, the TMA engine runs (one bulk copy per 32-k chunk, FMA-pipe-bound);
-   * results are bit-identical.  The caller re-packs after the weights change. */
+  /* the same weights pre-tiled by pcv_mlp_pack: required on every layer when the launch runs
+   * PCV_MLP_KERNEL_CLUSTER, ignored otherwise.  The caller re-packs after the weights change. */
   const float *Wp;
-  /* optional: the same weights split in tf32 hi | lo and pre-swizzled by pcv_mlp_tc_pack.  When EVERY layer of a
-   * launch carries one (and the block fits: assembled input <= 64 wide, layers <= 256 wide, no saved activations) the
-   * tensor-core engine runs (csrc/mlp_tc.cu: tcgen05 3xTF32, activations chained through TMEM).  fp32-grade results
-   * (~1e-6 relative of torch's addmm) but NOT bit-identical to the FFMA engines. */
+  /* the same weights split in tf32 hi | lo and pre-swizzled by pcv_mlp_tc_pack: required on every layer when the
+   * launch runs PCV_MLP_KERNEL_TC, ignored otherwise. */
   const float *Wt;
 } pcv_linear;
 
@@ -224,10 +221,28 @@ typedef struct {
   const uint64_t *offset_dev; /* optional device counter added to `offset` (CUDA-graph replays) */
 } pcv_mlp_desc;
 
-int pcv_mlp_fwd(const pcv_mlp_desc *d, int64_t B, pcv_stream_t stream);
+/* Engine policy of a launch (`engine` below). */
+#define PCV_MLP_EXACT 0 /* the FFMA engines: sequential-k FMA chain, bit-identical to the CPU oracle */
+#define PCV_MLP_TC 1    /* the tensor-core engine when every block of the launch fits it (assembled input <= 64 wide,
+                         * layers <= 256 wide, at most one one-hot segment of <= 16 clicks), the FFMA engines otherwise.
+                         * tcgen05 3xTF32, activations chained through TMEM: fp32-grade (~1e-6 relative of torch's
+                         * addmm) but NOT bit-identical to the FFMA engines */
+#define PCV_MLP_AUTO 2  /* PCV_MLP_TC from 2048 batch rows, PCV_MLP_EXACT below */
+/* The kernel that runs a launch. */
+#define PCV_MLP_KERNEL_TC 0      /* csrc/mlp_tc.cu; reads pcv_linear.Wt */
+#define PCV_MLP_KERNEL_CLUSTER 1 /* packed-weight FFMA engine (TMA-fed 4-CTA clusters); reads pcv_linear.Wp */
+#define PCV_MLP_KERNEL_STREAM 2  /* streaming FFMA engine; reads W; the only one that writes x0 / acts */
+
+/* *kernel = the kernel that pcv_mlp_fwd (b NULL) or pcv_mlp_fwd2 runs for these descriptors, B and engine.  It reads
+ * shapes and saved outputs only, no weight image, launches nothing and needs no GPU: the caller packs the image that
+ * kernel reads, then launches with the same arguments. */
+int pcv_mlp_plan(const pcv_mlp_desc *a, const pcv_mlp_desc *b, int64_t B, int engine, int *kernel);
+/* Runs the kernel pcv_mlp_plan names for the same arguments; PCV_ERR_ARG when a layer lacks the weight image that
+ * kernel reads (no fall-back to another engine). */
+int pcv_mlp_fwd(const pcv_mlp_desc *d, int64_t B, int engine, pcv_stream_t stream);
 /* Two chained blocks in ONE launch: b may read (as DENSE segments) what a writes for the same
  * batch rows, e.g. prior -> reparameterise -> PSM (pivotcvae.py:279-291, 204-210). */
-int pcv_mlp_fwd2(const pcv_mlp_desc *a, const pcv_mlp_desc *b, int64_t B, pcv_stream_t stream);
+int pcv_mlp_fwd2(const pcv_mlp_desc *a, const pcv_mlp_desc *b, int64_t B, int engine, pcv_stream_t stream);
 /* Pre-tile one nn.Linear weight [n_out, n_in] for pcv_linear.Wp: `packed` (device, 128-byte aligned)
  * holds pcv_mlp_packed_bytes(n_in, n_out) bytes. */
 size_t pcv_mlp_packed_bytes(int n_in, int n_out);

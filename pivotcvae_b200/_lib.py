@@ -20,6 +20,8 @@ NORM_NONE, NORM_SEGMENT = 0, 1
 SELECT_GREEDY, SELECT_EXPRACE = 0, 1
 ENGINE_AUTO, ENGINE_SIMT, ENGINE_TCGEN05, ENGINE_TCGEN05_F16 = 0, 1, 2, 3
 URM, URM_P, URM_P_MR = 0, 1, 2
+MLP_EXACT, MLP_TC, MLP_AUTO = 0, 1, 2
+MLP_KERNEL_TC, MLP_KERNEL_CLUSTER, MLP_KERNEL_STREAM = 0, 1, 2
 
 c_void_p, c_int, c_int64, c_uint64, c_size_t = (ctypes.c_void_p, ctypes.c_int, ctypes.c_int64,
                                                 ctypes.c_uint64, ctypes.c_size_t)
@@ -97,8 +99,9 @@ EXPORTS = {
     "pcv_sigmoid_categorical": (c_int, [c_void_p, c_void_p, c_int64, c_uint64, c_uint64, c_void_p, c_void_p, c_void_p, c_void_p]),
     "pcv_vp_pack_keys": (c_int, [c_void_p, c_void_p, c_int64, c_void_p, c_void_p]),
     "pcv_vp_unpack_keys": (c_int, [c_void_p, c_int64, c_void_p, c_void_p, c_void_p]),
-    "pcv_mlp_fwd": (c_int, [ctypes.POINTER(MlpDesc), c_int64, c_void_p]),
-    "pcv_mlp_fwd2": (c_int, [ctypes.POINTER(MlpDesc), ctypes.POINTER(MlpDesc), c_int64, c_void_p]),
+    "pcv_mlp_plan": (c_int, [ctypes.POINTER(MlpDesc), ctypes.POINTER(MlpDesc), c_int64, c_int, ctypes.POINTER(c_int)]),
+    "pcv_mlp_fwd": (c_int, [ctypes.POINTER(MlpDesc), c_int64, c_int, c_void_p]),
+    "pcv_mlp_fwd2": (c_int, [ctypes.POINTER(MlpDesc), ctypes.POINTER(MlpDesc), c_int64, c_int, c_void_p]),
     "pcv_gemm_tn": (c_int, [ctypes.POINTER(GemmDesc), c_void_p]),
     "pcv_transpose_batch": (c_int, [ctypes.POINTER(TransposeJob), c_int, c_void_p]),
     "pcv_wgrad_reduce": (c_int, [c_void_p, c_int, c_int64, c_int64, c_int, c_int, c_void_p, c_int64, c_void_p, c_int64, c_int64,

@@ -6,10 +6,9 @@ of the MLP blocks runs on the library's own tensor-core GEMMs (csrc/gemm_tc.cu):
 per layer one split-K weight-gradient GEMM (+ a deterministic reduce that also
 emits the bias gradient) and one input-gradient GEMM whose epilogue applies the
 activation derivative and writes the transposed copy the next weight-gradient
-GEMM consumes.  MLP_BWD_ENGINE = "tc3" (3xTF32: fp32-grade products, default),
-"tc" (one tf32 pass: the reduced-precision training config) or "torch" (the
-legacy torch.mm path, kept for A/B checks).  The PSM block never needs a backward
-(SURVEY F6).
+GEMM consumes.  MLP_BWD_ENGINE = "tc3" (3xTF32: fp32-grade products, default)
+or "tc" (one tf32 pass: the reduced-precision training config).  The PSM block
+never needs a backward (SURVEY F6).
 """
 import torch
 
@@ -170,7 +169,9 @@ class FusedMLPFn(torch.autograd.Function):
         Ws = saved[nl + 1:nl + 1 + nl]
         c0 = spec.out_col0
         g = None
-        if spec.latent and (d_z is not None) and c0 == 0 and ctx.n_out == 2 * spec.latent and MLP_BWD_ENGINE != "torch":
+        if MLP_BWD_ENGINE not in ("tc3", "tc"):
+            raise ValueError("MLP_BWD_ENGINE must be 'tc3' or 'tc'")
+        if spec.latent and (d_z is not None) and c0 == 0 and ctx.n_out == 2 * spec.latent:
             # [mu | logvar] block: the reparameterisation's backward and the sum with d_out in ONE kernel
             do = d_out if (d_out is None or d_out.stride(1) == 1) else d_out.contiguous()
             g = ops.reparam_bwd(do, d_z, saved[-1], out, spec.latent)
@@ -187,19 +188,9 @@ class FusedMLPFn(torch.autograd.Function):
         if g is None:
             return (None,) * (3 + ctx.n_dense + 2 * nl)
         g = g.contiguous()
-        grads_wb = [None] * (2 * nl)
-        if MLP_BWD_ENGINE != "torch":
-            g = _act_grad(g, out[:, c0:c0 + ctx.n_out], spec.acts[nl - 1])      # identity for every block of the path
-            need_in = any(s[0] == "dense" and ctx.needs_input_grad[3 + s[1]] for s in spec.segs)
-            grads_wb, g = _mlp_backward_tc(g, x0, acts, Ws, spec.acts, need_in, MLP_BWD_ENGINE == "tc3")
-        else:
-            for l in range(nl - 1, -1, -1):
-                a_out = out[:, c0:c0 + ctx.n_out] if l == nl - 1 else acts[l]
-                g = _act_grad(g, a_out, spec.acts[l])
-                a_prev = x0 if l == 0 else acts[l - 1]
-                grads_wb[2 * l] = g.t().mm(a_prev)
-                grads_wb[2 * l + 1] = g.sum(0)
-                g = g.mm(Ws[l])
+        g = _act_grad(g, out[:, c0:c0 + ctx.n_out], spec.acts[nl - 1])      # identity for every block of the path
+        need_in = any(s[0] == "dense" and ctx.needs_input_grad[3 + s[1]] for s in spec.segs)
+        grads_wb, g = _mlp_backward_tc(g, x0, acts, Ws, spec.acts, need_in, MLP_BWD_ENGINE == "tc3")
         d_dense = [None] * ctx.n_dense
         for si, s in enumerate(spec.segs):
             if s[0] == "dense" and ctx.needs_input_grad[3 + s[1]]:

@@ -698,7 +698,7 @@ using namespace pcv;
 
 extern "C" {
 
-static int mlp_prepare(const pcv_mlp_desc *d, MlpParams *Pp, int *maxw_out, int *bias_total) {
+static int mlp_prepare(const pcv_mlp_desc *d, MlpParams *Pp) {
   MlpParams &P = *Pp;
   PCV_CHECK_ARG(d != nullptr, "desc is NULL");
   PCV_CHECK_ARG(d->n_segments >= 1 && d->n_segments <= PCV_MAX_SEGMENTS, "bad n_segments");
@@ -727,7 +727,6 @@ static int mlp_prepare(const pcv_mlp_desc *d, MlpParams *Pp, int *maxw_out, int 
   P.n_in0 = off;
   int maxw = off;
   int prev = off;
-  int bt = 0;
   for (int l = 0; l < d->n_layers; ++l) {
     const pcv_linear &L = d->layer[l];
     PCV_CHECK_ARG(L.W && L.b, "layer weights are NULL");
@@ -739,7 +738,6 @@ static int mlp_prepare(const pcv_mlp_desc *d, MlpParams *Pp, int *maxw_out, int 
     PCV_CHECK_ARG(((uintptr_t)L.W & 15) == 0, "layer weight must be 16-byte aligned");
     if (L.n_out > maxw) maxw = L.n_out;
     prev = L.n_out;
-    bt += L.n_out;
   }
   PCV_CHECK_ARG(maxw <= PCV_MAX_WIDTH, "layer wider than PCV_MAX_WIDTH");
   PCV_CHECK_ARG(d->copy_seg < d->n_segments, "copy_seg out of range");
@@ -748,60 +746,73 @@ static int mlp_prepare(const pcv_mlp_desc *d, MlpParams *Pp, int *maxw_out, int 
     PCV_CHECK_ARG(prev == 2 * d->latent, "reparam needs the last layer to emit 2*latent");
     PCV_CHECK_ARG(d->z != nullptr, "z is NULL");
   }
-  *maxw_out = maxw;
-  *bias_total = bt;
+  P.ld = (maxw + 3) & ~3;
   return PCV_OK;
 }
 
-static bool mlp_all_packed(const MlpParams *P) {
-  for (int l = 0; l < P->d.n_layers; ++l)
-    if (P->d.layer[l].Wp == nullptr) return false;
-  return true;
+static bool mlp_saves(const MlpParams &P) {
+  for (int l = 0; l < P.d.n_layers - 1; ++l)
+    if (P.d.acts[l] != nullptr) return true;
+  return P.d.x0 != nullptr;
 }
 
-// packed-weight cluster engine: 32 rows per cluster of 4 CTAs
-static int mlp_launch_cluster(const MlpParams *Pa, const MlpParams *Pb, int64_t B, int ld, cudaStream_t st, bool *done) {
-  *done = false;
-  ld = (ld + MLP_KC - 1) / MLP_KC * MLP_KC;   // k ranges / column blocks are zero-padded to multiples of 32
-  const int64_t clusters = (B + MLPC_BM - 1) / MLPC_BM;
-  int sm_count = 148, dev = 0;
-  cudaGetDevice(&dev);
-  cudaDeviceGetAttribute(&sm_count, cudaDevAttrMultiProcessorCount, dev);
-  const int stages = (clusters * MLPC_CL > sm_count) ? 4 : MLPC_STAGES;
-  const size_t smem = (size_t)stages * MLPC_TILE_FLOATS * sizeof(float) + 2 * stages * 8 +
-                      (size_t)2 * ld * MLPC_ALD * sizeof(float);
-  if (smem > 227 * 1024) return PCV_OK;   // does not fit: the caller falls back to the streaming engine
-  MlpParams2 P2;
-  P2.a = *Pa;
-  P2.b = Pb ? *Pb : *Pa;
-  P2.a.ld = ld; P2.b.ld = ld;
+// packed-weight cluster engine: 32 rows per cluster of 4 CTAs; k ranges / column blocks are zero-padded to multiples
+// of 32; a grid of more than one wave gets the shallower weight ring
+static size_t mlpc_smem(int64_t B, int ld, int sm_count, int *stages) {
+  *stages = ((B + MLPC_BM - 1) / MLPC_BM * MLPC_CL > sm_count) ? 4 : MLPC_STAGES;
+  return (size_t)*stages * MLPC_TILE_FLOATS * sizeof(float) + 2 * *stages * 8 + (size_t)2 * ld * MLPC_ALD * sizeof(float);
+}
+static int mlpc_ld(int ld) { return (ld + MLP_KC - 1) / MLP_KC * MLP_KC; }
+
+// Validates the descriptors (b NULL = one block, then P->b = P->a; both blocks share the wider activation stride) and
+// chooses the kernel: the one decision behind pcv_mlp_plan, pcv_mlp_fwd and pcv_mlp_fwd2.  It reads shapes and saved
+// outputs, never a weight image.
+static int mlp_plan(const pcv_mlp_desc *a, const pcv_mlp_desc *b, int64_t B, int engine, MlpParams2 *P, int *sm_count,
+                    int *kernel) {
+  PCV_CHECK_ARG(B > 0, "B must be > 0");
+  PCV_CHECK_ARG(engine == PCV_MLP_EXACT || engine == PCV_MLP_TC || engine == PCV_MLP_AUTO, "unknown engine");
+  int rc = mlp_prepare(a, &P->a);
+  if (rc != PCV_OK) return rc;
+  P->b = P->a;
+  if (b && (rc = mlp_prepare(b, &P->b)) != PCV_OK) return rc;
+  P->a.ld = P->b.ld = P->a.ld > P->b.ld ? P->a.ld : P->b.ld;
+  int dev = 0;
+  if (cudaGetDevice(&dev) != cudaSuccess ||
+      cudaDeviceGetAttribute(sm_count, cudaDevAttrMultiProcessorCount, dev) != cudaSuccess) {
+    cudaGetLastError();
+    *sm_count = 148;   // no device (pcv_mlp_plan on a host without a GPU): a B200's count
+  }
+  int stages;
+  if (mlp_saves(P->a) || mlp_saves(P->b))
+    *kernel = PCV_MLP_KERNEL_STREAM;   // only the streaming engine writes x0 / acts
+  else if (mlp_tc_takes(*P, B, engine))
+    *kernel = PCV_MLP_KERNEL_TC;
+  else
+    *kernel = mlpc_smem(B, mlpc_ld(P->a.ld), *sm_count, &stages) <= 227 * 1024 ? PCV_MLP_KERNEL_CLUSTER
+                                                                              : PCV_MLP_KERNEL_STREAM;
+  return PCV_OK;
+}
+
+static int mlp_launch_cluster(MlpParams2 P2, int nblk, int64_t B, int sm_count, cudaStream_t st) {
+  P2.a.ld = P2.b.ld = mlpc_ld(P2.a.ld);
+  int stages;
+  const size_t smem = mlpc_smem(B, P2.a.ld, sm_count, &stages);
+  const unsigned grid = (unsigned)((B + MLPC_BM - 1) / MLPC_BM * MLPC_CL);
   if (stages == 4) {
     PCV_CUDA(cudaFuncSetAttribute(mlp_cluster_kernel<4>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
-    mlp_cluster_kernel<4><<<(unsigned)(clusters * MLPC_CL), MLPC_NC + 32, smem, st>>>(P2, Pb ? 2 : 1, B);
+    mlp_cluster_kernel<4><<<grid, MLPC_NC + 32, smem, st>>>(P2, nblk, B);
   } else {
     PCV_CUDA(cudaFuncSetAttribute(mlp_cluster_kernel<MLPC_STAGES>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
-    mlp_cluster_kernel<MLPC_STAGES><<<(unsigned)(clusters * MLPC_CL), MLPC_NC + 32, smem, st>>>(P2, Pb ? 2 : 1, B);
+    mlp_cluster_kernel<MLPC_STAGES><<<grid, MLPC_NC + 32, smem, st>>>(P2, nblk, B);
   }
   PCV_LAUNCH_CHECK();
-  *done = true;
   return PCV_OK;
 }
 
-static int mlp_launch(const MlpParams *Pa, const MlpParams *Pb, int64_t B, cudaStream_t st) {
-  int sm_count = 148;
-  int dev = 0;
-  cudaGetDevice(&dev);
-  cudaDeviceGetAttribute(&sm_count, cudaDevAttrMultiProcessorCount, dev);
-  if (mlp_tc_supported(Pa) && (!Pb || mlp_tc_supported(Pb))) return mlp_tc_launch(Pa, Pb, B, st);
-  if (mlp_all_packed(Pa) && (!Pb || mlp_all_packed(Pb))) {
-    const int ldp = Pb ? (Pa->ld > Pb->ld ? Pa->ld : Pb->ld) : Pa->ld;
-    bool done = false;
-    int rc = mlp_launch_cluster(Pa, Pb, B, ldp, st, &done);
-    if (rc != PCV_OK || done) return rc;
-  }
+static int mlp_launch_stream(const MlpParams2 &P2, int nblk, int64_t B, int sm_count, cudaStream_t st) {
+  const int ld = P2.a.ld;
   // rows per CTA: 8 / 16 / 32 — small batches spread over more SMs (and use 16 warps per CTA)
   int CT = (B <= (int64_t)sm_count * 16) ? 1 : (B <= (int64_t)sm_count * 64 ? 2 : 4);
-  const int ld = Pb ? (Pa->ld > Pb->ld ? Pa->ld : Pb->ld) : Pa->ld;
   auto smem_of = [&](int ct) { return (size_t)(2 * ld * (8 * ct + 4) + 2 * MLP_KC * MLP_WLD_MAX) * sizeof(float); };
   while (CT > 1 && smem_of(CT) > 227 * 1024) CT >>= 1;   // wide layers (up to PCV_MAX_WIDTH = 1024): fewer rows per CTA
   const int BM = 8 * CT;
@@ -812,15 +823,12 @@ static int mlp_launch(const MlpParams *Pa, const MlpParams *Pb, int64_t B, cudaS
   }
   int64_t blocks = (B + BM - 1) / BM;
 #define PCV_MLP_LAUNCH(CTv, RTv, THv)                                                                              \
-  if (Pb) {                                                                                                        \
-    MlpParams2 P2;                                                                                                 \
-    P2.a = *Pa; P2.b = *Pb;                                                                                        \
-    P2.a.ld = ld; P2.b.ld = ld;                                                                                    \
+  if (nblk == 2) {                                                                                                 \
     PCV_CUDA(cudaFuncSetAttribute(mlp_fwd2_kernel<CTv, RTv, THv>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem)); \
     mlp_fwd2_kernel<CTv, RTv, THv><<<(unsigned)blocks, THv, smem, st>>>(P2, B);                                  \
   } else {                                                                                                         \
     PCV_CUDA(cudaFuncSetAttribute(mlp_fwd_kernel<CTv, RTv, THv>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem)); \
-    mlp_fwd_kernel<CTv, RTv, THv><<<(unsigned)blocks, THv, smem, st>>>(*Pa, B);                                  \
+    mlp_fwd_kernel<CTv, RTv, THv><<<(unsigned)blocks, THv, smem, st>>>(P2.a, B);                                 \
   }
   if (CT == 1) { PCV_MLP_LAUNCH(1, 4, 512) } else if (CT == 2) { PCV_MLP_LAUNCH(2, 8, 256) } else { PCV_MLP_LAUNCH(4, 8, 256) }
 #undef PCV_MLP_LAUNCH
@@ -828,31 +836,43 @@ static int mlp_launch(const MlpParams *Pa, const MlpParams *Pb, int64_t B, cudaS
   return PCV_OK;
 }
 
-int pcv_mlp_fwd(const pcv_mlp_desc *d, int64_t B, pcv_stream_t stream) {
-  PCV_CHECK_ARG(B > 0, "B must be > 0");
-  MlpParams P;
-  int maxw = 0, bt = 0;
-  int rc = mlp_prepare(d, &P, &maxw, &bt);
+static int mlp_run(const pcv_mlp_desc *a, const pcv_mlp_desc *b, int64_t B, int engine, cudaStream_t st) {
+  MlpParams2 P;
+  int sm_count, kernel;
+  int rc = mlp_plan(a, b, B, engine, &P, &sm_count, &kernel);
   if (rc != PCV_OK) return rc;
+  const int nblk = b ? 2 : 1;
+  // the planned kernel reads its weight image on every layer: a missing one is an error, not a fallback
+  for (int blk = 0; blk < nblk && kernel != PCV_MLP_KERNEL_STREAM; ++blk)
+    for (int l = 0; l < (blk ? P.b : P.a).d.n_layers; ++l) {
+      const pcv_linear &L = (blk ? P.b : P.a).d.layer[l];
+      if ((kernel == PCV_MLP_KERNEL_TC ? L.Wt : L.Wp) == nullptr) {
+        set_error("pcv_mlp_fwd: block %d layer %d has no pcv_linear.%s, which the planned %s kernel reads", blk, l,
+                  kernel == PCV_MLP_KERNEL_TC ? "Wt" : "Wp", kernel == PCV_MLP_KERNEL_TC ? "tc" : "cluster");
+        return PCV_ERR_ARG;
+      }
+    }
   rc = check_arch();
   if (rc != PCV_OK) return rc;
-  P.ld = (maxw + 3) & ~3;
-  return mlp_launch(&P, nullptr, B, (cudaStream_t)stream);
+  if (kernel == PCV_MLP_KERNEL_TC) return mlp_tc_launch(P, nblk, B, st);
+  if (kernel == PCV_MLP_KERNEL_CLUSTER) return mlp_launch_cluster(P, nblk, B, sm_count, st);
+  return mlp_launch_stream(P, nblk, B, sm_count, st);
 }
 
-int pcv_mlp_fwd2(const pcv_mlp_desc *a, const pcv_mlp_desc *b, int64_t B, pcv_stream_t stream) {
-  PCV_CHECK_ARG(B > 0, "B must be > 0");
-  MlpParams Pa, Pb;
-  int wa = 0, wb = 0, bt = 0;
-  int rc = mlp_prepare(a, &Pa, &wa, &bt);
-  if (rc != PCV_OK) return rc;
-  rc = mlp_prepare(b, &Pb, &wb, &bt);
-  if (rc != PCV_OK) return rc;
-  rc = check_arch();
-  if (rc != PCV_OK) return rc;
-  Pa.ld = (wa + 3) & ~3;
-  Pb.ld = (wb + 3) & ~3;
-  return mlp_launch(&Pa, &Pb, B, (cudaStream_t)stream);
+int pcv_mlp_plan(const pcv_mlp_desc *a, const pcv_mlp_desc *b, int64_t B, int engine, int *kernel) {
+  PCV_CHECK_ARG(kernel != nullptr, "kernel is NULL");
+  MlpParams2 P;
+  int sm_count;
+  return mlp_plan(a, b, B, engine, &P, &sm_count, kernel);
+}
+
+int pcv_mlp_fwd(const pcv_mlp_desc *d, int64_t B, int engine, pcv_stream_t stream) {
+  return mlp_run(d, nullptr, B, engine, (cudaStream_t)stream);
+}
+
+int pcv_mlp_fwd2(const pcv_mlp_desc *a, const pcv_mlp_desc *b, int64_t B, int engine, pcv_stream_t stream) {
+  PCV_CHECK_ARG(b != nullptr, "desc b is NULL");
+  return mlp_run(a, b, B, engine, (cudaStream_t)stream);
 }
 
 size_t pcv_mlp_packed_bytes(int n_in, int n_out) {

@@ -41,8 +41,9 @@ struct MlpParams2 {
   MlpParams a, b;
 };
 
-// tensor-core engine (mlp_tc.cu): runs when every layer of the launch carries the tc-packed weights (pcv_linear.Wt)
-bool mlp_tc_supported(const MlpParams *P);
-int mlp_tc_launch(const MlpParams *Pa, const MlpParams *Pb, int64_t B, cudaStream_t st);
+// tensor-core engine (mlp_tc.cu).  mlp_tc_takes: the engine policy (PCV_MLP_*) asks for it at B rows and both blocks
+// of P fit it (one block: P.b = P.a); saved outputs are the caller's concern.  nblk = 1 | 2 blocks in the launch.
+bool mlp_tc_takes(const MlpParams2 &P, int64_t B, int engine);
+int mlp_tc_launch(const MlpParams2 &P2, int nblk, int64_t B, cudaStream_t st);
 
 }  // namespace pcv

@@ -41,6 +41,11 @@ constexpr int MT_BM = 128;                  // batch rows per CTA (TMEM lanes)
 constexpr int MT_KC = 32;                   // k-chunk: 32 fp32 = one 128-byte swizzle row
 constexpr int MT_MAXN = 256;                // widest layer (one TMEM region)
 constexpr int MT_MAXK0 = 64;                // widest assembled input (two operand chunks = both operand buffers)
+constexpr int MT_MAXCLICKS = 16;            // one-hot segment: clicks per row the prologue handles
+// PCV_MLP_AUTO takes this engine from this many batch rows: a CTA owns 128 rows and takes ~30 us per block whatever
+// the batch, while the FFMA cluster engine spreads 1024 rows over 128 CTAs in ~18 us but needs ~50 us at 4096 rows
+// and ~180 us at 16384.
+constexpr int64_t MT_AUTO_MIN_ROWS = 2048;
 constexpr int MT_TWOPASS_K = 64;            // layers deeper than this: small terms first, then hi*hi (see above)
 constexpr int MT_SLOT_N = 64;               // layers at most this wide keep FOUR accumulators per output in their 256-column
 constexpr int MT_NSLOT = 4;                 // region instead (slot 0: small terms, slots 1-3: hi*hi round-robin; added in fp32 RN
@@ -563,25 +568,25 @@ mlp_tc_kernel(const __grid_constant__ MlpParams2 P2, int n_blocks, int64_t B) {
   }
 }
 
-bool mlp_tc_supported(const MlpParams *P) {
+static bool mlp_tc_fits(const MlpParams *P) {
   const pcv_mlp_desc &d = P->d;
-  if (P->n_in0 > MT_MAXK0 || d.x0 != nullptr) return false;
+  if (P->n_in0 > MT_MAXK0) return false;
   int n_onehot = 0;
   for (int s = 0; s < d.n_segments; ++s)
     if (d.seg[s].kind == PCV_SEG_ONEHOT) {
-      if (++n_onehot > 1 || d.seg[s].count > 16) return false;
+      if (++n_onehot > 1 || d.seg[s].count > MT_MAXCLICKS) return false;
     }
-  for (int l = 0; l < d.n_layers; ++l) {
-    if (d.layer[l].Wt == nullptr || d.layer[l].n_out > MT_MAXN) return false;
-    if (l < d.n_layers - 1 && d.acts[l] != nullptr) return false;
-  }
+  for (int l = 0; l < d.n_layers; ++l)
+    if (d.layer[l].n_out > MT_MAXN) return false;
   return true;
 }
 
-int mlp_tc_launch(const MlpParams *Pa, const MlpParams *Pb, int64_t B, cudaStream_t st) {
-  MlpParams2 P2;
-  P2.a = *Pa;
-  P2.b = Pb ? *Pb : *Pa;
+bool mlp_tc_takes(const MlpParams2 &P, int64_t B, int engine) {
+  const bool wanted = engine == PCV_MLP_TC || (engine == PCV_MLP_AUTO && B >= MT_AUTO_MIN_ROWS);
+  return wanted && mlp_tc_fits(&P.a) && mlp_tc_fits(&P.b);
+}
+
+int mlp_tc_launch(const MlpParams2 &P2, int nblk, int64_t B, cudaStream_t st) {
   int dev = 0;
   cudaGetDevice(&dev);
   static bool attr_set[64] = {false};
@@ -594,7 +599,7 @@ int mlp_tc_launch(const MlpParams *Pa, const MlpParams *Pb, int64_t B, cudaStrea
     attr_set[dev & 63] = true;
   }
   const int64_t blocks = (B + MT_BM - 1) / MT_BM;
-  mlp_tc_kernel<<<(unsigned)blocks, MT_THREADS, MT_SMEM, st>>>(P2, Pb ? 2 : 1, B);
+  mlp_tc_kernel<<<(unsigned)blocks, MT_THREADS, MT_SMEM, st>>>(P2, nblk, B);
   cudaError_t e = cudaGetLastError();
   if (e != cudaSuccess) {
     set_error("pcv_mlp_fwd (tc engine): kernel launch -> %s", cudaGetErrorString(e));

@@ -394,22 +394,19 @@ def repack_stale():
             hit[0] = hit[4]._version
 
 
-PACK_WEIGHTS = True   # False: always stream nn.Linear weights as they are (the training engine)
 # Inference engine of the fused MLP blocks: "exact" = the FFMA engines (sequential-k FMA chain, bit-identical to the
-# CPU oracle); "tc" = the tcgen05 3xTF32 engine (csrc/mlp_tc.cu: fp32-grade, ~1e-6 of torch's addmm) wherever a block
-# fits it (input <= 64 wide, layers <= 256 wide), the exact engines elsewhere; "auto" = "tc" for batches of at least
-# TC_MIN_ROWS rows (a tcgen05 CTA owns 128 rows and takes ~30 us per block whatever the batch, the FFMA engine spreads
-# 1024 rows over 128 CTAs in ~18 us but needs ~50 us at 4096 rows and ~180 us at 16384), "exact" below.
+# CPU oracle); "tc" = the tcgen05 3xTF32 engine (csrc/mlp_tc.cu: fp32-grade, ~1e-6 of torch's addmm) wherever every
+# block of a launch fits it, the exact engines elsewhere; "auto" = "tc" for large batches, "exact" below.  The library
+# decides which kernel runs (pcv_mlp_plan, include/pcv_b200.h).
 MLP_ENGINE = "exact"
-TC_MAX_IN, TC_MAX_WIDTH = 64, 256
-TC_MIN_ROWS = 2048
+_MLP_POLICY = {"exact": L.MLP_EXACT, "tc": L.MLP_TC, "auto": L.MLP_AUTO}
 
 
 class mlp_engine:
     """Context manager: `with ops.mlp_engine("tc"): ...`"""
 
     def __init__(self, name):
-        if name not in ("exact", "tc", "auto"):
+        if name not in _MLP_POLICY:
             raise ValueError("mlp engine must be 'exact', 'tc' or 'auto'")
         self.name = name
 
@@ -423,8 +420,9 @@ class mlp_engine:
 
 
 def _mlp_desc(segments, layers, B, *, out=None, out_ld=None, out_col0=0, copy_seg=-1, save=False,
-              latent=0, eps=None, seed=0, offset=0, offset_dev=None, engine=None):
-    """Build a pcv_mlp_desc (+ its output tensors); returns (desc, results, keep-alive list, device)."""
+              latent=0, eps=None, seed=0, offset=0, offset_dev=None):
+    """Build a pcv_mlp_desc without weight images (+ its output tensors); returns ((desc, keep-alive list, the layers'
+    fp32 weights), results, device)."""
     if len(segments) > L.PCV_MAX_SEGMENTS or len(layers) > L.PCV_MAX_LAYERS:
         raise L.PcvError("too many segments / layers for one fused block")
     d = L.MlpDesc()
@@ -433,27 +431,17 @@ def _mlp_desc(segments, layers, B, *, out=None, out_ld=None, out_col0=0, copy_se
     for i, s in enumerate(segments):
         s.fill(d.seg[i], keep)
     n_in0 = sum(s.width for s in segments)
-    engine = engine or MLP_ENGINE
-    if engine not in ("exact", "tc", "auto"):
-        raise ValueError("mlp engine must be 'exact', 'tc' or 'auto'")
-    tc = ((engine == "tc" or (engine == "auto" and B >= TC_MIN_ROWS)) and not save and PACK_WEIGHTS and n_in0 <= TC_MAX_IN
-          and all(W.shape[0] <= TC_MAX_WIDTH for W, _, _ in layers))
     d.n_layers = len(layers)
     prev = n_in0
     dev = None
+    Ws = []
     for i, (W, b, act) in enumerate(layers):
         W, b = _f32(W, "weight"), _f32(b, "bias")
         dev = W.device
         d.layer[i].W, d.layer[i].b = W.data_ptr(), b.data_ptr()
         d.layer[i].n_in, d.layer[i].n_out, d.layer[i].act = W.shape[1], W.shape[0], act
         keep.extend([W, b])
-        if not save and PACK_WEIGHTS:
-            Wp = packed_weight(W, "tc" if tc else "ffma")
-            if tc:
-                d.layer[i].Wt = Wp.data_ptr()
-            else:
-                d.layer[i].Wp = Wp.data_ptr()
-            keep.append(Wp)
+        Ws.append(W)
         prev = W.shape[0]
     n_out = prev
     if out is None:
@@ -486,7 +474,27 @@ def _mlp_desc(segments, layers, B, *, out=None, out_ld=None, out_col0=0, copy_se
             res["eps"] = eo
         d.seed, d.offset = int(seed), int(offset)
         d.offset_dev = offset_dev.data_ptr() if offset_dev is not None else None
-    return d, res, keep, dev
+    return (d, keep, Ws), res, dev
+
+
+def _mlp_launch(blocks, B, dev):
+    """One launch of one or two blocks from _mlp_desc under MLP_ENGINE: the library plans which kernel runs them, every
+    layer gets the weight image that kernel reads, then the same call launches it."""
+    lib, engine = L.load(), _MLP_POLICY[MLP_ENGINE]
+    descs = [ctypes.byref(d) for d, _, _ in blocks]
+    with torch.cuda.device(dev):
+        kernel = ctypes.c_int()
+        L.check(lib.pcv_mlp_plan(descs[0], descs[1] if len(descs) > 1 else None, int(B), engine, ctypes.byref(kernel)),
+                "pcv_mlp_plan")
+        if kernel.value != L.MLP_KERNEL_STREAM:
+            field, kind = ("Wt", "tc") if kernel.value == L.MLP_KERNEL_TC else ("Wp", "ffma")
+            for d, keep, Ws in blocks:
+                for i, W in enumerate(Ws):
+                    keep.append(packed_weight(W, kind))
+                    setattr(d.layer[i], field, keep[-1].data_ptr())
+        name = "pcv_mlp_fwd" if len(descs) == 1 else "pcv_mlp_fwd2"
+        with _timed(name[4:]):
+            L.check(getattr(lib, name)(*descs, int(B), engine, _stream()), name)
 
 
 def mlp_forward(segments, layers, B, **kw):
@@ -495,20 +503,18 @@ def mlp_forward(segments, layers, B, **kw):
     segments: list of Dense/OneHot/Gather; layers: list of (W[n_out,n_in], b[n_out], act).
     Returns dict(out=..., z=..., eps=..., x0=..., acts=[...]) (entries present when requested).
     """
-    d, res, keep, dev = _mlp_desc(segments, layers, B, **kw)
-    with torch.cuda.device(dev), _timed("mlp_fwd"):
-        L.check(L.load().pcv_mlp_fwd(ctypes.byref(d), int(B), _stream()), "pcv_mlp_fwd")
+    block, res, dev = _mlp_desc(segments, layers, B, **kw)
+    _mlp_launch([block], B, dev)
     return res
 
 
 def mlp_forward_chain(first, second_builder, B):
     """Two chained blocks in one launch.  first = (segments, layers, kwargs); second_builder(res_first)
     -> (segments, layers, kwargs) may reference the first block's output tensors (e.g. its z)."""
-    da, ra, ka, dev = _mlp_desc(first[0], first[1], B, **first[2])
+    block_a, ra, dev = _mlp_desc(first[0], first[1], B, **first[2])
     segs_b, layers_b, kw_b = second_builder(ra)
-    db, rb, kb, _ = _mlp_desc(segs_b, layers_b, B, **kw_b)
-    with torch.cuda.device(dev), _timed("mlp_fwd2"):
-        L.check(L.load().pcv_mlp_fwd2(ctypes.byref(da), ctypes.byref(db), int(B), _stream()), "pcv_mlp_fwd2")
+    block_b, rb, _ = _mlp_desc(segs_b, layers_b, B, **kw_b)
+    _mlp_launch([block_a, block_b], B, dev)
     return ra, rb
 
 

@@ -174,17 +174,13 @@ def test_mlp_block_bitexact(ops, B, dims):
 @pytest.mark.parametrize("dims", [(54, 256, 256, 32), (38, 64, 8), (47, 300, 512, 40), (33, 16), (62, 256, 72)])
 def test_mlp_packed_engine_bitexact(ops, B, dims):
     """Inference (save=False) runs the packed-weight TMA engine: bit-identical to the oracle and to the
-    streaming engine, also after the weights change in place (cache re-pack on the version counter)."""
+    streaming engine (save=True), also after the weights change in place (cache re-pack on the version counter)."""
     rng = np.random.default_rng(B + sum(dims))
     acts = [1] * (len(dims) - 2) + [0]
     segs, layers, x, ref = _mlp_case(ops, rng, B, dims, acts, 3)
     got = ops.mlp_forward(segs, layers, B)
     assert np.array_equal(N(got["out"]), ref)
-    ops.PACK_WEIGHTS = False
-    try:
-        plain = ops.mlp_forward(segs, layers, B)
-    finally:
-        ops.PACK_WEIGHTS = True
+    plain = ops.mlp_forward(segs, layers, B, save=True)
     assert torch.equal(got["out"], plain["out"])
     layers[0][0].mul_(0.5)                          # in-place update -> version bump -> re-pack
     h = x

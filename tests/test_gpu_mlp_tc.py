@@ -167,6 +167,41 @@ def test_mlp_tc_chain_reparam_and_copy_seg(ops):
     assert torch.equal(out[:, :8], T(piv)) and torch.allclose(out, ex, rtol=1e-4, atol=1e-5)
 
 
+def test_tc_policy_runs_blocks_it_does_not_fit_bit_exact(ops):
+    """Under "tc", a block with a 17-click one-hot and a chain whose second block is 86 wide ([z 16 | one-hot 6 |
+    user 64]) do not fit the tc engine: they run on the FFMA cluster engine, bit-identical to the oracle."""
+    rng = np.random.default_rng(17)
+    B, Z = 777, 16
+    mk = lambda o, i: (T((rng.standard_normal((o, i)) / np.sqrt(i)).astype(np.float32)), T(rng.standard_normal(o).astype(np.float32) * 0.1))
+    r17 = (rng.random((B, 17)) < 0.5).astype(np.float32)
+    layers = [mk(128, 18) + (1,), mk(8, 128) + (0,)]
+    with ops.mlp_engine("tc"):
+        out = ops.mlp_forward([ops.OneHot(T(r17))], layers, B)["out"]
+    h = oracle.condition(r17)
+    for (W, b, a) in layers:
+        h = oracle.linear(h, N(W), N(b), a)
+    assert np.array_equal(N(out), h)
+
+    r = (rng.random((B, 5)) < 0.5).astype(np.float32)
+    user = rng.standard_normal((B, 64)).astype(np.float32)
+    eps = rng.standard_normal((B, Z)).astype(np.float32)
+    pl = [mk(128, 6) + (1,), mk(2 * Z, 128) + (0,)]
+    nl = [mk(256, Z + 6 + 64) + (1,), mk(8, 256) + (0,)]
+    cond = ops.OneHot(T(r))
+    with ops.mlp_engine("tc"):
+        ra, rb = ops.mlp_forward_chain(([cond], pl, dict(latent=Z, eps=T(eps))),
+                                       lambda res: ([ops.Dense(res["z"]), cond, ops.Dense(T(user))], nl, {}), B)
+    h = oracle.condition(r)
+    for (W, b, a) in pl:
+        h = oracle.linear(h, N(W), N(b), a)
+    z = oracle.reparam(h[:, :Z], h[:, Z:], eps)
+    assert np.array_equal(N(ra["out"]), h) and np.array_equal(N(ra["z"]), z)
+    g = np.concatenate([z, oracle.condition(r), user], 1)
+    for (W, b, a) in nl:
+        g = oracle.linear(g, N(W), N(b), a)
+    assert np.array_equal(N(rb["out"]), g)
+
+
 @pytest.mark.parametrize("name", ["pivot_c1", "pivot_small", "pivot_small_nouser"])
 def test_tc_engine_recommend_matches_reference_fixtures(ops, name):
     """recommend() with the tc engine against the UNMODIFIED reference's outputs (tests/golden/make_golden.py):

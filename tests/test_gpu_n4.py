@@ -15,7 +15,7 @@ class _E:
 
 
 @pytest.mark.parametrize("tag,no_user", [("mlp_user", False), ("mlp_nouser", True)])
-@pytest.mark.parametrize("engine", ["tc3", "torch"])
+@pytest.mark.parametrize("engine", ["tc3"])
 def test_response_pretrain_step(golden, tag, no_user, engine):
     from pivotcvae_b200 import autograd as ag
     from pivotcvae_b200.env.response_model import UserResponseModel_MLP
