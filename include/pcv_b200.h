@@ -315,11 +315,13 @@ typedef struct {
   const uint32_t *bitmask; /* parity mode: [M, ceil(N/32)] bit j%32 of word j/32 = Bernoulli draw (target is OR-ed in by the kernel) */
   uint64_t seed, offset;   /* Philox mode (bitmask == NULL && keep_prob < 1)         */
   const uint64_t *offset_dev; /* optional device counter added to `offset` (CUDA-graph replays) */
-  int engine;              /* PCV_CE_ENGINE_*: EXACT (default) or TF32 (dense mask, dim 8: logits AND the gradient
-                              contraction on the tensor cores, loss ~1e-4 / dq ~1e-3 relative — the reduced-precision
-                              tolerance).  The first TF32 call on a table handle builds its transposed tile image
-                              (one-off allocation + device sync, like pcv_table_create): run it once outside any
-                              CUDA-graph capture */
+  int engine;              /* PCV_CE_ENGINE_*: EXACT (default) or TF32 (dense mask, dim 8, 16, 32, 64 or 128: logits
+                              AND the gradient contraction on the tensor cores, loss ~1e-4 / dq ~1e-3 relative — the
+                              reduced-precision tolerance; other dims return PCV_ERR_UNSUPPORTED).  The first TF32
+                              call on a table handle builds its transposed tile image (one-off allocation + device
+                              sync, like pcv_table_create): run it once outside any CUDA-graph capture.  The handle
+                              keeps that image until it is destroyed: n_rows * dim * 4 bytes (rounded up to whole
+                              tiles) at dim >= 16, twice that at dim 8 */
 } pcv_ce_mask;
 #define PCV_CE_ENGINE_EXACT 0
 #define PCV_CE_ENGINE_TF32 1
@@ -334,7 +336,7 @@ int pcv_ce_fwd_bwd(const pcv_table *t, const float *Q, const int64_t *targets,
                    pcv_stream_t stream);
 
 /* Vocab-parallel CE (SURVEY §8e): the same streaming pass over ONE row shard of the table (pcv_table_create with
- * row_offset), full-catalog soft-max only (keep_prob >= 1; engine EXACT or TF32).  rec_out: [M, 2 + dim] per-row
+ * row_offset), full-catalog soft-max only (keep_prob >= 1; engine EXACT, or TF32 at dim 8 to 128).  rec_out: [M, 2 + dim] per-row
  * partial records {m, l, acc[dim]}: m = max logit over the shard, l = sum_j e^{x_j - m}, acc = sum_j e^{x_j - m} w_j.
  * The caller all-gathers the records of the G shards (ONE collective of M * (2 + dim) floats per rank) and
  * pcv_ce_vp_merge combines them: lse = M' + log sum_g l_g e^{m_g - M'}, loss = lse - <q, w_t>,

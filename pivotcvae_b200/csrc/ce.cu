@@ -604,7 +604,7 @@ static int ce_dispatch(const Table *t, const CEPlan &p, const float *Q, const in
   return PCV_ERR_UNSUPPORTED;
 }
 
-// tensor-core engine (ce_tc.cu)
+// tensor-core engine (ce_tc2.cu)
 bool ce_tc_supported(const Table *t);
 size_t ce_tc_workspace(const Table *t, int64_t M);
 int ce_tc_launch(const Table *t, const float *Q, const int64_t *targets, int64_t M, float *part, size_t ws_bytes, cudaStream_t st);
@@ -688,7 +688,7 @@ static int ce_run(const pcv_table *th, const float *Q, const int64_t *targets, i
     rc = ce_dispatch<CE_BITMASK>(t, p, Q, targets, M, mask->bitmask, mask_words, 0, 0, nullptr, 0, part, st);
   } else if (mask->keep_prob >= 1.0 && mask->engine == PCV_CE_ENGINE_TF32) {
     if (!ce_tc_supported(t)) {
-      set_error("ce: the tf32 engine needs dim 8 and an unsharded table");
+      set_error("ce: the tf32 engine serves dims 8, 16, 32, 64 and 128 (this table has dim %d)", t->dim);
       return PCV_ERR_UNSUPPORTED;
     }
     const int n_parts = ce_tc_launch(t, Q, targets, M, part, workspace_bytes, st);

@@ -24,7 +24,8 @@ struct Table {
   int sm_count;
   // tcgen05 path: pre-swizzled (SWIZZLE_32B image) copy of W owned by the handle
   float *packed;
-  float *packed_t;   // transposed per-tile image for the CE gradient MMA (ce_tc2.cu), built on first use
+  float *packed_t;   // transposed per-tile image for the CE gradient MMA (ce_tc2.cu), built on first use; as large as
+                     // the table at D >= 16 (twice at D = 8)
   void *packed_h;    // D = 8: f16 image (8 dims + constant dimension, SWIZZLE_32B) for the f16 filter (score_select_tc.cu)
   int tmap_valid;  // 1 when the tcgen05 engine can serve this table
   float max_row_norm;  // max_j |w_j|_2 (error bound of the tf32 filter)

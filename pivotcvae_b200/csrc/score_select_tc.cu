@@ -851,7 +851,6 @@ static void tc_plan(const Table *t, int64_t M, TcPlan *p) {
   }
 }
 
-static bool tc_dim_ok(int dim) { return dim == 8 || dim == 16 || dim == 32 || dim == 64 || dim == 128; }
 bool score_select_tc_supported(const Table *t) { return tc_dim_ok(t->dim) && t->tmap_valid; }
 
 size_t score_select_tc_workspace(const Table *t, int64_t M) {

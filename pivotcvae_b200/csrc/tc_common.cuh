@@ -15,6 +15,9 @@ constexpr int TC_SW = TC_BN / TC_SLICES;             // columns per slice
 constexpr int TC_THREADS = 64 + 32 * TC_EPI_WARPS;  // warp0 TMA, warp1 MMA/TMEM, 8 epilogue warps
 constexpr uint32_t TC_TILE_BYTES = TC_BN * TC_D * 4;
 
+// embedding dims served by the tcgen05 engines (filter and cross-entropy): 1, 2, 4, 8 or 16 k-atoms of 8 fp32
+inline bool tc_dim_ok(int dim) { return dim == 8 || dim == 16 || dim == 32 || dim == 64 || dim == 128; }
+
 __device__ __forceinline__ uint32_t smem_u32(const void *p) { return (uint32_t)__cvta_generic_to_shared(p); }
 
 __device__ __forceinline__ void mbar_init(void *bar, uint32_t count) {

@@ -66,7 +66,7 @@ class BaseCVAE(nn.Module):
         # sampled pivots without caller-supplied noise: "rejection" = exact O(1)-per-row sampler (csrc/sampler.cu),
         # "race" = the exponential race over the whole catalog with in-kernel Philox noise (O(N) per row)
         self.pivot_sampler = "rejection"
-        self.ce_engine = "exact"   # "tf32": full-catalog CE logits on the tensor cores (reduced-precision tolerance)
+        self.ce_engine = "exact"   # "tf32": full-catalog CE logits and gradient on the tensor cores, D = 8..128 (reduced-precision tolerance)
         # Opt-in extension, OFF by default because the reference has no such logic (SURVEY F1: cvae.py:97-101 picks
         # every slot independently, duplicates allowed).  True: a slot never repeats an item an earlier slot of
         # the same slate took (sequential arg-max without replacement; include/pcv_b200.h pcv_slate_no_repeat).
