@@ -94,7 +94,9 @@ typedef struct {
                          allowed (cvae.py:97-101; SURVEY F1).  L > 0 (opt-in extension, greedy mode, L <= 16, M % L == 0):
                          rows are the L consecutive slots of M/L slates and slot l takes its best item that slots
                          0..l-1 of the same slate have not taken (pcv_slate_no_repeat runs after the top-1 pass; the
-                         workspace must then hold pcv_score_select_workspace_bytes + pcv_score_topk_workspace_bytes) */
+                         workspace must then hold pcv_score_select_workspace_bytes + pcv_score_topk_workspace_bytes).
+                         A row shard (row_offset > 0) runs the select without it and then the sharded pair
+                         pcv_slate_no_repeat_partials + pcv_slate_no_repeat_merge */
   const uint64_t *offset_dev; /* optional DEVICE counter added to `offset` at run time, so a
                                  captured CUDA graph draws fresh noise on every replay  */
 } pcv_select_opts;
@@ -140,6 +142,21 @@ int pcv_score_topk(const pcv_table *t, const float *Q, int64_t M, int k, int64_t
  * top-L, one pass).  Workspace: pcv_score_topk_workspace_bytes(t, B*L).  The table must be the whole catalog. */
 int pcv_slate_no_repeat(const pcv_table *t, const float *Q, int64_t B, int L, int64_t *items, float *vals,
                         void *workspace, size_t workspace_bytes, pcv_stream_t stream);
+/* The same selection on a vocab-parallel catalog: every rank runs the partials on its shard, the caller all-gathers
+ * the [B*L, L] keys of the G ranks (one collective), and every rank runs the merge.  Neither call syncs the host or
+ * allocates, so both can be captured in a CUDA graph.
+ * Shard half.  shard: any row shard (row_offset allowed, n_rows may be < L).  Q: [B*L, dim] slot queries (the whole
+ * batch, identical on every rank), items: [B*L] the GLOBAL top-1 picks (identical on every rank, i.e. after the
+ * vocab-parallel merge).  For every slate whose picks hold a duplicate, writes this shard's exact top-L of each of its
+ * L rows into keys[row * L + e] (e = 0..L-1, best first), as order-preserving int64 keys (the pcv_vp_pack_keys
+ * encoding, global index).  Missing entries (shard smaller than L) and all rows of duplicate-free slates hold
+ * INT64_MIN.  Workspace: pcv_score_topk_workspace_bytes(shard, B*L). */
+int pcv_slate_no_repeat_partials(const pcv_table *shard, const float *Q, int64_t B, int L, const int64_t *items,
+                                 int64_t *keys, void *workspace, size_t workspace_bytes, pcv_stream_t stream);
+/* keys: [G, B*L, L] the partials of the G shards in shard order (G <= 32).  Re-selects the slates of `items` that hold a
+ * duplicate, in place, exactly as pcv_slate_no_repeat does on the whole catalog; vals (optional) gets the winning scores. */
+int pcv_slate_no_repeat_merge(const int64_t *keys, int G, int64_t B, int L, int64_t *items, float *vals,
+                              pcv_stream_t stream);
 /* Vocab-parallel merge (SURVEY §8e): vals/idx are [G, M] partials gathered from G
  * shards in shard order; winner = max val, ties -> lowest global index. */
 int pcv_vp_merge_select(const float *vals, const int64_t *idx, int G, int64_t M,

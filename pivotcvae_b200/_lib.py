@@ -95,6 +95,9 @@ EXPORTS = {
     "pcv_score_topk_workspace_bytes": (c_int, [c_void_p, c_int64, ctypes.POINTER(c_size_t)]),
     "pcv_score_topk": (c_int, [c_void_p, c_void_p, c_int64, c_int, c_void_p, c_void_p, c_void_p, c_size_t, c_void_p]),
     "pcv_slate_no_repeat": (c_int, [c_void_p, c_void_p, c_int64, c_int, c_void_p, c_void_p, c_void_p, c_size_t, c_void_p]),
+    "pcv_slate_no_repeat_partials": (c_int, [c_void_p, c_void_p, c_int64, c_int, c_void_p, c_void_p, c_void_p, c_size_t,
+                                             c_void_p]),
+    "pcv_slate_no_repeat_merge": (c_int, [c_void_p, c_int, c_int64, c_int, c_void_p, c_void_p, c_void_p]),
     "pcv_vp_merge_select": (c_int, [c_void_p, c_void_p, c_int, c_int64, c_void_p, c_void_p, c_void_p]),
     "pcv_sigmoid_categorical": (c_int, [c_void_p, c_void_p, c_int64, c_uint64, c_uint64, c_void_p, c_void_p, c_void_p, c_void_p]),
     "pcv_vp_pack_keys": (c_int, [c_void_p, c_void_p, c_int64, c_void_p, c_void_p]),

@@ -174,6 +174,25 @@ __device__ __forceinline__ float warp_sum(float v) {
 __device__ __forceinline__ bool better(float v, int64_t i, float bv, int64_t bi) {
   return (v > bv) || (v == bv && i < bi);
 }
+
+// Order-preserving int64 key of a (score, global index < 2^32) pair: key = (order-preserving float bits << 32) |
+// (0xffffffff - index), top bit flipped, so that the SIGNED 64-bit maximum is the better pair of `better` (largest
+// value, equal values -> lowest index).  -0 is packed as +0 so that equal scores compare equal.  No score packs to
+// PCV_KEY_NONE (it would be a NaN), which marks an empty list entry.
+constexpr long long PCV_KEY_NONE = (long long)0x8000000000000000ull;
+__device__ __forceinline__ long long pcv_pack_key(float v, int64_t idx) {
+  uint32_t b = __float_as_uint(v + 0.0f);
+  b = (b & 0x80000000u) ? ~b : (b | 0x80000000u);
+  const unsigned long long k = ((unsigned long long)b << 32) | (uint32_t)(0xffffffffu - (uint32_t)idx);
+  return (long long)(k ^ 0x8000000000000000ull);
+}
+__device__ __forceinline__ float pcv_unpack_key(long long key, int64_t &idx) {
+  const unsigned long long k = (unsigned long long)key ^ 0x8000000000000000ull;
+  uint32_t b = (uint32_t)(k >> 32);
+  b = (b & 0x80000000u) ? (b & 0x7fffffffu) : ~b;
+  idx = (int64_t)(0xffffffffu - (uint32_t)k);
+  return __uint_as_float(b);
+}
 #endif
 
 }  // namespace pcv

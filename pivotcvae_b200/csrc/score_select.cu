@@ -287,29 +287,23 @@ __global__ void vp_merge_kernel(const float *__restrict__ vals, const int64_t *_
   if (out_val) out_val[i] = v;
 }
 
-// Vocab-parallel exchange as ONE all-reduce(MAX) on int64 keys: key = (order-preserving float bits << 32) |
-// (0xffffffff - global index), top bit flipped so that the SIGNED 64-bit maximum is: largest value first,
-// equal values -> lowest global index (the reference's tie rule, SURVEY F2).
+// Vocab-parallel exchange as ONE all-reduce(MAX) on int64 keys (pcv_pack_key): the signed maximum over the shards
+// is the largest value, equal values -> lowest global index (the reference's tie rule, SURVEY F2).
 __global__ void vp_pack_keys_kernel(const float *__restrict__ vals, const int64_t *__restrict__ idx, int64_t M,
                                     long long *__restrict__ keys) {
   int64_t i = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
   if (i >= M) return;
-  const float v = vals[i] + 0.0f;   // -0 -> +0: equal scores must compare equal
-  uint32_t b = __float_as_uint(v);
-  b = (b & 0x80000000u) ? ~b : (b | 0x80000000u);
-  const unsigned long long k = ((unsigned long long)b << 32) | (uint32_t)(0xffffffffu - (uint32_t)idx[i]);
-  keys[i] = (long long)(k ^ 0x8000000000000000ull);
+  keys[i] = pcv_pack_key(vals[i], idx[i]);
 }
 
 __global__ void vp_unpack_keys_kernel(const long long *__restrict__ keys, int64_t M, int64_t *__restrict__ out_idx,
                                       float *__restrict__ out_val) {
   int64_t i = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
   if (i >= M) return;
-  const unsigned long long k = (unsigned long long)keys[i] ^ 0x8000000000000000ull;
-  uint32_t b = (uint32_t)(k >> 32);
-  b = (b & 0x80000000u) ? (b & 0x7fffffffu) : ~b;
-  out_idx[i] = (int64_t)(0xffffffffu - (uint32_t)k);
-  if (out_val) out_val[i] = __uint_as_float(b);
+  int64_t ix;
+  const float v = pcv_unpack_key(keys[i], ix);
+  out_idx[i] = ix;
+  if (out_val) out_val[i] = v;
 }
 
 __global__ void philox_exponential_kernel(uint64_t seed, uint64_t offset, int64_t M,

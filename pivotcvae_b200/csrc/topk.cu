@@ -10,6 +10,9 @@
 //      every other exact path, SURVEY F3);
 //   4. nr_resolve_kernel walks each flagged slate slot by slot.
 // The same kernel serves pcv_score_topk (torch.topk over the catalog, models/deterministic.py:119 in the reference).
+// On a vocab-parallel catalog the global top-L of a row is the merge of the G shards' top-L lists: each rank runs
+// steps 2-3 on its shard and writes its lists as pcv_pack_key keys by row (pcv_slate_no_repeat_partials); after an
+// all-gather, nr_merge_kernel does step 4 over the G shard lists (pcv_slate_no_repeat_merge).
 //
 // topk_kernel layout: a CTA owns 8 warps x R query rows (registers) and one contiguous split of the catalog; tiles are
 // staged with cp.async in the float4-SoA layout of score_select.cu; every lane keeps a sorted 16-entry (val, idx) list
@@ -197,31 +200,42 @@ topk_kernel(const float *__restrict__ W, int64_t n_items, const float *__restric
   }
 }
 
-// k-way merge of the per-split sorted lists of one (compact) row: lane = split (splits hold increasing index ranges).
-// Returns the e-th best in lane-uniform registers through the callback.
-template <class F>
-__device__ __forceinline__ void tk_merge_row(const float *__restrict__ part_val, const int32_t *__restrict__ part_idx,
-                                             int n_split, int64_t M, int64_t c, int k, F &&emit) {
+// The sorted lists tk_merge_row reads, as pcv_pack_key keys with global indices.
+// topk_kernel's per-split partials: (val, local idx), empty entries hold idx 0x7fffffff.
+struct TkSplitLists {
+  const float *val;
+  const int32_t *idx;
+  int64_t row_offset;
+  __device__ __forceinline__ long long operator()(size_t o) const {
+    const int32_t i = idx[o];
+    return i == 0x7fffffff ? PCV_KEY_NONE : pcv_pack_key(val[o], (int64_t)i + row_offset);
+  }
+};
+// Keys already packed (the shard lists of pcv_slate_no_repeat_partials).
+struct TkKeyLists {
+  const long long *keys;
+  __device__ __forceinline__ long long operator()(size_t o) const { return keys[o]; }
+};
+
+// k-way merge of sorted lists of `len` entries, one lane per list: list g of row `row` starts at
+// g * list_stride + row * len.  The lists hold disjoint items (catalog splits or shards), so keys are unique and
+// exactly one lane pops per round.  Emits the e-th best key (PCV_KEY_NONE past the end) lane-uniformly.
+template <class Lists, class F>
+__device__ __forceinline__ void tk_merge_row(const Lists &lists, int n_lists, size_t list_stride, int64_t row, int len,
+                                             int k, F &&emit) {
   const int lane = threadIdx.x & 31;
   int cur = 0;
   for (int e = 0; e < k; ++e) {
-    float hv = -INFINITY;
-    int32_t hi = 0x7fffffff;
-    if (lane < n_split && cur < TK_MAX) {
-      const size_t o = (((size_t)lane * M + c) * TK_MAX) + cur;
-      hv = part_val[o];
-      hi = part_idx[o];
-    }
-    float bv = hv;
-    int32_t bi = hi;
+    const long long head = (lane < n_lists && cur < len) ? lists((size_t)lane * list_stride + (size_t)row * len + cur)
+                                                         : PCV_KEY_NONE;
+    long long best = head;
 #pragma unroll
     for (int o = 16; o > 0; o >>= 1) {
-      const float ov = __shfl_xor_sync(0xffffffffu, bv, o);
-      const int32_t oi = __shfl_xor_sync(0xffffffffu, bi, o);
-      if (ov > bv || (ov == bv && oi < bi)) { bv = ov; bi = oi; }
+      const long long other = __shfl_xor_sync(0xffffffffu, best, o);
+      best = other > best ? other : best;
     }
-    if (bi == hi && bi != 0x7fffffff) ++cur;
-    emit(e, bv, bi);
+    if (best == head && best != PCV_KEY_NONE) ++cur;
+    emit(e, best);
   }
 }
 
@@ -231,30 +245,64 @@ __global__ void topk_finalize_kernel(const float *__restrict__ part_val, const i
   const int64_t row = (int64_t)blockIdx.x * (blockDim.x >> 5) + (threadIdx.x >> 5);
   if (row >= M) return;
   const int lane = threadIdx.x & 31;
-  tk_merge_row(part_val, part_idx, n_split, M, row, k, [&](int e, float bv, int32_t bi) {
+  tk_merge_row(TkSplitLists{part_val, part_idx, row_offset}, n_split, (size_t)M * TK_MAX, row, TK_MAX, k,
+               [&](int e, long long key) {
     if (lane == 0) {
-      out_idx[row * k + e] = bi == 0x7fffffff ? (int64_t)-1 : (int64_t)bi + row_offset;   // -1: fewer than k items
-      if (out_val) out_val[row * k + e] = bv;
+      int64_t ix;
+      const float v = pcv_unpack_key(key, ix);
+      out_idx[row * k + e] = key == PCV_KEY_NONE ? (int64_t)-1 : ix;   // -1: fewer than k items
+      if (out_val) out_val[row * k + e] = key == PCV_KEY_NONE ? -INFINITY : v;
     }
   });
 }
 
-// ---- no-repeat: flag the slates that hold a duplicate and list their rows (slot order kept)
+// ---- no-repeat
+// slate b holds a duplicate among its picks
+__device__ __forceinline__ bool nr_has_dup(const int64_t *__restrict__ items, int64_t b, int L) {
+  for (int l = 1; l < L; ++l)
+    for (int m = 0; m < l; ++m)
+      if (items[b * L + l] == items[b * L + m]) return true;
+  return false;
+}
+
+// flag the slates that hold a duplicate and list their rows (slot order kept)
 __global__ void nr_flag_kernel(const int64_t *__restrict__ items, int64_t B, int L, unsigned int *__restrict__ n_rows_dev,
                                int32_t *__restrict__ rows) {
   const int64_t b = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
   if (b >= B) return;
-  bool dup = false;
-  for (int l = 1; l < L && !dup; ++l)
-    for (int m = 0; m < l; ++m)
-      if (items[b * L + l] == items[b * L + m]) { dup = true; break; }
-  if (dup) {
+  if (nr_has_dup(items, b, L)) {
     const unsigned int pos = atomicAdd(n_rows_dev, (unsigned int)L);
     for (int l = 0; l < L; ++l) rows[pos + l] = (int32_t)(b * L + l);
   }
 }
 
-// one warp per flagged slate: merge the top-L lists of its rows slot by slot, skipping what earlier slots took
+// Slot-by-slot resolve of one slate by one warp: merge_row(l, emit) streams slot l's candidates best first as keys;
+// slot l takes the first whose item slots 0..l-1 have not taken, and take(l, item, val) stores it.
+template <class MergeRow, class Take>
+__device__ __forceinline__ void nr_resolve_slate(int L, MergeRow &&merge_row, Take &&take) {
+  int64_t taken[TK_MAX];
+#pragma unroll
+  for (int e = 0; e < TK_MAX; ++e) taken[e] = -1;
+  for (int l = 0; l < L; ++l) {
+    bool done = false;
+    merge_row(l, [&](int e, long long key) {
+      if (done || key == PCV_KEY_NONE) return;
+      int64_t item;
+      const float v = pcv_unpack_key(key, item);
+      bool used = false;
+#pragma unroll
+      for (int m = 0; m < TK_MAX; ++m) used |= (m < l && taken[m] == item);
+      if (!used) {
+        done = true;
+#pragma unroll
+        for (int m = 0; m < TK_MAX; ++m) if (m == l) taken[m] = item;
+        take(l, item, v);
+      }
+    });
+  }
+}
+
+// one warp per flagged slate: the top-L lists of its rows come from the catalog splits of this table
 __global__ void nr_resolve_kernel(const float *__restrict__ part_val, const int32_t *__restrict__ part_idx, int n_split,
                                   int64_t M, int L, int64_t row_offset, const int32_t *__restrict__ rows,
                                   unsigned int *__restrict__ n_rows_dev, int64_t *__restrict__ items,
@@ -263,31 +311,59 @@ __global__ void nr_resolve_kernel(const float *__restrict__ part_val, const int3
   const int64_t n_work = min((unsigned long long)M, (unsigned long long)*n_rows_dev);
   if (s * L >= n_work) return;
   const int lane = threadIdx.x & 31;
-  int32_t taken[TK_MAX];
-#pragma unroll
-  for (int e = 0; e < TK_MAX; ++e) taken[e] = -1;
-  for (int l = 0; l < L; ++l) {
-    const int64_t c = s * L + l;
-    bool done = false;
-    tk_merge_row(part_val, part_idx, n_split, M, c, L, [&](int e, float bv, int32_t bi) {
-      if (done) return;
-      bool used = false;
-#pragma unroll
-      for (int m = 0; m < TK_MAX; ++m) used |= (m < l && taken[m] == bi);
-      if (!used) {
-        done = true;
-#pragma unroll
-        for (int m = 0; m < TK_MAX; ++m) if (m == l) taken[m] = bi;
-        if (lane == 0) {
-          items[rows[c]] = (int64_t)bi + row_offset;
-          if (vals) vals[rows[c]] = bv;
-        }
-      }
-    });
-  }
+  const TkSplitLists lists{part_val, part_idx, row_offset};
+  nr_resolve_slate(L, [&](int l, auto &&emit) { tk_merge_row(lists, n_split, (size_t)M * TK_MAX, s * L + l, TK_MAX, L, emit); },
+                   [&](int l, int64_t item, float v) {
+    if (lane == 0) {
+      items[rows[s * L + l]] = item;
+      if (vals) vals[rows[s * L + l]] = v;
+    }
+  });
 }
 
 __global__ void nr_reset_kernel(unsigned int *n_rows_dev) { *n_rows_dev = 0u; }
+
+// ---- no-repeat over a vocab-parallel catalog: shard partials + merge of the G shards' lists
+// counter reset + every key PCV_KEY_NONE (duplicate-free slates, and entries past the end of a small shard)
+__global__ void nr_partials_init_kernel(unsigned int *__restrict__ n_rows_dev, long long *__restrict__ keys, int64_t n) {
+  const int64_t i0 = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
+  if (i0 == 0) *n_rows_dev = 0u;
+  for (int64_t i = i0; i < n; i += (int64_t)gridDim.x * blockDim.x) keys[i] = PCV_KEY_NONE;
+}
+
+// one warp per compact (flagged) row: this shard's top-L, scattered to the row's own place so that the lists of all
+// ranks line up (the compact order comes from atomics and differs between ranks)
+__global__ void nr_partials_kernel(const float *__restrict__ part_val, const int32_t *__restrict__ part_idx, int n_split,
+                                   int64_t M, int L, int64_t row_offset, const int32_t *__restrict__ rows,
+                                   const unsigned int *__restrict__ n_rows_dev, long long *__restrict__ keys) {
+  const int64_t c = (int64_t)blockIdx.x * (blockDim.x >> 5) + (threadIdx.x >> 5);
+  const int64_t n_work = min((unsigned long long)M, (unsigned long long)*n_rows_dev);
+  if (c >= n_work) return;
+  const int lane = threadIdx.x & 31;
+  const int64_t row = rows[c];
+  tk_merge_row(TkSplitLists{part_val, part_idx, row_offset}, n_split, (size_t)M * TK_MAX, c, TK_MAX, L,
+               [&](int e, long long key) {
+    if (lane == 0) keys[row * L + e] = key;
+  });
+}
+
+// one warp per slate: re-detects the duplicate from the (replicated) picks, so no compaction and the same result
+// on every rank; the top-L lists of its rows come from the G shards (one lane each, shards in index order)
+__global__ void nr_merge_kernel(const long long *__restrict__ keys, int G, int64_t B, int L, int64_t *__restrict__ items,
+                                float *__restrict__ vals) {
+  const int64_t b = (int64_t)blockIdx.x * (blockDim.x >> 5) + (threadIdx.x >> 5);
+  if (b >= B || !nr_has_dup(items, b, L)) return;
+  const int lane = threadIdx.x & 31;
+  const size_t M = (size_t)B * L;
+  __syncwarp();   // every lane has read the picks before lane 0 rewrites them
+  nr_resolve_slate(L, [&](int l, auto &&emit) { tk_merge_row(TkKeyLists{keys}, G, M * L, b * L + l, L, L, emit); },
+                   [&](int l, int64_t item, float v) {
+    if (lane == 0) {
+      items[b * L + l] = item;
+      if (vals) vals[b * L + l] = v;
+    }
+  });
+}
 
 template <int D>
 static int launch_topk(const Table *t, const TKPlan &p, const float *Q, int64_t M, const int32_t *rows,
@@ -404,6 +480,61 @@ int pcv_slate_no_repeat(const pcv_table *th, const float *Q, int64_t B, int L, i
   if (rc != PCV_OK) return rc;
   nr_resolve_kernel<<<(unsigned)((B + 7) / 8), 256, 0, st>>>(pv, pi, p.n_split, M, L, t->row_offset, rows, n_rows_dev,
                                                            items, vals);
+  PCV_LAUNCH_CHECK();
+  return PCV_OK;
+}
+
+int pcv_slate_no_repeat_partials(const pcv_table *th, const float *Q, int64_t B, int L, const int64_t *items,
+                                 int64_t *keys, void *workspace, size_t workspace_bytes, pcv_stream_t stream) {
+  PCV_CHECK_ARG(th && Q && items && keys, "NULL pointer");
+  PCV_CHECK_ARG(B > 0, "B must be > 0");
+  PCV_CHECK_ARG(L >= 1 && L <= TK_MAX, "slate size must be in [1, 16]");
+  const Table *t = reinterpret_cast<const Table *>(th);
+  PCV_CHECK_ARG(t->n_rows < 0x7fffffffLL && B * L < 0x7fffffffLL, "problem too large for 32-bit row ids");
+  int rc = check_arch();
+  if (rc != PCV_OK) return rc;
+  const int64_t M = B * L;
+  size_t need = 0;
+  rc = pcv_score_topk_workspace_bytes(th, M, &need);
+  if (rc != PCV_OK) return rc;
+  if (workspace == nullptr || workspace_bytes < need) {
+    set_error("slate_no_repeat_partials: workspace too small (%zu < %zu)", workspace_bytes, need);
+    return PCV_ERR_WORKSPACE;
+  }
+  TKPlan p;
+  tk_plan(t, M, &p);
+  cudaStream_t st = (cudaStream_t)stream;
+  unsigned int *n_rows_dev = static_cast<unsigned int *>(workspace);
+  int32_t *rows = reinterpret_cast<int32_t *>(static_cast<char *>(workspace) + 256);
+  char *base = static_cast<char *>(workspace) + 256 + (((size_t)M * 4 + 255) & ~(size_t)255);
+  float *pv = reinterpret_cast<float *>(base);
+  int32_t *pi = reinterpret_cast<int32_t *>(pv + (size_t)p.n_split * M * TK_MAX);
+  long long *k = reinterpret_cast<long long *>(keys);
+  const int64_t n_keys = M * L;
+  const int64_t init_blocks = (n_keys + 255) / 256 < 1024 ? (n_keys + 255) / 256 : 1024;
+  nr_partials_init_kernel<<<(unsigned)init_blocks, 256, 0, st>>>(n_rows_dev, k, n_keys);
+  PCV_LAUNCH_CHECK();
+  if (L == 1) return PCV_OK;   // a one-item slate never repeats
+  nr_flag_kernel<<<(unsigned)((B + 255) / 256), 256, 0, st>>>(items, B, L, n_rows_dev, rows);
+  PCV_LAUNCH_CHECK();
+  rc = dispatch_topk(t, p, Q, M, rows, n_rows_dev, pv, pi, st);
+  if (rc != PCV_OK) return rc;
+  nr_partials_kernel<<<(unsigned)((M + 7) / 8), 256, 0, st>>>(pv, pi, p.n_split, M, L, t->row_offset, rows, n_rows_dev, k);
+  PCV_LAUNCH_CHECK();
+  return PCV_OK;
+}
+
+int pcv_slate_no_repeat_merge(const int64_t *keys, int G, int64_t B, int L, int64_t *items, float *vals,
+                              pcv_stream_t stream) {
+  PCV_CHECK_ARG(keys && items, "NULL pointer");
+  PCV_CHECK_ARG(B > 0, "B must be > 0");
+  PCV_CHECK_ARG(L >= 1 && L <= TK_MAX, "slate size must be in [1, 16]");
+  PCV_CHECK_ARG(G >= 1 && G <= 32, "G must be in [1, 32] (one lane per shard)");
+  PCV_CHECK_ARG(B * L < 0x7fffffffLL, "problem too large for 32-bit row ids");
+  int rc = check_arch();
+  if (rc != PCV_OK) return rc;
+  nr_merge_kernel<<<(unsigned)((B + 7) / 8), 256, 0, (cudaStream_t)stream>>>(reinterpret_cast<const long long *>(keys),
+                                                                             G, B, L, items, vals);
   PCV_LAUNCH_CHECK();
   return PCV_OK;
 }

@@ -229,15 +229,20 @@ class BaseCVAE(nn.Module):
     def get_recommended_item(self, embeddings):
         """arg-max item per row over the whole catalog (cvae.py:97-101) -> int64 (rows,)."""
         q = embeddings.reshape(-1, self.feature_size)
+        q = q.detach()
         if getattr(self, "no_repeat", False):
-            if self._vp is not None:
-                raise L.PcvError("no_repeat selection is not available in vocab-parallel mode (it needs the whole "
-                                 "catalog on the rank)")
             if q.shape[0] % self.slate_size:
                 raise L.PcvError("no_repeat: rows must be whole slates (multiple of slate_size)")
-            return ops.score_select(self.item_table(), q.detach(), "greedy", engine=self.select_engine, want_val=False,
-                                    no_repeat=self.slate_size)[0]
-        return self._select(q.detach(), "greedy")
+            if self._vp is None:
+                return ops.score_select(self.item_table(), q, "greedy", engine=self.select_engine, want_val=False,
+                                        no_repeat=self.slate_size)[0]
+            # vocab-parallel: sharded top-1, then this shard's top-L lists of the duplicate-holding slates, one
+            # all-gather of them and the same merge on every rank
+            from ..parallel import no_repeat_exchange
+            table, Ls = self.item_table(), self.slate_size
+            items = self._select(q, "greedy")
+            return no_repeat_exchange(lambda it: ops.slate_no_repeat_partials(table, q, it, Ls), items, Ls, self._vp[0])
+        return self._select(q, "greedy")
 
     def sample_encoding(self, s, r, u=None):
         """encoder only (cvae.py:103-115) -> (z_mu, z_logvar)."""

@@ -231,6 +231,42 @@ def slate_no_repeat(table, Q, items, slate_size, vals=None):
     return items
 
 
+def slate_no_repeat_partials(table, Q, items, slate_size):
+    """Shard half of the no-repeat selection on a vocab-parallel catalog: for the slates of `items` ([B*L] GLOBAL top-1
+    picks) that hold a duplicate, this shard's top-L of each row -> int64 [B*L, L] keys (include/pcv_b200.h)."""
+    Q, items = _f32(Q, "Q"), _i64(items, "items")
+    M, D = Q.shape
+    if D != table.dim:
+        raise L.PcvError("Q has dim %d, table has dim %d" % (D, table.dim))
+    if M % slate_size or items.numel() != M:
+        raise L.PcvError("items / Q rows must be B * slate_size")
+    keys = torch.empty(M, slate_size, dtype=torch.int64, device=Q.device)
+    ws = table.workspace("topk", M)
+    with torch.cuda.device(Q.device), _timed("slate_no_repeat_partials_M%d" % M):
+        L.check(L.load().pcv_slate_no_repeat_partials(table.handle, _ptr(Q), M // slate_size, int(slate_size), _ptr(items),
+                                                      _ptr(keys), _ptr(ws), ws.numel(), _stream()),
+                "pcv_slate_no_repeat_partials")
+    return keys
+
+
+def slate_no_repeat_merge(keys, items, slate_size, vals=None):
+    """In place: re-select the duplicate-holding slates of `items` from keys [G, B*L, L], the partials of the G shards
+    in shard order; the result equals slate_no_repeat on the whole catalog."""
+    keys = _i64(keys, "keys")
+    if not items.is_cuda or items.dtype != torch.int64 or not items.is_contiguous():
+        raise L.PcvError("items must be a contiguous int64 CUDA tensor (it is updated in place)")
+    if vals is not None and (not vals.is_cuda or vals.dtype != torch.float32 or not vals.is_contiguous()
+                             or vals.numel() != items.numel()):
+        raise L.PcvError("vals must be a contiguous float32 CUDA tensor like items (it is updated in place)")
+    M = items.numel()
+    if keys.dim() != 3 or tuple(keys.shape[1:]) != (M, slate_size) or M % slate_size:
+        raise L.PcvError("keys must be [G, B * slate_size, slate_size]")
+    with torch.cuda.device(items.device), _timed("slate_no_repeat_merge_M%d" % M):
+        L.check(L.load().pcv_slate_no_repeat_merge(_ptr(keys), keys.shape[0], M // slate_size, int(slate_size),
+                                                   _ptr(items), _ptr(vals), _stream()), "pcv_slate_no_repeat_merge")
+    return items
+
+
 def sigmoid_categorical(table, Q, seed=0, offset=0, offset_dev=None, want_iters=False):
     """idx[i] ~ Categorical(sigmoid(Q[i] . W^T)) over the whole catalog, exact rejection sampler (csrc/sampler.cu)."""
     Q = _f32(Q, "Q")

@@ -10,7 +10,9 @@ Two ways the path shards, both one process per GPU over torch.distributed:
   step merges the per-row partial winners (val f32, global idx) with the reference's
   tie rule (largest value, equal values -> lowest global index): on GPUs an
   all-reduce(MAX) of order-preserving int64 keys, on the gloo test path an
-  all-gather + merge.
+  all-gather + merge.  The opt-in no-repeat selection adds one all-gather of
+  every shard's top-L lists for the slates whose picks repeat an item
+  (no_repeat_exchange).
 
 The host logic here is backend-agnostic so that the gloo/CPU tests can exercise the
 exchange + merge with a stand-in local scorer.
@@ -111,6 +113,51 @@ class VocabParallelSelector:
         idxs = out[:, 1].contiguous()
         merge = self.merge or merge_partials
         return merge(vals.contiguous(), idxs)
+
+
+def no_repeat_exchange(local_partials, items, L, group=None, merge=None):
+    """Vocab-parallel no-repeat selection, in place on `items` ([B*L] global top-1 picks, identical on every rank).
+
+    local_partials(items) -> int64 [B*L, L] this rank's shard lists (ops.slate_no_repeat_partials on a B200).  ONE
+    all-gather of them (B*L*L*8 bytes per rank, capturable in a CUDA graph), then every rank runs the same merge:
+    ops.slate_no_repeat_merge on CUDA tensors, merge_no_repeat_partials otherwise."""
+    keys = local_partials(items).contiguous()
+    world = dist.get_world_size(group)
+    gathered = torch.empty((world * keys.shape[0], keys.shape[1]), dtype=keys.dtype, device=keys.device)
+    dist.all_gather_into_tensor(gathered, keys, group=group)
+    if merge is None:
+        if keys.is_cuda:
+            from . import ops
+            merge = ops.slate_no_repeat_merge
+        else:
+            merge = merge_no_repeat_partials
+    return merge(gathered.view(world, keys.shape[0], keys.shape[1]), items, L)
+
+
+KEY_NONE = -(1 << 63)   # empty entry of a shard list (include/pcv_b200.h pcv_slate_no_repeat_partials)
+
+
+def merge_no_repeat_partials(keys, items, L):
+    """keys: [G, B*L, L] shard lists of order-preserving int64 keys (larger key = larger score, equal scores -> lower
+    global index; index = 0xffffffff - low 32 bits).  In place on `items`: every slate holding a duplicate is
+    re-selected slot by slot, slot l taking its best item slots 0..l-1 have not taken.  Pure torch restatement of
+    pcv_slate_no_repeat_merge for the CPU / gloo tests."""
+    G, M, _ = keys.shape
+    sl = items.view(-1, L)
+    for b in range(sl.shape[0]):
+        if len(set(sl[b].tolist())) == L:
+            continue
+        taken = []
+        for l in range(L):
+            cand = keys[:, b * L + l].reshape(-1)
+            cand = cand[cand != KEY_NONE].sort(descending=True).values
+            for k in cand.tolist():
+                j = 0xffffffff - (k & 0xffffffff)
+                if j not in taken:
+                    taken.append(j)
+                    sl[b, l] = j
+                    break
+    return items
 
 
 def shard_table(ops, weight, group=None):
