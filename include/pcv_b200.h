@@ -30,7 +30,7 @@
 extern "C" {
 #endif
 
-#define PCV_ABI_VERSION 2
+#define PCV_ABI_VERSION 3
 
 #define PCV_OK 0
 #define PCV_ERR_ARG (-1)
@@ -73,10 +73,11 @@ int pcv_normalize_rows(const float *W, int64_t n_rows, int dim, float *out,
 /* ------------------------------------------------------------------ */
 /* Fused score + select over the catalog                               */
 /*   greedy : cvae.py:97-101 (get_recommended_item), pivotcvae.py:191  */
-/*   exprace: pivotcvae.py:349-351,389-391 (Categorical(sigmoid(.)))   */
+/*   exprace: pivotcvae.py:389-391, parity mode (Exp(1) noise from     */
+/*            the caller); throughput: pcv_sigmoid_categorical         */
 /* ------------------------------------------------------------------ */
-#define PCV_SELECT_GREEDY 0  /* argmax_j <q, w_j>, ties -> lowest j               */
-#define PCV_SELECT_EXPRACE 1 /* argmax_j sigmoid(<q, w_j>) / E_j, E_j ~ Exp(1)     */
+#define PCV_SELECT_GREEDY 0  /* argmax_j <q, w_j>, ties -> lowest j                 */
+#define PCV_SELECT_EXPRACE 1 /* argmax_j sigmoid(<q_i, w_j>) / noise[i, j]          */
 
 #define PCV_ENGINE_AUTO 0
 #define PCV_ENGINE_SIMT 1    /* exact fp32 FMA chain on CUDA cores                  */
@@ -87,9 +88,7 @@ int pcv_normalize_rows(const float *W, int64_t n_rows, int dim, float *out,
 typedef struct {
   int mode;           /* PCV_SELECT_*                                              */
   int engine;         /* PCV_ENGINE_*                                              */
-  const float *noise; /* exprace: [M, n_rows] Exp(1) draws (parity mode) or NULL   */
-  uint64_t seed;      /* exprace with noise==NULL: Philox4x32-10 key               */
-  uint64_t offset;    /* Philox stream offset (added to the row counter word)      */
+  const float *noise; /* exprace: [M, n_rows] Exp(1) draws, required; greedy: NULL */
   int no_repeat;      /* 0 (default) = the reference's behaviour: independent per-row arg-max, duplicates inside a slate
                          allowed (cvae.py:97-101; SURVEY F1).  L > 0 (opt-in extension, greedy mode, L <= 16, M % L == 0):
                          rows are the L consecutive slots of M/L slates and slot l takes its best item that slots
@@ -97,8 +96,6 @@ typedef struct {
                          workspace must then hold pcv_score_select_workspace_bytes + pcv_score_topk_workspace_bytes).
                          A row shard (row_offset > 0) runs the select without it and then the sharded pair
                          pcv_slate_no_repeat_partials + pcv_slate_no_repeat_merge */
-  const uint64_t *offset_dev; /* optional DEVICE counter added to `offset` at run time, so a
-                                 captured CUDA graph draws fresh noise on every replay  */
 } pcv_select_opts;
 
 /* The workspace must be ZERO-FILLED once when it is allocated (the tcgen05 engine keeps a few
@@ -114,17 +111,13 @@ int pcv_score_select(const pcv_table *t, const float *Q, int64_t M,
  * out[M, n_rows] = Q @ W^T, exact fp32 sequential-k FMA chain. */
 int pcv_score_logits(const pcv_table *t, const float *Q, int64_t M, float *out,
                      pcv_stream_t stream);
-/* Materialise the Exp(1) draws the fused exprace kernel uses for (seed, offset):
- * out[M, n_rows]; test hook for the Philox path. */
-int pcv_philox_exponential(uint64_t seed, uint64_t offset, int64_t M, int64_t n_cols,
-                           int64_t col_offset, float *out, pcv_stream_t stream);
 /* Throughput-mode sampled pivot (pivotcvae.py:349-351 and the other *_spi / spt / sgt variants):
  * out_idx[i] ~ Categorical(sigmoid(<q_i, w_j>) / sum_j) over the WHOLE catalog, drawn exactly by rejection
  * (uniform proposal, accept with sigmoid(s_j) / sigmoid(|q_i| max_j|w_j|)): ~2 proposals per row instead of one
  * exponential per (row, item).  Philox4x32-10(seed, row + offset [+ *offset_dev]); every operation is portable
  * IEEE, so the oracle reproduces the draws bit for bit.  The table must be the full catalog (row_offset 0).
  * out_iters (optional): proposals used per row, -1 = inverse-CDF fallback after 1024 rejections.
- * Parity mode (caller-supplied torch noise) stays pcv_score_select(PCV_SELECT_EXPRACE, noise). */
+ * Parity mode (caller-supplied torch noise) is pcv_score_select(PCV_SELECT_EXPRACE, noise). */
 int pcv_sigmoid_categorical(const pcv_table *t, const float *Q, int64_t M, uint64_t seed, uint64_t offset,
                             const uint64_t *offset_dev, int64_t *out_idx, int32_t *out_iters,
                             pcv_stream_t stream);
@@ -157,12 +150,8 @@ int pcv_slate_no_repeat_partials(const pcv_table *shard, const float *Q, int64_t
  * duplicate, in place, exactly as pcv_slate_no_repeat does on the whole catalog; vals (optional) gets the winning scores. */
 int pcv_slate_no_repeat_merge(const int64_t *keys, int G, int64_t B, int L, int64_t *items, float *vals,
                               pcv_stream_t stream);
-/* Vocab-parallel merge (SURVEY §8e): vals/idx are [G, M] partials gathered from G
- * shards in shard order; winner = max val, ties -> lowest global index. */
-int pcv_vp_merge_select(const float *vals, const int64_t *idx, int G, int64_t M,
-                        int64_t *out_idx, float *out_val, pcv_stream_t stream);
-/* The same merge as ONE all-reduce: keys[i] = int64 whose SIGNED maximum over the shards is the winner
- * (largest value, equal values -> lowest global index < 2^32).  The caller runs
+/* Vocab-parallel merge (SURVEY §8e) of the per-shard winners of pcv_score_select as ONE all-reduce: keys[i] = int64
+ * whose SIGNED maximum over the shards is the winner (largest value, equal values -> lowest global index < 2^32).  The caller runs
  * all_reduce(keys, MAX) (NCCL, int64) between pack and unpack; nothing else crosses NVLink. */
 int pcv_vp_pack_keys(const float *vals, const int64_t *idx, int64_t M, int64_t *keys, pcv_stream_t stream);
 int pcv_vp_unpack_keys(const int64_t *keys, int64_t M, int64_t *out_idx, float *out_val, pcv_stream_t stream);

@@ -86,12 +86,6 @@ def philox4x32_10(ctr, key):
     return o
 
 
-def exprace_uniform(seed, offset, M, n_cols, col_offset=0):
-    u = np.empty((M, n_cols), dtype=np.float32)
-    lib().orc_exprace_uniform(U64(seed), U64(offset), I64(M), I64(n_cols), I64(col_offset), _p(u))
-    return u
-
-
 def bernoulli_bitmask(seed, offset, M, N, keep_prob):
     bits = np.empty((M, (N + 31) // 32), dtype=np.uint32)
     lib().orc_bernoulli_bitmask(U64(seed), U64(offset), I64(M), I64(N), ctypes.c_double(keep_prob), _p(bits))

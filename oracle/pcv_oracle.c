@@ -106,30 +106,6 @@ void orc_philox4x32_10(const uint32_t ctr[4], const uint32_t key[2], uint32_t ou
   out[0] = c0; out[1] = c1; out[2] = c2; out[3] = c3;
 }
 
-/* The library's column -> (call, component) mapping: within each 128-column block
- * lane (j & 31) makes one call whose 4 outputs serve columns blk*128 + 32*e + lane. */
-static inline uint32_t lib_word(uint64_t seed, uint64_t offset, uint32_t stream, int64_t row,
-                                int64_t jglobal) {
-  int64_t call = ((jglobal >> 7) << 5) + (jglobal & 31);
-  int e = (int)((jglobal >> 5) & 3);
-  uint64_t r = (uint64_t)row + offset;
-  uint32_t ctr[4] = {(uint32_t)call, (uint32_t)r, (uint32_t)(r >> 32), stream};
-  uint32_t key[2] = {(uint32_t)seed, (uint32_t)(seed >> 32)};
-  uint32_t o[4];
-  orc_philox4x32_10(ctr, key, o);
-  return o[e];
-}
-
-/* uniforms behind the exponential race: E = -log(u), u = ((w >> 8) + 0.5) * 2^-24 */
-void orc_exprace_uniform(uint64_t seed, uint64_t offset, int64_t M, int64_t n_cols,
-                         int64_t col_offset, float *u) {
-  for (int64_t i = 0; i < M; ++i)
-    for (int64_t j = 0; j < n_cols; ++j) {
-      uint32_t w = lib_word(seed, offset, 1u, i, j + col_offset);
-      u[i * n_cols + j] = ((float)(w >> 8) + 0.5f) * 5.9604644775390625e-8f;
-    }
-}
-
 /* Bernoulli(keep_prob) bitmask of the CE Philox mode (train_generative.py:39), bit (j & 31) of
  * word j >> 5.  The library draws it as a gap process: inside every block of 1024 consecutive
  * columns the distance to the next kept column is Geometric(keep) (memoryless => the columns are

@@ -32,8 +32,7 @@ class PcvError(RuntimeError):
 
 
 class SelectOpts(ctypes.Structure):
-    _fields_ = [("mode", c_int), ("engine", c_int), ("noise", c_void_p), ("seed", c_uint64),
-                ("offset", c_uint64), ("no_repeat", c_int), ("offset_dev", c_void_p)]
+    _fields_ = [("mode", c_int), ("engine", c_int), ("noise", c_void_p), ("no_repeat", c_int)]
 
 
 class Linear(ctypes.Structure):
@@ -91,14 +90,12 @@ EXPORTS = {
     "pcv_score_select": (c_int, [c_void_p, c_void_p, c_int64, ctypes.POINTER(SelectOpts), c_void_p,
                                  c_void_p, c_void_p, c_size_t, c_void_p]),
     "pcv_score_logits": (c_int, [c_void_p, c_void_p, c_int64, c_void_p, c_void_p]),
-    "pcv_philox_exponential": (c_int, [c_uint64, c_uint64, c_int64, c_int64, c_int64, c_void_p, c_void_p]),
     "pcv_score_topk_workspace_bytes": (c_int, [c_void_p, c_int64, ctypes.POINTER(c_size_t)]),
     "pcv_score_topk": (c_int, [c_void_p, c_void_p, c_int64, c_int, c_void_p, c_void_p, c_void_p, c_size_t, c_void_p]),
     "pcv_slate_no_repeat": (c_int, [c_void_p, c_void_p, c_int64, c_int, c_void_p, c_void_p, c_void_p, c_size_t, c_void_p]),
     "pcv_slate_no_repeat_partials": (c_int, [c_void_p, c_void_p, c_int64, c_int, c_void_p, c_void_p, c_void_p, c_size_t,
                                              c_void_p]),
     "pcv_slate_no_repeat_merge": (c_int, [c_void_p, c_int, c_int64, c_int, c_void_p, c_void_p, c_void_p]),
-    "pcv_vp_merge_select": (c_int, [c_void_p, c_void_p, c_int, c_int64, c_void_p, c_void_p, c_void_p]),
     "pcv_sigmoid_categorical": (c_int, [c_void_p, c_void_p, c_int64, c_uint64, c_uint64, c_void_p, c_void_p, c_void_p, c_void_p]),
     "pcv_vp_pack_keys": (c_int, [c_void_p, c_void_p, c_int64, c_void_p, c_void_p]),
     "pcv_vp_unpack_keys": (c_int, [c_void_p, c_int64, c_void_p, c_void_p, c_void_p]),

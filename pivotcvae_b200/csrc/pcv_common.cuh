@@ -142,22 +142,11 @@ __host__ __device__ __forceinline__ float pcv_u01(uint32_t bits) {
   return ((float)(bits >> 8) + 0.5f) * 5.9604644775390625e-8f;  // 2^-24
 }
 
-// Stream ids keep the library's Philox consumers disjoint (counter word 3).
-enum : uint32_t { PCV_STREAM_EXPRACE = 1, PCV_STREAM_NORMAL = 2, PCV_STREAM_BERNOULLI = 3 };
+// Stream ids keep the library's Philox consumers disjoint (counter word 3).  The values are part of every draw:
+// changing one changes the eps / mask noise of a given (seed, offset).
+enum : uint32_t { PCV_STREAM_NORMAL = 2, PCV_STREAM_BERNOULLI = 3 };
 
 #ifdef __CUDACC__
-// Exp(1) draw for (row, col) of the exponential race; four columns share a call.
-__device__ __forceinline__ void pcv_exp4(uint64_t seed, uint64_t offset, int64_t row,
-                                         int64_t col4, float e[4]) {
-  uint64_t r = (uint64_t)row + offset;
-  Philox4 p = philox4x32_10((uint32_t)col4, (uint32_t)r, (uint32_t)(r >> 32),
-                            PCV_STREAM_EXPRACE, (uint32_t)seed, (uint32_t)(seed >> 32));
-  e[0] = -__logf(pcv_u01(p.x));
-  e[1] = -__logf(pcv_u01(p.y));
-  e[2] = -__logf(pcv_u01(p.z));
-  e[3] = -__logf(pcv_u01(p.w));
-}
-
 __device__ __forceinline__ float warp_max(float v) {
 #pragma unroll
   for (int o = 16; o > 0; o >>= 1) v = fmaxf(v, __shfl_xor_sync(0xffffffffu, v, o));
@@ -169,15 +158,9 @@ __device__ __forceinline__ float warp_sum(float v) {
   return v;
 }
 
-// (val, idx) "better" predicate: larger value wins, equal values -> lower index
-// (torch.max first-index semantics, SURVEY F2).  Float compare, so -0 == +0.
-__device__ __forceinline__ bool better(float v, int64_t i, float bv, int64_t bi) {
-  return (v > bv) || (v == bv && i < bi);
-}
-
 // Order-preserving int64 key of a (score, global index < 2^32) pair: key = (order-preserving float bits << 32) |
-// (0xffffffff - index), top bit flipped, so that the SIGNED 64-bit maximum is the better pair of `better` (largest
-// value, equal values -> lowest index).  -0 is packed as +0 so that equal scores compare equal.  No score packs to
+// (0xffffffff - index), top bit flipped, so that the SIGNED 64-bit maximum is the better pair (largest value, equal
+// values -> lowest index: torch.max first-index semantics, SURVEY F2).  -0 is packed as +0 so that equal scores compare equal.  No score packs to
 // PCV_KEY_NONE (it would be a NaN), which marks an empty list entry.
 constexpr long long PCV_KEY_NONE = (long long)0x8000000000000000ull;
 __device__ __forceinline__ long long pcv_pack_key(float v, int64_t idx) {

@@ -24,7 +24,7 @@ constexpr int SS_WARPS = 8;
 constexpr int SS_THREADS = SS_WARPS * 32;
 constexpr int SS_TILE_FLOATS = 8192;  // 32 KB per stage
 
-enum { SS_GREEDY = 0, SS_EXPRACE_NOISE = 1, SS_EXPRACE_PHILOX = 2, SS_LOGITS = 3 };
+enum { SS_GREEDY = 0, SS_EXPRACE_NOISE = 1, SS_LOGITS = 3 };
 
 template <int D>
 struct SSCfg {
@@ -88,26 +88,12 @@ __device__ __forceinline__ void cp_async_wait() {
   asm volatile("cp.async.wait_group %0;\n" ::"n"(N));
 }
 
-// Philox call index / component for catalog column j (global index): within each
-// 128-column block, lane (j & 31) issues ONE Philox call and uses its four
-// outputs for columns blk*128 + 32*e + lane, e = 0..3.
-__device__ __forceinline__ float exprace_noise_philox(uint64_t seed, uint64_t offset,
-                                                      int64_t row, int64_t jglobal) {
-  int64_t call = ((jglobal >> 7) << 5) + (jglobal & 31);
-  int e = (int)((jglobal >> 5) & 3);
-  float ex[4];
-  pcv_exp4(seed, offset, row, call, ex);
-  return ex[e];
-}
-
 template <int D, int MODE>
 __global__ void __launch_bounds__(SS_THREADS, (D <= 32 ? 2 : 1))
-score_select_kernel(const float *__restrict__ W, int64_t n_rows, int64_t row_offset,
+score_select_kernel(const float *__restrict__ W, int64_t n_rows,
                     const float *__restrict__ Q, int64_t M, int64_t items_per_split,
-                    const float *__restrict__ noise, uint64_t seed, uint64_t offset,
-                    const uint64_t *__restrict__ offset_dev, float *__restrict__ part_val,
+                    const float *__restrict__ noise, float *__restrict__ part_val,
                     int32_t *__restrict__ part_idx, float *__restrict__ logits_out) {
-  if (MODE == SS_EXPRACE_PHILOX && offset_dev) offset += *offset_dev;
   using Cfg = SSCfg<D>;
   constexpr int R = Cfg::R, TILE = Cfg::TILE, C4 = Cfg::C4;
   extern __shared__ __align__(16) unsigned char smem_raw[];
@@ -161,72 +147,35 @@ score_select_kernel(const float *__restrict__ W, int64_t n_rows, int64_t row_off
     const float4 *cur = tile4 + (size_t)(t & 1) * C4 * TILE;
     const int64_t base = j_begin + (int64_t)t * TILE;
     const int n_valid = (int)min((int64_t)TILE, j_end - base);
-    if (MODE == SS_EXPRACE_PHILOX) {
-      // 128-column blocks: one Philox call per (row, lane) serves 4 items.
-      // (tile bases are multiples of 128 in global coordinates)
-      for (int i0 = 0; i0 < n_valid; i0 += 128) {
-        float ex[R][4];
-        const int64_t call = (((base + row_offset + i0) >> 7) << 5) + lane;
-#pragma unroll
-        for (int r = 0; r < R; ++r) pcv_exp4(seed, offset, row0 + r, call, ex[r]);
-#pragma unroll
-        for (int e = 0; e < 4; ++e) {
-          const int i = i0 + 32 * e + lane;
-          if (i < n_valid) {
-            float s[R];
-#pragma unroll
-            for (int r = 0; r < R; ++r) s[r] = 0.f;
-#pragma unroll
-            for (int c = 0; c < C4; ++c) {
-              const float4 v = cur[c * TILE + i];
-#pragma unroll
-              for (int r = 0; r < R; ++r) {
-                s[r] = fmaf(q[r][4 * c + 0], v.x, s[r]);
-                s[r] = fmaf(q[r][4 * c + 1], v.y, s[r]);
-                s[r] = fmaf(q[r][4 * c + 2], v.z, s[r]);
-                s[r] = fmaf(q[r][4 * c + 3], v.w, s[r]);
-              }
-            }
-            const int32_t j = (int32_t)(base + i);
-#pragma unroll
-            for (int r = 0; r < R; ++r) {
-              float key = -(ex[r][e] * (1.0f + pcv_expf(-s[r])));
-              if (key > best[r]) { best[r] = key; bidx[r] = j; }
-            }
-          }
-        }
-      }
-    } else {
 #pragma unroll 2
-      for (int i = lane; i < n_valid; i += 32) {
-        float s[R];
+    for (int i = lane; i < n_valid; i += 32) {
+      float s[R];
 #pragma unroll
-        for (int r = 0; r < R; ++r) s[r] = 0.f;
+      for (int r = 0; r < R; ++r) s[r] = 0.f;
 #pragma unroll
-        for (int c = 0; c < C4; ++c) {
-          const float4 v = cur[c * TILE + i];
-#pragma unroll
-          for (int r = 0; r < R; ++r) {
-            s[r] = fmaf(q[r][4 * c + 0], v.x, s[r]);
-            s[r] = fmaf(q[r][4 * c + 1], v.y, s[r]);
-            s[r] = fmaf(q[r][4 * c + 2], v.z, s[r]);
-            s[r] = fmaf(q[r][4 * c + 3], v.w, s[r]);
-          }
-        }
-        const int32_t j = (int32_t)(base + i);
+      for (int c = 0; c < C4; ++c) {
+        const float4 v = cur[c * TILE + i];
 #pragma unroll
         for (int r = 0; r < R; ++r) {
-          if (MODE == SS_LOGITS) {
-            if (row0 + r < M) logits_out[(row0 + r) * n_rows + j] = s[r];
-          } else {
-            float key = s[r];
-            if (MODE == SS_EXPRACE_NOISE) {
-              // race time T = E * (1 + exp(-s)) = E / sigmoid(s); winner = min T.
-              float e = (row0 + r < M) ? __ldg(noise + (row0 + r) * n_rows + j) : 1.f;
-              key = -(e * (1.0f + pcv_expf(-s[r])));
-            }
-            if (key > best[r]) { best[r] = key; bidx[r] = j; }
+          s[r] = fmaf(q[r][4 * c + 0], v.x, s[r]);
+          s[r] = fmaf(q[r][4 * c + 1], v.y, s[r]);
+          s[r] = fmaf(q[r][4 * c + 2], v.z, s[r]);
+          s[r] = fmaf(q[r][4 * c + 3], v.w, s[r]);
+        }
+      }
+      const int32_t j = (int32_t)(base + i);
+#pragma unroll
+      for (int r = 0; r < R; ++r) {
+        if (MODE == SS_LOGITS) {
+          if (row0 + r < M) logits_out[(row0 + r) * n_rows + j] = s[r];
+        } else {
+          float key = s[r];
+          if (MODE == SS_EXPRACE_NOISE) {
+            // race time T = E * (1 + exp(-s)) = E / sigmoid(s); winner = min T.
+            float e = (row0 + r < M) ? __ldg(noise + (row0 + r) * n_rows + j) : 1.f;
+            key = -(e * (1.0f + pcv_expf(-s[r])));
           }
+          if (key > best[r]) { best[r] = key; bidx[r] = j; }
         }
       }
     }
@@ -271,22 +220,6 @@ __global__ void select_finalize_kernel(const float *__restrict__ part_val,
   if (out_val) out_val[i] = v;
 }
 
-__global__ void vp_merge_kernel(const float *__restrict__ vals, const int64_t *__restrict__ idx,
-                                int G, int64_t M, int64_t *__restrict__ out_idx,
-                                float *__restrict__ out_val) {
-  int64_t i = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
-  if (i >= M) return;
-  float v = vals[i];
-  int64_t ix = idx[i];
-  for (int g = 1; g < G; ++g) {
-    float ov = vals[(int64_t)g * M + i];
-    int64_t oi = idx[(int64_t)g * M + i];
-    if (better(ov, oi, v, ix)) { v = ov; ix = oi; }
-  }
-  out_idx[i] = ix;
-  if (out_val) out_val[i] = v;
-}
-
 // Vocab-parallel exchange as ONE all-reduce(MAX) on int64 keys (pcv_pack_key): the signed maximum over the shards
 // is the largest value, equal values -> lowest global index (the reference's tie rule, SURVEY F2).
 __global__ void vp_pack_keys_kernel(const float *__restrict__ vals, const int64_t *__restrict__ idx, int64_t M,
@@ -306,20 +239,8 @@ __global__ void vp_unpack_keys_kernel(const long long *__restrict__ keys, int64_
   if (out_val) out_val[i] = v;
 }
 
-__global__ void philox_exponential_kernel(uint64_t seed, uint64_t offset, int64_t M,
-                                          int64_t n_cols, int64_t col_offset,
-                                          float *__restrict__ out) {
-  int64_t total = M * n_cols;
-  for (int64_t f = (int64_t)blockIdx.x * blockDim.x + threadIdx.x; f < total;
-       f += (int64_t)gridDim.x * blockDim.x) {
-    int64_t row = f / n_cols, j = f % n_cols;
-    out[f] = exprace_noise_philox(seed, offset, row, j + col_offset);
-  }
-}
-
 template <int D, int MODE>
-static int launch_ss(const Table *t, const SSPlan &p, const float *Q, int64_t M,
-                     const float *noise, uint64_t seed, uint64_t offset, const uint64_t *offset_dev,
+static int launch_ss(const Table *t, const SSPlan &p, const float *Q, int64_t M, const float *noise,
                      float *pv, int32_t *pi, float *logits, cudaStream_t st) {
   using Cfg = SSCfg<D>;
   auto kern = score_select_kernel<D, MODE>;
@@ -329,23 +250,21 @@ static int launch_ss(const Table *t, const SSPlan &p, const float *Q, int64_t M,
     attr_set[t->device & 63] = true;
   }
   dim3 grid((unsigned)p.row_tiles, (unsigned)p.n_split);
-  kern<<<grid, SS_THREADS, Cfg::SMEM, st>>>(t->W, t->n_rows, t->row_offset, Q, M,
-                                             p.items_per_split, noise, seed, offset, offset_dev, pv, pi, logits);
+  kern<<<grid, SS_THREADS, Cfg::SMEM, st>>>(t->W, t->n_rows, Q, M, p.items_per_split, noise, pv, pi, logits);
   PCV_LAUNCH_CHECK();
   return PCV_OK;
 }
 
 template <int MODE>
-static int dispatch_dim(const Table *t, const SSPlan &p, const float *Q, int64_t M,
-                        const float *noise, uint64_t seed, uint64_t offset, const uint64_t *offset_dev,
+static int dispatch_dim(const Table *t, const SSPlan &p, const float *Q, int64_t M, const float *noise,
                         float *pv, int32_t *pi, float *logits, cudaStream_t st) {
   switch (t->dim) {
-    case 4: return launch_ss<4, MODE>(t, p, Q, M, noise, seed, offset, offset_dev, pv, pi, logits, st);
-    case 8: return launch_ss<8, MODE>(t, p, Q, M, noise, seed, offset, offset_dev, pv, pi, logits, st);
-    case 16: return launch_ss<16, MODE>(t, p, Q, M, noise, seed, offset, offset_dev, pv, pi, logits, st);
-    case 32: return launch_ss<32, MODE>(t, p, Q, M, noise, seed, offset, offset_dev, pv, pi, logits, st);
-    case 64: return launch_ss<64, MODE>(t, p, Q, M, noise, seed, offset, offset_dev, pv, pi, logits, st);
-    case 128: return launch_ss<128, MODE>(t, p, Q, M, noise, seed, offset, offset_dev, pv, pi, logits, st);
+    case 4: return launch_ss<4, MODE>(t, p, Q, M, noise, pv, pi, logits, st);
+    case 8: return launch_ss<8, MODE>(t, p, Q, M, noise, pv, pi, logits, st);
+    case 16: return launch_ss<16, MODE>(t, p, Q, M, noise, pv, pi, logits, st);
+    case 32: return launch_ss<32, MODE>(t, p, Q, M, noise, pv, pi, logits, st);
+    case 64: return launch_ss<64, MODE>(t, p, Q, M, noise, pv, pi, logits, st);
+    case 128: return launch_ss<128, MODE>(t, p, Q, M, noise, pv, pi, logits, st);
   }
   set_error("score_select: dim %d unsupported (use 4, 8, 16, 32, 64 or 128)", t->dim);
   return PCV_ERR_UNSUPPORTED;
@@ -393,6 +312,8 @@ int pcv_score_select(const pcv_table *th, const float *Q, int64_t M,
   PCV_CHECK_ARG(th && Q && opts && out_idx, "NULL pointer");
   PCV_CHECK_ARG(M > 0, "M must be > 0");
   PCV_CHECK_ARG(opts->mode == PCV_SELECT_GREEDY || opts->mode == PCV_SELECT_EXPRACE, "bad mode");
+  PCV_CHECK_ARG(opts->mode != PCV_SELECT_EXPRACE || opts->noise,
+                "exprace needs the [M, n_rows] Exp(1) noise (sampled pivots without it: pcv_sigmoid_categorical)");
   const Table *t = reinterpret_cast<const Table *>(th);
   if (opts->no_repeat != 0) {
     // opt-in extension (the reference has no mask, SURVEY F1): top-1 pass on the head of the workspace, then the
@@ -444,15 +365,8 @@ int pcv_score_select(const pcv_table *th, const float *Q, int64_t M,
   float *pv = reinterpret_cast<float *>(workspace);
   int32_t *pi = reinterpret_cast<int32_t *>(pv + (size_t)p.n_split * M);
 
-  if (opts->mode == PCV_SELECT_GREEDY) {
-    rc = dispatch_dim<SS_GREEDY>(t, p, Q, M, nullptr, 0, 0, nullptr, pv, pi, nullptr, st);
-  } else if (opts->noise) {
-    rc = dispatch_dim<SS_EXPRACE_NOISE>(t, p, Q, M, opts->noise, 0, 0, nullptr, pv, pi, nullptr, st);
-  } else {
-    PCV_CHECK_ARG(t->row_offset % 128 == 0, "Philox exprace needs row_offset % 128 == 0");
-    rc = dispatch_dim<SS_EXPRACE_PHILOX>(t, p, Q, M, nullptr, opts->seed, opts->offset, opts->offset_dev,
-                                         pv, pi, nullptr, st);
-  }
+  rc = opts->mode == PCV_SELECT_GREEDY ? dispatch_dim<SS_GREEDY>(t, p, Q, M, nullptr, pv, pi, nullptr, st)
+                                       : dispatch_dim<SS_EXPRACE_NOISE>(t, p, Q, M, opts->noise, pv, pi, nullptr, st);
   if (rc != PCV_OK) return rc;
   int threads = 256;
   select_finalize_kernel<<<(unsigned)((M + threads - 1) / threads), threads, 0, st>>>(
@@ -474,22 +388,7 @@ int pcv_score_logits(const pcv_table *th, const float *Q, int64_t M, float *out,
     set_error("score_logits: dim %d unsupported", t->dim);
     return PCV_ERR_UNSUPPORTED;
   }
-  return dispatch_dim<SS_LOGITS>(t, p, Q, M, nullptr, 0, 0, nullptr, nullptr, nullptr, out,
-                                 (cudaStream_t)stream);
-}
-
-int pcv_philox_exponential(uint64_t seed, uint64_t offset, int64_t M, int64_t n_cols,
-                           int64_t col_offset, float *out, pcv_stream_t stream) {
-  PCV_CHECK_ARG(out && M > 0 && n_cols > 0, "bad arguments");
-  PCV_CHECK_ARG(col_offset % 128 == 0, "col_offset % 128 != 0");
-  int rc = check_arch();
-  if (rc != PCV_OK) return rc;
-  int64_t total = M * n_cols;
-  int blocks = (int)((total + 255) / 256 > 4096 ? 4096 : (total + 255) / 256);
-  philox_exponential_kernel<<<blocks, 256, 0, (cudaStream_t)stream>>>(seed, offset, M, n_cols,
-                                                                      col_offset, out);
-  PCV_LAUNCH_CHECK();
-  return PCV_OK;
+  return dispatch_dim<SS_LOGITS>(t, p, Q, M, nullptr, nullptr, nullptr, out, (cudaStream_t)stream);
 }
 
 int pcv_vp_pack_keys(const float *vals, const int64_t *idx, int64_t M, int64_t *keys, pcv_stream_t stream) {
@@ -510,18 +409,6 @@ int pcv_vp_unpack_keys(const int64_t *keys, int64_t M, int64_t *out_idx, float *
   if (rc != PCV_OK) return rc;
   vp_unpack_keys_kernel<<<(unsigned)((M + 255) / 256), 256, 0, (cudaStream_t)stream>>>(
       reinterpret_cast<const long long *>(keys), M, out_idx, out_val);
-  PCV_LAUNCH_CHECK();
-  return PCV_OK;
-}
-
-int pcv_vp_merge_select(const float *vals, const int64_t *idx, int G, int64_t M,
-                        int64_t *out_idx, float *out_val, pcv_stream_t stream) {
-  PCV_CHECK_ARG(vals && idx && out_idx, "NULL pointer");
-  PCV_CHECK_ARG(G >= 1 && M > 0, "bad shape");
-  int rc = check_arch();
-  if (rc != PCV_OK) return rc;
-  vp_merge_kernel<<<(unsigned)((M + 255) / 256), 256, 0, (cudaStream_t)stream>>>(vals, idx, G, M,
-                                                                                 out_idx, out_val);
   PCV_LAUNCH_CHECK();
   return PCV_OK;
 }

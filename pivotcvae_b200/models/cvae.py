@@ -63,9 +63,6 @@ class BaseCVAE(nn.Module):
                              "(every reference subclass hard-codes fine_tune=False)")
         self.noise = NoiseSource()
         self.select_engine = "auto"
-        # sampled pivots without caller-supplied noise: "rejection" = exact O(1)-per-row sampler (csrc/sampler.cu),
-        # "race" = the exponential race over the whole catalog with in-kernel Philox noise (O(N) per row)
-        self.pivot_sampler = "rejection"
         self.ce_engine = "exact"   # "tf32": full-catalog CE logits and gradient on the tensor cores, D = 8..128 (reduced-precision tolerance)
         # Opt-in extension, OFF by default because the reference has no such logic (SURVEY F1: cvae.py:97-101 picks
         # every slot independently, duplicates allowed).  True: a slot never repeats an item an earlier slot of
@@ -123,15 +120,15 @@ class BaseCVAE(nn.Module):
         return kw
 
     def _select(self, q, mode="greedy", **kw):
-        """score+select over the (possibly sharded) catalog -> global item ids int64 (rows,)."""
-        if self._vp is None:
-            return ops.score_select(self.item_table(), q, mode, engine=self.select_engine if mode == "greedy" else "auto",
-                                    want_val=False, **kw)[0]
+        """score+select over the (possibly sharded) catalog -> global item ids int64 (rows,).  While recommend() shards
+        the MLP rows (self._rows), each rank's rows are scored against the whole catalog, which every rank keeps anyway
+        (<= 320 MB), so the pick needs no exchange."""
+        engine = self.select_engine if mode == "greedy" else "auto"
+        if self._vp is None or getattr(self, "_rows", None) is not None:
+            return ops.score_select(self.full_table(), q, mode, engine=engine, want_val=False, **kw)[0]
         from ..parallel import VocabParallelSelector
-        group = self._vp[0]
-        local = lambda x: ops.score_select(self.item_table(), x, mode,
-                                           engine=self.select_engine if mode == "greedy" else "auto", **kw)
-        return VocabParallelSelector(local, group)(q)[0]
+        local = lambda x: ops.score_select(self.item_table(), x, mode, engine=engine, **kw)
+        return VocabParallelSelector(local, self._vp[0])(q)[0]
 
     def _apply(self, fn, *a, **k):
         self._table = None
@@ -243,6 +240,32 @@ class BaseCVAE(nn.Module):
             items = self._select(q, "greedy")
             return no_repeat_exchange(lambda it: ops.slate_no_repeat_partials(table, q, it, Ls), items, Ls, self._vp[0])
         return self._select(q, "greedy")
+
+    @with_mlp_engine
+    def recommend(self, r, u=None, return_item=False):
+        """prior -> z -> decoder (_generate) -> per-slot arg-max items, or the flat (B, L*D) slate features; and z_mu.
+        Vocab-parallel with shard_rows, this rank runs _generate on its B/world rows and ONE all-gather carries
+        [rx | z_mu] of every rank; the per-slot scoring then is the catalog-sharded select of _select()."""
+        with torch.no_grad():
+            r, u, _ = self._inputs(r, u)
+            B = r.shape[0]
+            sl = self._vp_row_slice(B)
+            if sl is not None:
+                _, r0, per = sl
+                r, u = r[r0:r0 + per], None if u is None else u[r0:r0 + per]
+                self._rows = (r0, B)
+            try:
+                out, rx = self._generate(r, u)
+            finally:
+                self._rows = None
+            z_mu = out[:, :self.latent_size]
+            if sl is not None:
+                from ..parallel import all_gather_rows
+                both = all_gather_rows(torch.cat([rx, z_mu], 1), self._vp[0])       # [B, L * D + Z]
+                rx, z_mu = both[:, :rx.shape[1]].contiguous(), both[:, rx.shape[1]:]
+            res = self.get_recommended_item(rx) if return_item else rx
+            self.noise.flush_eager()
+            return res, z_mu
 
     def sample_encoding(self, s, r, u=None):
         """encoder only (cvae.py:103-115) -> (z_mu, z_logvar)."""

@@ -5,7 +5,7 @@ Same as PivotCVAE minus the pivot: one decoder MLP emits all L*D slate features.
 import torch
 
 from .. import _lib as L
-from .cvae import BaseCVAE, with_mlp_engine
+from .cvae import BaseCVAE
 
 
 class UserListCVAEWithPrior(BaseCVAE):
@@ -55,30 +55,10 @@ class UserListCVAEWithPrior(BaseCVAE):
         p = self._logits(rx.view(-1, self.feature_size), candidates)
         return p, rx, z, emb, mu, lv
 
-    @with_mlp_engine
-    def recommend(self, r, u=None, return_item=False):
-        """listcvae.py:170-188."""
-        with torch.no_grad():
-            r, u, _ = self._inputs(r, u)
-            sl = self._vp_row_slice(r.shape[0])
-            if sl is not None:      # vocab-parallel with the MLP rows sharded: all-gather [rx | z_mu], sharded select
-                from ..parallel import all_gather_rows
-                world, r0, per = sl
-                self._rows = (r0, r.shape[0])
-                try:
-                    out, z, rx = self._prior_chain(r[r0:r0 + per], None if u is None else u[r0:r0 + per], self.decMLP)
-                finally:
-                    self._rows = None
-                both = all_gather_rows(torch.cat([rx, out[:, :self.latent_size]], 1), self._vp[0])
-                rx, z_mu = both[:, :rx.shape[1]].contiguous(), both[:, rx.shape[1]:]
-                res = self.get_recommended_item(rx) if return_item else rx
-                self.noise.flush_eager()
-                return res, z_mu
-            out, z, rx = self._prior_chain(r, u, self.decMLP)      # prior -> z -> decoder in one launch
-            z_mu = out[:, :self.latent_size]
-            res = self.get_recommended_item(rx) if return_item else rx
-            self.noise.flush_eager()
-            return res, z_mu
+    def _generate(self, r, u):
+        """prior -> z -> decoder in one launch -> (prior [mu | logvar], rx (B, L*D)); recommend() is listcvae.py:170-188."""
+        out, _, rx = self._prior_chain(r, u, self.decMLP)
+        return out, rx
 
     def log(self, logger):
         for k, v in (("feature size", self.feature_size), ("slate size", self.slate_size),

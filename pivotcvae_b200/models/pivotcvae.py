@@ -11,7 +11,7 @@ strings; the reference's class names are kept so pickles and imports resolve.
 import torch
 
 from .. import _lib as L
-from .cvae import BaseCVAE, with_mlp_engine
+from .cvae import BaseCVAE
 
 
 class UserPivotCVAE(BaseCVAE):
@@ -66,12 +66,10 @@ class UserPivotCVAE(BaseCVAE):
             if self._vp is not None:      # external noise is [B, N]: every shard reads its own columns
                 noise = noise[:, self._vp[1]:self._vp[2]].contiguous()
             return self._select(q, "exprace", noise=noise)
-        if self.pivot_sampler == "rejection":
-            # throughput mode: the same Categorical(sigmoid(scores)) drawn exactly in O(1) per row (csrc/sampler.cu);
-            # needs the whole catalog, which every vocab-parallel rank keeps anyway -> no collective
-            from .. import ops
-            return ops.sigmoid_categorical(self.full_table(), q, **self._stream_args(q.shape[0]))
-        return self._select(q, "exprace", **self.noise.stream_args(q.shape[0]))
+        # throughput mode: the same Categorical(sigmoid(scores)) drawn exactly in O(1) per row (csrc/sampler.cu);
+        # needs the whole catalog, which every vocab-parallel rank keeps anyway -> no collective
+        from .. import ops
+        return ops.sigmoid_categorical(self.full_table(), q, **self._stream_args(q.shape[0]))
 
     def pick_pivot(self, pivot_output, true_pivot=[]):
         return self.docEmbed.weight[self._pick_index(pivot_output, true_pivot)]
@@ -125,52 +123,16 @@ class UserPivotCVAE(BaseCVAE):
         p = self._logits(rx.view(-1, self.feature_size), candidates)
         return p, rx.view(B, self.slate_size, self.feature_size), z, emb, mu, lv
 
-    @with_mlp_engine
-    def recommend(self, r, u=None, return_item=False, random_pivot=False):
-        """prior -> z -> pivot -> slate completion -> arg-max items (pivotcvae.py:278-296)."""
-        with torch.no_grad():
-            r, u, _ = self._inputs(r, u)
-            sl = self._vp_row_slice(r.shape[0])
-            if sl is not None and (self.infer_pick == "max" or self.pivot_sampler == "rejection"):
-                return self._recommend_vp_rows(r, u, return_item, sl)
-            # prior -> z -> PSM in one launch, pivot pick, SCM, per-slot arg-max
-            out, z, pivot_output = self._prior_chain(r, u, self.psmMLP)
-            user_seg = None if self.noUser else self._user_seg(u)
-            rx = self._scm(z, ("onehot", r), self._pick_index(pivot_output, None), user_seg, [])
-            z_mu = out[:, :self.latent_size]
-            res = self.get_recommended_item(rx) if return_item else rx.view(r.shape[0], self.slate_size, self.feature_size)
-            self.noise.flush_eager()
-            return res, z_mu
+    def _generate(self, r, u):
+        """prior -> z -> PSM in one launch, pivot pick, SCM -> (prior [mu | logvar], rx (B, L*D))."""
+        out, z, pivot_output = self._prior_chain(r, u, self.psmMLP)
+        user_seg = None if self.noUser else self._user_seg(u)
+        return out, self._scm(z, ("onehot", r), self._pick_index(pivot_output, None), user_seg, [])
 
-    def _recommend_vp_rows(self, r, u, return_item, sl):
-        """Vocab-parallel recommend() with the MLP rows sharded too.  This rank runs prior -> z -> PSM -> pivot pick ->
-        SCM on its B/world rows; the pivot pick (1/(L+1) of the scoring work) is row-parallel against the whole
-        catalog, which every rank keeps anyway (<= 320 MB), so it needs no exchange — greedy and sampled alike.  ONE
-        all-gather then carries [rx | z_mu] of every rank, and the per-slot scoring (L/(L+1) of the work) is the
-        catalog-sharded select + all-reduce(MAX) of _select()."""
-        from .. import ops
-        from ..parallel import all_gather_rows
-        world, r0, per = sl
-        group = self._vp[0]
-        B, Z, D = r.shape[0], self.latent_size, self.feature_size
-        rl = r[r0:r0 + per]
-        ul = None if u is None else u[r0:r0 + per]
-        self._rows = (r0, B)
-        try:
-            out, z, pivot_output = self._prior_chain(rl, ul, self.psmMLP)
-            if self.infer_pick == "max":
-                pivot = ops.score_select(self.full_table(), pivot_output, "greedy", engine=self.select_engine, want_val=False)[0]
-            else:
-                pivot = self._pick_index(pivot_output, None)
-            user_seg = None if self.noUser else self._user_seg(ul)
-            rx_local = self._scm(z, ("onehot", rl), pivot, user_seg, [])
-        finally:
-            self._rows = None
-        both = all_gather_rows(torch.cat([rx_local, out[:, :Z]], 1), group)          # [B, L * D + Z]
-        rx, z_mu = both[:, :rx_local.shape[1]].contiguous(), both[:, rx_local.shape[1]:]
-        res = self.get_recommended_item(rx) if return_item else rx.view(B, self.slate_size, D)
-        self.noise.flush_eager()
-        return res, z_mu
+    def recommend(self, r, u=None, return_item=False, random_pivot=False):
+        """prior -> z -> pivot -> slate completion -> arg-max items, or rx as (B, L, D) (pivotcvae.py:278-296)."""
+        res, z_mu = super().recommend(r, u, return_item)
+        return (res if return_item else res.view(res.shape[0], self.slate_size, self.feature_size)), z_mu
 
     def log(self, logger):
         for k, v in (("feature size", self.feature_size), ("slate size", self.slate_size),

@@ -174,10 +174,10 @@ def counter_add(counter, inc):
         L.check(L.load().pcv_counter_add(_ptr(counter), int(inc), _stream()), "pcv_counter_add")
 
 
-def score_select(table, Q, mode="greedy", noise=None, seed=0, offset=0, engine="auto", want_val=True,
-                 offset_dev=None, no_repeat=0):
-    """-> (idx int64[M], val f32[M]).  mode 'greedy' | 'exprace'.  no_repeat=L (opt-in, NOT reference behaviour):
-    rows are the L slots of M/L slates; a slot never repeats an item an earlier slot of its slate took."""
+def score_select(table, Q, mode="greedy", noise=None, engine="auto", want_val=True, no_repeat=0):
+    """-> (idx int64[M], val f32[M]).  mode 'greedy' | 'exprace' (needs noise: [M, n_rows] Exp(1) draws).  no_repeat=L
+    (opt-in, NOT reference behaviour): rows are the L slots of M/L slates; a slot never repeats an item an earlier slot
+    of its slate took."""
     Q = _f32(Q, "Q")
     M, D = Q.shape
     if D != table.dim:
@@ -191,8 +191,7 @@ def score_select(table, Q, mode="greedy", noise=None, seed=0, offset=0, engine="
         if tuple(noise.shape) != (M, table.n_rows):
             raise L.PcvError("noise must be [M, n_rows]")
     opts.noise = noise.data_ptr() if noise is not None else None
-    opts.seed, opts.offset, opts.no_repeat = int(seed), int(offset), int(no_repeat)
-    opts.offset_dev = offset_dev.data_ptr() if offset_dev is not None else None
+    opts.no_repeat = int(no_repeat)
     idx = torch.empty(M, dtype=torch.int64, device=Q.device)
     val = torch.empty(M, dtype=torch.float32, device=Q.device) if want_val else None
     ws = table.workspace("select_nr" if no_repeat else "select", M)
@@ -287,26 +286,6 @@ def score_logits(table, Q):
     with torch.cuda.device(Q.device):
         L.check(L.load().pcv_score_logits(table.handle, _ptr(Q), Q.shape[0], _ptr(out), _stream()), "pcv_score_logits")
     return out
-
-
-def philox_exponential(seed, offset, M, n_cols, device, col_offset=0):
-    out = torch.empty(M, n_cols, dtype=torch.float32, device=device)
-    with torch.cuda.device(out.device):
-        L.check(L.load().pcv_philox_exponential(int(seed), int(offset), M, n_cols, col_offset, _ptr(out), _stream()),
-                "pcv_philox_exponential")
-    return out
-
-
-def vp_merge_select(vals, idx):
-    """vals/idx: [G, M] partial winners in shard order -> (idx[M], val[M])."""
-    vals, idx = _f32(vals, "vals"), _i64(idx, "idx")
-    G, M = vals.shape
-    oi = torch.empty(M, dtype=torch.int64, device=vals.device)
-    ov = torch.empty(M, dtype=torch.float32, device=vals.device)
-    with torch.cuda.device(vals.device):
-        L.check(L.load().pcv_vp_merge_select(_ptr(vals), _ptr(idx), G, M, _ptr(oi), _ptr(ov), _stream()),
-                "pcv_vp_merge_select")
-    return oi, ov
 
 
 def vp_pack_keys(vals, idx):

@@ -20,7 +20,7 @@ exchange + merge with a stand-in local scorer.
 import torch
 import torch.distributed as dist
 
-SHARD_ALIGN = 128  # Philox column blocks and TMA tiles stay aligned across shards
+SHARD_ALIGN = 128  # the tensor-core select's TMA tiles stay aligned across shards
 
 
 def shard_bounds(n_rows, world, rank, align=SHARD_ALIGN):
@@ -34,8 +34,8 @@ def shard_bounds(n_rows, world, rank, align=SHARD_ALIGN):
 
 def merge_partials(vals, idx):
     """vals/idx: [G, M] partial winners in shard order (torch tensors, any device).
-    Winner = largest value, equal values -> lowest global index.  Pure torch (used by the
-    CPU tests; the GPU path calls ops.vp_merge_select)."""
+    Winner = largest value, equal values -> lowest global index.  Pure torch: the merge of the
+    backend-agnostic all-gather path (gloo / CPU tests); CUDA partials merge by all-reduce(MAX) of packed keys."""
     G, M = vals.shape
     best_v, best_i = vals[0].clone(), idx[0].clone()
     for g in range(1, G):
@@ -80,20 +80,18 @@ class VocabParallelSelector:
     """score+select over a catalog sharded across the ranks of `group`.
 
     local_select(Q) -> (idx_global int64[M], val f32[M]) scores the local shard; on a B200 it is
-    ops.score_select on a Table built with row_offset=lo.  merge defaults to the CUDA merge
-    kernel when the partials live on a GPU."""
+    ops.score_select on a Table built with row_offset=lo."""
 
-    def __init__(self, local_select, group=None, merge=None):
+    def __init__(self, local_select, group=None):
         self.local_select = local_select
         self.group = group
-        self.merge = merge
 
     def __call__(self, Q):
         idx, val = self.local_select(Q)
         world = dist.get_world_size(self.group)
         if world == 1:
             return idx, val
-        if val.is_cuda and self.merge is None:
+        if val.is_cuda:
             # ONE collective per scoring step and nothing else: (val, idx) -> order-preserving int64 key,
             # all-reduce(MAX) over NVLink (in-switch where NCCL picks NVLS), key -> (idx, val).  Capturable
             # in the step's CUDA graph.
@@ -111,8 +109,7 @@ class VocabParallelSelector:
         out = flat.view(world, 2, M)
         vals = out[:, 0].to(torch.int32).view(torch.float32)
         idxs = out[:, 1].contiguous()
-        merge = self.merge or merge_partials
-        return merge(vals.contiguous(), idxs)
+        return merge_partials(vals.contiguous(), idxs)
 
 
 def no_repeat_exchange(local_partials, items, L, group=None, merge=None):

@@ -75,44 +75,26 @@ def test_select_exprace_external_noise(ops, golden, name, tag):
     assert np.array_equal(N(idx), ref["pivot"])
 
 
-def test_select_exprace_philox(ops):
-    rng = np.random.default_rng(5)
-    n_items, M, D = 5003, 77, 8
-    W = rng.standard_normal((n_items, D)).astype(np.float32)
-    W /= np.linalg.norm(W, axis=1, keepdims=True)
-    Q = rng.standard_normal((M, D)).astype(np.float32)
-    tab = ops.Table(T(W))
-    seed, off = 0x1234ABCD5678, 1000
-    E = ops.philox_exponential(seed, off, M, n_items, dev())
-    u = oracle.exprace_uniform(seed, off, M, n_items)
-    np.testing.assert_allclose(N(E), -np.log(u.astype(np.float64)), rtol=2e-6, atol=1e-7)  # integer stream exact
-    a, av = ops.score_select(tab, T(Q), "exprace", seed=seed, offset=off)
-    b, bv = ops.score_select(tab, T(Q), "exprace", noise=E)
-    assert torch.equal(a, b) and torch.equal(av, bv)          # fused Philox == external noise path
-    oi, _ = oracle.score_select(W, Q, "exprace", N(E))
-    assert np.array_equal(N(a), oi)
-    # a different offset gives different draws; the same one is reproducible
-    c, _ = ops.score_select(tab, T(Q), "exprace", seed=seed, offset=off + M)
-    assert not torch.equal(a, c)
-    d, _ = ops.score_select(tab, T(Q), "exprace", seed=seed, offset=off)
-    assert torch.equal(a, d)
-
-
-def test_exprace_is_sigmoid_categorical(ops):
+def test_exprace_with_exp1_noise_is_sigmoid_categorical(ops):
     """Distribution check: P(pick j) ∝ sigmoid(score_j) (pivotcvae.py:349-350)."""
     rng = np.random.default_rng(11)
     W = rng.standard_normal((6, 8)).astype(np.float32)
     W /= np.linalg.norm(W, axis=1, keepdims=True)
     q = (3 * W[2]).reshape(1, 8)
     M = 40000
-    idx, _ = ops.score_select(ops.Table(T(W)), T(np.repeat(q, M, 0)), "exprace", seed=99, offset=0)
+    g = torch.Generator(device=dev()).manual_seed(99)
+    E = torch.empty(M, 6, device=dev()).exponential_(generator=g)
+    idx, _ = ops.score_select(ops.Table(T(W)), T(np.repeat(q, M, 0)), "exprace", noise=E)
+    with pytest.raises(ops.L.PcvError, match="exprace needs"):    # the race draws only caller-supplied noise
+        ops.score_select(ops.Table(T(W)), T(q), "exprace")
     freq = np.bincount(N(idx), minlength=6) / M
     p = 1 / (1 + np.exp(-(W @ q[0])))
     np.testing.assert_allclose(freq, p / p.sum(), atol=0.01)
 
 
-def test_vp_merge(ops):
-    """Vocab-parallel shards + merge == one-shot (SURVEY §8e), incl. ties across shards."""
+def test_vp_merge_by_packed_key_max(ops):
+    """Vocab-parallel shards + merge == one-shot (SURVEY §8e), incl. ties across shards.  The merge is the production
+    one: packed keys, all-reduce(MAX) (here the max over the stacked shards on one device), unpack."""
     rng = np.random.default_rng(3)
     n_items, M, D, G = 4096, 100, 8, 4
     W = rng.standard_normal((n_items, D)).astype(np.float32)
@@ -123,14 +105,13 @@ def test_vp_merge(ops):
     Q[0] = W[100]
     Wd = T(W)
     full_i, full_v = ops.score_select(ops.Table(Wd), T(Q), "greedy", engine="simt")
-    vals, idxs = [], []
+    keys = []
     per = n_items // G
     for g in range(G):
         t = ops.Table(Wd[g * per:(g + 1) * per], row_offset=g * per)
         i, v = ops.score_select(t, T(Q), "greedy", engine="simt")
-        vals.append(v)
-        idxs.append(i)
-    mi, mv = ops.vp_merge_select(torch.stack(vals), torch.stack(idxs))
+        keys.append(ops.vp_pack_keys(v, i))
+    mi, mv = ops.vp_unpack_keys(torch.stack(keys).max(0).values)
     assert torch.equal(mi, full_i) and torch.equal(mv, full_v)
     assert int(mi[0]) == 100
 

@@ -137,7 +137,7 @@ def test_tc_unnormalised_table_and_zero_query(ops, tc_engine):
     assert np.array_equal(N(idx), oi) and np.array_equal(N(val), ov) and N(idx)[3] == 0
 
 
-def test_tc_full_size_properties(ops, tc_engine):
+def test_tc_full_size_properties_packed_key_merge(ops, tc_engine):
     """BASELINE C4 size (1M items, 20480 rows): shard-merge invariance, planted maxima, and the
     winning value re-derived from the returned index (no oracle run at this size)."""
     g = torch.Generator(device="cuda").manual_seed(1)
@@ -155,13 +155,12 @@ def test_tc_full_size_properties(ops, tc_engine):
     assert bool((ps.max(1).values <= val + 1e-5).all())
     G = 4
     per = n_items // G
-    vals, idxs = [], []
+    keys = []
     for s in range(G):
         t = ops.Table(W[s * per:(s + 1) * per], row_offset=s * per)
         i, v = ops.score_select(t, Q, "greedy", engine=tc_engine)
-        vals.append(v)
-        idxs.append(i)
-    mi, mv = ops.vp_merge_select(torch.stack(vals), torch.stack(idxs))
+        keys.append(ops.vp_pack_keys(v, i))
+    mi, mv = ops.vp_unpack_keys(torch.stack(keys).max(0).values)     # the all-reduce(MAX) merge, on one device
     assert torch.equal(mi, idx) and torch.equal(mv, val)
     si, sv = ops.score_select(full, Q[:2048], "greedy", engine="simt")
     assert torch.equal(si, idx[:2048]) and torch.equal(sv, val[:2048])

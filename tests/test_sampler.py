@@ -102,8 +102,8 @@ def test_gpu_sampler_fallback_and_distribution():
 
 @pytest.mark.gpu
 def test_model_sampled_pivot_uses_the_sampler_and_matches_the_oracle(golden):
-    """recommend() of a *_spi model without caller noise: pivot = the sampler's draw on the PSM output; the race
-    engine stays selectable and external noise still takes the parity path."""
+    """recommend() of a *_spi model without caller noise: pivot = the sampler's draw on the PSM output; external
+    noise still takes the parity path."""
     from gpu_util import N, T, build_pivot
     fx = golden("pivot_c1")
     m = build_pivot(fx, "pivotcvae_gt_spi")
@@ -121,12 +121,6 @@ def test_model_sampled_pivot_uses_the_sampler_and_matches_the_oracle(golden):
     rx = np.concatenate([W[pidx].reshape(cfg["B"], 1, -1), out.reshape(cfg["B"], cfg["L"] - 1, -1)], 1)
     want, _ = oracle.score_select(W, rx.reshape(-1, cfg["D"]), "greedy")
     assert np.array_equal(N(items), want)
-    m.pivot_sampler = "race"
-    m.noise.reseed(31337)
-    m.noise.push("eps", T(fx[tag + "eps"]))
-    items_race, _ = m.recommend(T(fx[tag + "ctx"]), T(fx["in/users"]), return_item=True)
-    assert items_race.shape == items.shape
-    m.pivot_sampler = "rejection"
     m.noise.push("eps", T(fx[tag + "eps"]))
     m.noise.push("race", T(fx[tag + "noise"]))
     items_par, _ = m.recommend(T(fx[tag + "ctx"]), T(fx["in/users"]), return_item=True)
