@@ -314,7 +314,8 @@ int pcv_kl_fwd_bwd(const float *mu, const float *logvar, const float *pmu,
 /* 1024-column blocks, integer inverse CDF) and visits only the kept columns:    */
 /* O(n_neg) work per row instead of O(N).                                        */
 /* (not -inf) exactly as `pred * mask` does (SURVEY F7).               */
-/* dq[i,:] = d loss_row[i] / d q_i  (the table is frozen: no dW).      */
+/* dq[i,:] = d loss_row[i] / d q_i.  The gradient w.r.t. the table is a  */
+/* second pass, pcv_ce_table_grad (fine_tune=True).                    */
 /* ------------------------------------------------------------------ */
 typedef struct {
   double keep_prob;        /* n_neg / N; >= 1 means full-catalog soft-max, no RNG    */
@@ -362,6 +363,32 @@ int pcv_ce_vp_merge(const float *recs, int G, const float *W_full, int dim, cons
 int pcv_cand_ce_fwd_bwd(const pcv_table *t, const float *Q, const int64_t *candidates,
                         const int64_t *target_pos, int64_t M, int n_cand, float *loss_rows,
                         float *lse, float *dq, float *logits_out, pcv_stream_t stream);
+
+/* Gradient of the catalog CE w.r.t. the item table (fine_tune=True trains docEmbed, cvae.py:27-33):
+ *   dW[j] = sum_i row_scale[i] * m_ij * (e^{x_ij - lse_i} - [t_i = j]) * q_i
+ * with the forward's mask m (masked-out logits are constant zeros: no gradient).  Q, targets, M and mask are those of
+ * the pcv_ce_fwd_bwd call, lse [M] is what it returned, row_scale [M] = d loss / d loss_rows[i] (device).  dW [n_rows,
+ * dim] is OVERWRITTEN.  Whole table only (row_offset 0), dims 4..128 as the forward.  Paths (the forward's routing):
+ *  - bitmask, or keep_prob >= 1 with engine EXACT: item-major exact pass — a CTA owns 128 items and streams every
+ *    query row, logits re-derived with the forward's fp32 FMA chain, rows summed in a fixed order (+ a fixed-order
+ *    reduce of row splits when the catalog is small).  REPRODUCIBLE bit for bit;
+ *  - keep_prob >= 1 with engine TF32 (dims 8..128, else PCV_ERR_UNSUPPORTED): the same item-major sweep on the tensor
+ *    cores (tcgen05 kind::tf32: logits S^T = W_slab . Q^T, then dW += P^T . Q with P^T read from tensor memory; dW
+ *    stays in TMEM for the whole sweep).  Reduced precision like the tf32 forward (tf32 logits, within 2^-9 |q| |w|;
+ *    tf32 products in the contraction), REPRODUCIBLE bit for bit; needs no workspace beyond the query;
+ *  - Philox (keep_prob < 1, no bitmask): regenerates exactly the forward's gap-process mask from seed, offset and
+ *    *offset_dev, O(M * n_neg) work, float atomics: NOT reproducible bit for bit (last-bit differences run to run).
+ * Workspace: pcv_ce_table_grad_workspace_bytes for the same table, M and mask (no zero-fill needed).  No allocation,
+ * no host sync. */
+int pcv_ce_table_grad_workspace_bytes(const pcv_table *t, int64_t M, const pcv_ce_mask *mask, size_t *bytes_host);
+int pcv_ce_table_grad(const pcv_table *t, const float *Q, const int64_t *targets, int64_t M,
+                      const pcv_ce_mask *mask, const float *lse, const float *row_scale,
+                      float *dW, void *workspace, size_t workspace_bytes, pcv_stream_t stream);
+/* Candidate mode: dW[candidates[i, c]] += row_scale[i] * (softmax_c(p[i, :]) - [c = target_pos[i]]) * q_i for every
+ * column c (a duplicate candidate once per occurrence), logits re-derived from lse (of pcv_cand_ce_fwd_bwd).  ADDS
+ * into dW: the caller zero-fills it.  Float atomics: not reproducible bit for bit. */
+int pcv_cand_ce_table_grad(const pcv_table *t, const float *Q, const int64_t *candidates, const int64_t *target_pos,
+                           int64_t M, int n_cand, const float *lse, const float *row_scale, float *dW, pcv_stream_t stream);
 
 /* ------------------------------------------------------------------ */
 /* Simulator response models, gather-plus-dot (env/response_model.py)  */

@@ -121,6 +121,11 @@ EXPORTS = {
                                 c_void_p]),
     "pcv_cand_ce_fwd_bwd": (c_int, [c_void_p, c_void_p, c_void_p, c_void_p, c_int64, c_int, c_void_p, c_void_p, c_void_p,
                                     c_void_p, c_void_p]),
+    "pcv_ce_table_grad_workspace_bytes": (c_int, [c_void_p, c_int64, ctypes.POINTER(CeMask), ctypes.POINTER(c_size_t)]),
+    "pcv_ce_table_grad": (c_int, [c_void_p, c_void_p, c_void_p, c_int64, ctypes.POINTER(CeMask), c_void_p, c_void_p, c_void_p,
+                                  c_void_p, c_size_t, c_void_p]),
+    "pcv_cand_ce_table_grad": (c_int, [c_void_p, c_void_p, c_void_p, c_void_p, c_int64, c_int, c_void_p, c_void_p, c_void_p,
+                                       c_void_p]),
     "pcv_mlp_packed_bytes": (ctypes.c_size_t, [c_int, c_int]),
     "pcv_mlp_pack": (c_int, [c_void_p, c_int, c_int, c_void_p, c_void_p]),
     "pcv_mlp_tc_packed_bytes": (ctypes.c_size_t, [c_int, c_int]),

@@ -1,7 +1,8 @@
 """autograd glue around the fused CUDA blocks.
 
 Forward passes are single calls into libpcv_b200.so.  Backward of the catalog
-cross-entropy is free (the forward kernel already produced d loss/d q).  Backward
+cross-entropy w.r.t. the queries is free (the forward kernel already produced d loss/d q);
+w.r.t. a trainable item table (fine_tune=True) it is one more pass, pcv_ce_table_grad.  Backward
 of the MLP blocks runs on the library's own tensor-core GEMMs (csrc/gemm_tc.cu):
 per layer one split-K weight-gradient GEMM (+ a deterministic reduce that also
 emits the bias gradient) and one input-gradient GEMM whose epilogue applies the
@@ -22,12 +23,22 @@ class MlpSpec:
     segs: list of ('dense', k) | ('onehot', r) | ('gather', table, idx[, normalize]);
           ('dense', k) refers to the k-th differentiable dense input of the call.
     acts: activation id per layer.
+    train_tables: with save, every un-normalised gather segment whose table requires grad is listed in
+          `train_segs`, and the caller passes those tables after the parameters (FusedMLPFn) so that they get a
+          gradient.  Off: every gather table is treated as frozen, whatever its requires_grad.
     """
 
     def __init__(self, segs, acts, latent=0, eps=None, seed=0, offset=0, out_ld=None, out_col0=0, copy_seg=-1,
-                 save=True, offset_dev=None):
+                 save=True, offset_dev=None, train_tables=False):
         self.segs, self.acts = segs, list(acts)
         self.save = save
+        self.train_segs = []
+        if save and train_tables:
+            for i, s in enumerate(segs):
+                if s[0] == "gather" and s[1].requires_grad:
+                    if len(s) > 3 and s[3]:
+                        raise L.PcvError("a normalised gather segment has no table gradient here")
+                    self.train_segs.append(i)
         self.latent, self.eps, self.seed, self.offset = latent, eps, seed, offset
         self.offset_dev = offset_dev
         self.out_ld, self.out_col0, self.copy_seg = out_ld, out_col0, copy_seg
@@ -131,13 +142,18 @@ def _act_grad(g, a_out, act):
 
 
 class FusedMLPFn(torch.autograd.Function):
-    """apply(spec, B, n_dense, *dense_inputs, W0, b0, W1, b1, ...) -> out[, z]"""
+    """apply(spec, B, n_dense, *dense_inputs, W0, b0, W1, b1, ..., *tables) -> out[, z]
+
+    tables: the tables of spec.train_segs, in that order (none unless the spec was built with train_tables): each
+    gets the gradient of its gather segment, scattered into a table-shaped tensor."""
 
     @staticmethod
     def forward(ctx, spec, B, n_dense, *tensors):
         ctx.set_materialize_grads(False)      # an unused output (out or z) arrives as None, not as a zero-filled tensor
+        n_tab = len(spec.train_segs)
+        ctx.n_tables = n_tab
         dense = tensors[:n_dense]
-        wb = tensors[n_dense:]
+        wb = tensors[n_dense:len(tensors) - n_tab]
         layers = [(wb[2 * i], wb[2 * i + 1], spec.acts[i]) for i in range(len(wb) // 2)]
         need = spec.save and any(t.requires_grad for t in tensors)
         segments = spec.build_segments(dense)
@@ -186,17 +202,27 @@ class FusedMLPFn(torch.autograd.Function):
                     gz = torch.cat([d_z, d_z * eps * 0.5 * std], 1)
                     g = gz if g is None else g + gz
         if g is None:
-            return (None,) * (3 + ctx.n_dense + 2 * nl)
+            return (None,) * (3 + ctx.n_dense + 2 * nl + ctx.n_tables)
         g = g.contiguous()
         g = _act_grad(g, out[:, c0:c0 + ctx.n_out], spec.acts[nl - 1])      # identity for every block of the path
-        need_in = any(s[0] == "dense" and ctx.needs_input_grad[3 + s[1]] for s in spec.segs)
+        tab0 = 3 + ctx.n_dense + 2 * nl                  # input index of the first trainable table
+        need_tab = [ctx.needs_input_grad[tab0 + k] for k in range(ctx.n_tables)]
+        need_in = any(s[0] == "dense" and ctx.needs_input_grad[3 + s[1]] for s in spec.segs) or any(need_tab)
         grads_wb, g = _mlp_backward_tc(g, x0, acts, Ws, spec.acts, need_in, MLP_BWD_ENGINE == "tc3")
         d_dense = [None] * ctx.n_dense
         for si, s in enumerate(spec.segs):
             if s[0] == "dense" and ctx.needs_input_grad[3 + s[1]]:
                 o = ctx.seg_off[si]
                 d_dense[s[1]] = g[:, o:o + ctx.seg_width[si]]
-        return (None, None, None, *d_dense, *grads_wb)
+        d_tab = [None] * ctx.n_tables
+        for k, si in enumerate(spec.train_segs):
+            if need_tab[k]:
+                # the segment is count gathered rows of width D: scatter its B * count gradient rows into the table
+                table, idx = spec.segs[si][1], spec.segs[si][2]
+                o, D = ctx.seg_off[si], table.shape[1]
+                rows = g[:, o:o + ctx.seg_width[si]].reshape(-1, D)
+                d_tab[k] = torch.zeros_like(table).index_add_(0, idx.reshape(-1), rows)
+        return (None, None, None, *d_dense, *grads_wb, *d_tab)
 
 
 class CatalogCEFn(torch.autograd.Function):
@@ -204,23 +230,47 @@ class CatalogCEFn(torch.autograd.Function):
     (train_generative.py:36-42, 59) without materialising logits."""
 
     @staticmethod
-    def forward(ctx, q, table, targets, keep_prob, bitmask, seed, offset, offset_dev=None, engine="exact"):
+    def forward(ctx, q, table, targets, keep_prob, bitmask, seed, offset, offset_dev=None, engine="exact", weight=None):
+        """weight: the tensor `table` views (docEmbed.weight); when it requires grad, backward returns d loss / d weight
+        (pcv_ce_table_grad over the same mask)."""
         ctx.set_materialize_grads(False)
         loss_rows, lse, dq = ops.ce_fwd_bwd(table, q, targets, keep_prob, bitmask, seed, offset,
                                             want_dq=q.requires_grad, offset_dev=offset_dev, engine=engine)
         ctx.M = q.shape[0]
-        if dq is not None:
-            ctx.save_for_backward(dq)
+        ctx.want_dq = dq is not None
+        ctx.want_dw = weight is not None and weight.requires_grad
+        saved = [dq] if dq is not None else []
+        if ctx.want_dw:
+            saved += [q.detach(), targets, lse]
+            # the device-side Philox counter may advance before backward (NoiseSource.flush_eager): keep the value the
+            # forward read, so that the backward regenerates the forward's mask
+            snap = offset_dev.clone() if offset_dev is not None else None
+            ctx.table, ctx.mask_args = table, (keep_prob, bitmask, seed, offset, snap, engine)
+        ctx.save_for_backward(*saved)
         ctx.mark_non_differentiable(lse)
         return loss_rows.mean(), loss_rows, lse
 
     @staticmethod
     def backward(ctx, g_mean, g_rows, _g_lse):
-        (dq,) = ctx.saved_tensors
-        d = dq * (g_mean / ctx.M) if g_mean is not None else None
-        if g_rows is not None:
-            d = dq * g_rows.unsqueeze(1) if d is None else d + dq * g_rows.unsqueeze(1)
-        return d, None, None, None, None, None, None, None, None
+        saved = ctx.saved_tensors
+        d = dW = None
+        if ctx.want_dq:
+            dq = saved[0]
+            d = dq * (g_mean / ctx.M) if g_mean is not None else None
+            if g_rows is not None:
+                d = dq * g_rows.unsqueeze(1) if d is None else d + dq * g_rows.unsqueeze(1)
+        if ctx.want_dw and (g_mean is not None or g_rows is not None):
+            q, targets, lse = saved[-3:]
+            dW = ops.ce_table_grad(ctx.table, q, targets, lse, _row_scale(g_mean, g_rows, ctx.M), *ctx.mask_args)
+        return d, None, None, None, None, None, None, None, None, dW
+
+
+def _row_scale(g_mean, g_rows, M):
+    """[M] device tensor d loss / d loss_rows[i] = g_mean / M (+ g_rows[i]), without a host sync."""
+    rs = (g_mean / M).expand(M) if g_mean is not None else None
+    if g_rows is not None:
+        rs = g_rows if rs is None else rs + g_rows
+    return rs.to(torch.float32).contiguous()
 
 
 class VocabParallelCEFn(torch.autograd.Function):
@@ -306,44 +356,71 @@ class LogitsFn(torch.autograd.Function):
     """p = q @ W^T materialised, for forward()'s API parity (pivotcvae.py:274)."""
 
     @staticmethod
-    def forward(ctx, q, table):
+    def forward(ctx, q, table, weight=None):
         ctx.table = table
+        ctx.want_dw = weight is not None and weight.requires_grad
+        if ctx.want_dw:
+            ctx.save_for_backward(q.detach())
         return ops.score_logits(table, q)
 
     @staticmethod
     def backward(ctx, dp):
-        return dp.mm(ctx.table.weight), None
+        dW = dp.t().mm(ctx.saved_tensors[0]) if ctx.want_dw else None
+        return dp.mm(ctx.table.weight) if ctx.needs_input_grad[0] else None, None, dW
 
 
 class CandidateCEFn(torch.autograd.Function):
     """mean CE over per-row candidate lists (train_generative.py:52-56)."""
 
     @staticmethod
-    def forward(ctx, q, table, candidates, target_pos):
+    def forward(ctx, q, table, candidates, target_pos, weight=None):
+        """weight: the tensor `table` views; when it requires grad, backward returns d loss / d weight
+        (pcv_cand_ce_table_grad)."""
         loss_rows, lse, dq, _ = ops.cand_ce_fwd_bwd(table, q, candidates, target_pos, want_dq=q.requires_grad)
         ctx.M = q.shape[0]
-        if dq is not None:
-            ctx.save_for_backward(dq)
+        ctx.want_dq = dq is not None
+        ctx.want_dw = weight is not None and weight.requires_grad
+        saved = [dq] if dq is not None else []
+        if ctx.want_dw:
+            saved += [q.detach(), candidates, target_pos, lse]
+            ctx.table = table
+        ctx.save_for_backward(*saved)
         return loss_rows.mean()
 
     @staticmethod
     def backward(ctx, g):
-        (dq,) = ctx.saved_tensors
-        return dq * (g / ctx.M), None, None, None
+        saved = ctx.saved_tensors
+        d = saved[0] * (g / ctx.M) if ctx.want_dq else None
+        dW = None
+        if ctx.want_dw:
+            q, cand, tpos, lse = saved[-4:]
+            dW = ops.cand_ce_table_grad(ctx.table, q, cand, tpos, lse, _row_scale(g, None, ctx.M))
+        return d, None, None, None, dW
 
 
 class CandidateLogitsFn(torch.autograd.Function):
     """p[i, c] = <W[cand[i, c]], q_i> materialised (forward()'s candidate branch, pivotcvae.py:265-271)."""
 
     @staticmethod
-    def forward(ctx, q, table, candidates):
+    def forward(ctx, q, table, candidates, weight=None):
         M = q.shape[0]
         tp = torch.zeros(M, dtype=torch.int64, device=q.device)
         _, _, _, p = ops.cand_ce_fwd_bwd(table, q, candidates, tp, want_dq=False, want_logits=True)
         ctx.table, ctx.cand = table, candidates
+        ctx.want_dw = weight is not None and weight.requires_grad
+        if ctx.want_dw:
+            ctx.save_for_backward(q.detach())
         return p
 
     @staticmethod
     def backward(ctx, dp):
-        w = ctx.table.weight[ctx.cand.reshape(dp.shape[0], -1)]          # (M, nC, D) plain gather
-        return torch.bmm(dp.unsqueeze(1), w).squeeze(1), None, None
+        cand = ctx.cand.reshape(dp.shape[0], -1)
+        dq = dW = None
+        if ctx.needs_input_grad[0]:
+            w = ctx.table.weight[cand]                                   # (M, nC, D) plain gather
+            dq = torch.bmm(dp.unsqueeze(1), w).squeeze(1)
+        if ctx.want_dw:
+            q = ctx.saved_tensors[0]
+            rows = (dp.unsqueeze(2) * q.unsqueeze(1)).reshape(-1, q.shape[1])    # (M * nC, D): dp[i, c] q_i
+            dW = torch.zeros_like(ctx.table.weight).index_add_(0, cand.reshape(-1), rows)
+        return dq, None, None, dW

@@ -10,7 +10,8 @@
 // Semantics kept (SURVEY F7): masked-OUT logits become 0 (not -inf):
 //   lse_i  = log( sum_{j in mask_i} e^{x_ij} + (N - |mask_i|) )
 //   loss_i = lse_i - x_{i,t_i}
-//   dq_i   = sum_{j in mask_i} softmax_ij * w_j - w_{t_i}          (table frozen: no dW)
+//   dq_i   = sum_{j in mask_i} softmax_ij * w_j - w_{t_i}
+// The table gradient (fine_tune=True) is a separate pass, pcv_ce_table_grad (below).
 //
 // Layout mirrors score_select.cu: CTA = 8 warps x R rows, catalog split over
 // blockIdx.y, cp.async double-buffered float4-SoA tiles.  Each lane keeps an
@@ -604,10 +605,315 @@ static int ce_dispatch(const Table *t, const CEPlan &p, const float *Q, const in
   return PCV_ERR_UNSUPPORTED;
 }
 
+// ---------------------------------------------------------------------------
+// Gradient w.r.t. the item table (fine_tune=True trains docEmbed, cvae.py:27-33):
+//   dW[j] = sum_i g_i m_ij (p_ij - [t_i = j]) q_i,   p_ij = e^{x_ij - lse_i},   g_i = row_scale[i]
+// where m_ij is the forward's mask (masked-out logits are the constant 0: no gradient, SURVEY F7) and lse_i is what
+// pcv_ce_fwd_bwd returned.  Item-major: a CTA owns TG_ITEMS items (one per thread, its dW row in registers) and
+// streams query rows through shared memory, TG_ROWS at a time; every logit is recomputed with the forward's exact
+// fp32 FMA chain.  Rows are summed in ascending order; when the catalog gives too few CTAs the rows are cut into
+// n_split ranges whose partial rows ce_tg_reduce_kernel adds in split order.  No atomics: reproducible bit for bit.
+// ---------------------------------------------------------------------------
+constexpr int TG_ITEMS = 128;   // items per CTA = threads
+constexpr int TG_ROWS = 32;     // query rows per shared-memory tile
+
+template <int D>
+struct TGCfg {
+  static constexpr bool W_REG = D <= 64;   // D = 128: the item row lives in shared memory (acc alone is 128 registers)
+  static constexpr int UNROLL = D <= 64 ? 2 : 1;   // rows in flight per thread
+  static constexpr size_t Q_BYTES = (size_t)TG_ROWS * D * sizeof(float);
+  static constexpr size_t W_BYTES = W_REG ? 0 : (size_t)TG_ITEMS * D * sizeof(float);
+  static constexpr size_t SMEM = Q_BYTES + W_BYTES + TG_ROWS * (2 * sizeof(float) + sizeof(int64_t));
+};
+
+struct TGPlan {
+  int item_ctas, n_split;
+  int64_t rows_per_split;
+  size_t ws_bytes;
+};
+
+static void tg_plan(const Table *t, int64_t M, TGPlan *p) {
+  p->item_ctas = (int)((t->n_rows + TG_ITEMS - 1) / TG_ITEMS);
+  const int64_t row_tiles = (M + TG_ROWS - 1) / TG_ROWS;
+  int64_t ns = (4LL * t->sm_count + p->item_ctas - 1) / p->item_ctas;   // ~4 CTAs (16 warps) per SM
+  if (ns > 64) ns = 64;
+  if (ns > row_tiles) ns = row_tiles;
+  if (ns < 1) ns = 1;
+  const int64_t tiles_per = (row_tiles + ns - 1) / ns;
+  p->rows_per_split = tiles_per * TG_ROWS;
+  p->n_split = (int)((M + p->rows_per_split - 1) / p->rows_per_split);
+  p->ws_bytes = p->n_split > 1 ? (size_t)p->n_split * (size_t)t->n_rows * t->dim * sizeof(float) : 0;
+}
+
+template <int D, int MODE>
+__global__ void __launch_bounds__(TG_ITEMS, D <= 16 ? 8 : 1)
+ce_table_grad_kernel(const float *__restrict__ W, int64_t n_rows, const float *__restrict__ Q,
+                     const int64_t *__restrict__ targets, const float *__restrict__ lse,
+                     const float *__restrict__ row_scale, int64_t M, int64_t rows_per_split,
+                     const uint32_t *__restrict__ bitmask, int64_t mask_words, float *__restrict__ out) {
+  using Cfg = TGCfg<D>;
+  constexpr int C4 = D / 4;
+  extern __shared__ __align__(16) unsigned char smem_raw[];
+  float4 *qs4 = reinterpret_cast<float4 *>(smem_raw);                                   // [TG_ROWS][C4]
+  float *wsm = reinterpret_cast<float *>(smem_raw + Cfg::Q_BYTES);                       // [D][TG_ITEMS] (D = 128)
+  float *ls = reinterpret_cast<float *>(smem_raw + Cfg::Q_BYTES + Cfg::W_BYTES);         // [TG_ROWS]
+  float *gs = ls + TG_ROWS;                                                              // [TG_ROWS]
+  int64_t *ts = reinterpret_cast<int64_t *>(gs + TG_ROWS);                               // [TG_ROWS]
+
+  const int tid = threadIdx.x;
+  const int64_t j = (int64_t)blockIdx.x * TG_ITEMS + tid;
+  const bool live = j < n_rows;
+  const int64_t i_begin = (int64_t)blockIdx.y * rows_per_split;
+  const int64_t i_end = min(M, i_begin + rows_per_split);
+
+  float w[Cfg::W_REG ? D : 1];
+#pragma unroll
+  for (int c = 0; c < C4; ++c) {
+    const float4 v = live ? __ldg(reinterpret_cast<const float4 *>(W + j * D) + c) : make_float4(0.f, 0.f, 0.f, 0.f);
+    if constexpr (Cfg::W_REG) {
+      w[4 * c] = v.x; w[4 * c + 1] = v.y; w[4 * c + 2] = v.z; w[4 * c + 3] = v.w;
+    } else {
+      wsm[(4 * c + 0) * TG_ITEMS + tid] = v.x; wsm[(4 * c + 1) * TG_ITEMS + tid] = v.y;
+      wsm[(4 * c + 2) * TG_ITEMS + tid] = v.z; wsm[(4 * c + 3) * TG_ITEMS + tid] = v.w;
+    }
+  }
+  float acc[D];
+#pragma unroll
+  for (int k = 0; k < D; ++k) acc[k] = 0.f;
+
+  for (int64_t i0 = i_begin; i0 < i_end; i0 += TG_ROWS) {
+    const int nr = (int)min((int64_t)TG_ROWS, i_end - i0);
+    __syncthreads();
+    const float4 *src = reinterpret_cast<const float4 *>(Q + i0 * D);
+    for (int f = tid; f < nr * C4; f += TG_ITEMS) qs4[f] = __ldg(src + f);
+    if (tid < nr) {
+      ls[tid] = lse[i0 + tid];
+      gs[tid] = row_scale[i0 + tid];
+      ts[tid] = targets[i0 + tid];
+    }
+    __syncthreads();
+#pragma unroll(Cfg::UNROLL)
+    for (int r = 0; r < nr; ++r) {
+      const int64_t t = ts[r];
+      bool keep = live;
+      if (MODE == CE_BITMASK) {
+        // 32 consecutive items of a warp share one mask word (TG_ITEMS is a multiple of 32)
+        const uint32_t word = live ? __ldg(bitmask + (i0 + r) * mask_words + (j >> 5)) : 0u;
+        keep = live && ((((word >> (j & 31)) & 1u) != 0u) || j == t);
+      }
+      if (!keep) continue;
+      const float4 *qr = qs4 + r * C4;
+      float s = 0.f;
+#pragma unroll(Cfg::W_REG ? C4 : 4)
+      for (int c = 0; c < C4; ++c) {
+        const float4 v = qr[c];
+        if constexpr (Cfg::W_REG) {
+          s = fmaf(v.x, w[4 * c], s); s = fmaf(v.y, w[4 * c + 1], s);
+          s = fmaf(v.z, w[4 * c + 2], s); s = fmaf(v.w, w[4 * c + 3], s);
+        } else {
+          s = fmaf(v.x, wsm[(4 * c) * TG_ITEMS + tid], s); s = fmaf(v.y, wsm[(4 * c + 1) * TG_ITEMS + tid], s);
+          s = fmaf(v.z, wsm[(4 * c + 2) * TG_ITEMS + tid], s); s = fmaf(v.w, wsm[(4 * c + 3) * TG_ITEMS + tid], s);
+        }
+      }
+      const float p = __expf(s - ls[r]);
+      const float coef = gs[r] * (j == t ? p - 1.f : p);
+      // D = 128: read the query row from shared memory again rather than keep its 128 floats live next to acc
+      if constexpr (!Cfg::W_REG) asm volatile("" ::: "memory");
+#pragma unroll
+      for (int c = 0; c < C4; ++c) {
+        const float4 v = qr[c];
+        acc[4 * c] = fmaf(coef, v.x, acc[4 * c]); acc[4 * c + 1] = fmaf(coef, v.y, acc[4 * c + 1]);
+        acc[4 * c + 2] = fmaf(coef, v.z, acc[4 * c + 2]); acc[4 * c + 3] = fmaf(coef, v.w, acc[4 * c + 3]);
+      }
+    }
+  }
+  if (!live) return;
+  float4 *dst = reinterpret_cast<float4 *>(out + ((int64_t)blockIdx.y * n_rows + j) * D);
+#pragma unroll
+  for (int c = 0; c < C4; ++c) dst[c] = make_float4(acc[4 * c], acc[4 * c + 1], acc[4 * c + 2], acc[4 * c + 3]);
+}
+
+// dW[e] = sum_s part[s][e] in split order (e over the n_rows * D floats of the table)
+__global__ void __launch_bounds__(256)
+ce_tg_reduce_kernel(const float4 *__restrict__ part, int n_split, int64_t n4, float4 *__restrict__ dW) {
+  const int64_t e = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
+  if (e >= n4) return;
+  float4 a = part[e];
+  for (int s = 1; s < n_split; ++s) {
+    const float4 v = part[(int64_t)s * n4 + e];
+    a.x += v.x; a.y += v.y; a.z += v.z; a.w += v.w;
+  }
+  dW[e] = a;
+}
+
+template <int D, int MODE>
+static int launch_table_grad(const Table *t, const TGPlan &p, const float *Q, const int64_t *targets, const float *lse,
+                             const float *row_scale, int64_t M, const uint32_t *bitmask, float *dW, float *part,
+                             cudaStream_t st) {
+  using Cfg = TGCfg<D>;
+  auto kern = ce_table_grad_kernel<D, MODE>;
+  static bool attr_set[64] = {false};
+  if (!attr_set[t->device & 63]) {
+    PCV_CUDA(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)Cfg::SMEM));
+    attr_set[t->device & 63] = true;
+  }
+  const int64_t mask_words = (t->n_rows + 31) / 32;
+  dim3 grid((unsigned)p.item_ctas, (unsigned)p.n_split);
+  kern<<<grid, TG_ITEMS, Cfg::SMEM, st>>>(t->W, t->n_rows, Q, targets, lse, row_scale, M, p.rows_per_split, bitmask,
+                                           mask_words, p.n_split > 1 ? part : dW);
+  PCV_LAUNCH_CHECK();
+  if (p.n_split > 1) {
+    const int64_t n4 = t->n_rows * D / 4;
+    ce_tg_reduce_kernel<<<(unsigned)((n4 + 255) / 256), 256, 0, st>>>(reinterpret_cast<const float4 *>(part), p.n_split,
+                                                                        n4, reinterpret_cast<float4 *>(dW));
+    PCV_LAUNCH_CHECK();
+  }
+  return PCV_OK;
+}
+
+template <int MODE>
+static int table_grad_dispatch(const Table *t, const TGPlan &p, const float *Q, const int64_t *targets, const float *lse,
+                               const float *row_scale, int64_t M, const uint32_t *bitmask, float *dW, float *part,
+                               cudaStream_t st) {
+  switch (t->dim) {
+    case 4: return launch_table_grad<4, MODE>(t, p, Q, targets, lse, row_scale, M, bitmask, dW, part, st);
+    case 8: return launch_table_grad<8, MODE>(t, p, Q, targets, lse, row_scale, M, bitmask, dW, part, st);
+    case 16: return launch_table_grad<16, MODE>(t, p, Q, targets, lse, row_scale, M, bitmask, dW, part, st);
+    case 32: return launch_table_grad<32, MODE>(t, p, Q, targets, lse, row_scale, M, bitmask, dW, part, st);
+    case 64: return launch_table_grad<64, MODE>(t, p, Q, targets, lse, row_scale, M, bitmask, dW, part, st);
+    case 128: return launch_table_grad<128, MODE>(t, p, Q, targets, lse, row_scale, M, bitmask, dW, part, st);
+  }
+  set_error("ce_table_grad: dim %d unsupported (use 4, 8, 16, 32, 64 or 128)", t->dim);
+  return PCV_ERR_UNSUPPORTED;
+}
+
+// Philox gap-process mask (keep_prob < 1): the same walk as ce_sparse_kernel — one warp per row, lane = 1024-column
+// block, Philox keyed on (block, row + offset) — regenerates exactly the forward's kept columns, O(n_neg) per row.
+// Each kept column adds g (p - [j = t]) q_i to its dW row with vector float atomics: NOT reproducible bit for bit
+// (the summation order over rows follows the schedule).  The caller's dW is zeroed by the entry point first.
+template <int D>
+__global__ void __launch_bounds__(256)
+ce_sparse_table_grad_kernel(const float *__restrict__ W, int64_t n_rows, const float *__restrict__ Q,
+                            const int64_t *__restrict__ targets, const float *__restrict__ lse,
+                            const float *__restrict__ row_scale, int64_t M, const uint32_t *__restrict__ T,
+                            uint64_t seed, uint64_t offset, const uint64_t *__restrict__ offset_dev,
+                            float *__restrict__ dW) {
+  const int lane = threadIdx.x & 31;
+  const int64_t row = (int64_t)blockIdx.x * (blockDim.x >> 5) + (threadIdx.x >> 5);
+  if (row >= M) return;
+  const float g = row_scale[row];
+  if (g == 0.f) return;     // every contribution of the row is a signed zero
+  if (offset_dev) offset += *offset_dev;
+  const uint64_t rr = (uint64_t)row + offset;
+  float q[D];
+#pragma unroll
+  for (int c = 0; c < D / 4; ++c) {
+    const float4 v = __ldg(reinterpret_cast<const float4 *>(Q + row * D) + c);
+    q[4 * c] = v.x; q[4 * c + 1] = v.y; q[4 * c + 2] = v.z; q[4 * c + 3] = v.w;
+  }
+  const int64_t tgt = targets[row];
+  const float l_row = lse[row];
+  bool seen_tgt = false;
+  auto visit = [&](int64_t j) {
+    float s = 0.f;
+#pragma unroll
+    for (int c = 0; c < D / 4; ++c) {
+      const float4 v = __ldg(reinterpret_cast<const float4 *>(W + j * D) + c);
+      s = fmaf(q[4 * c], v.x, s); s = fmaf(q[4 * c + 1], v.y, s);
+      s = fmaf(q[4 * c + 2], v.z, s); s = fmaf(q[4 * c + 3], v.w, s);
+    }
+    const float p = __expf(s - l_row);
+    const float coef = g * (j == tgt ? p - 1.f : p);
+    float4 *dst = reinterpret_cast<float4 *>(dW + j * D);
+#pragma unroll
+    for (int c = 0; c < D / 4; ++c)
+      atomicAdd(dst + c, make_float4(coef * q[4 * c], coef * q[4 * c + 1], coef * q[4 * c + 2], coef * q[4 * c + 3]));
+  };
+  const int64_t n_blocks = (n_rows + CE_GB - 1) / CE_GB;
+  for (int64_t b = lane; b < n_blocks; b += 32) {
+    int c = -1;
+    Philox4 ph = {0, 0, 0, 0};
+    for (int k = 0;; ++k) {
+      if ((k & 3) == 0)
+        ph = philox4x32_10((uint32_t)b, (uint32_t)rr, (uint32_t)(rr >> 32),
+                           PCV_STREAM_BERNOULLI + ((uint32_t)(k >> 2) << 4), (uint32_t)seed, (uint32_t)(seed >> 32));
+      const uint32_t u = (k & 3) == 0 ? ph.x : ((k & 3) == 1 ? ph.y : ((k & 3) == 2 ? ph.z : ph.w));
+      c += 1 + gap_from_u(T, u);
+      if (c >= CE_GB) break;
+      const int64_t j = b * CE_GB + c;
+      if (j >= n_rows) break;
+      if (j == tgt) seen_tgt = true;
+      visit(j);
+    }
+  }
+  // the target column is always part of the mask (train_generative.py:38)
+  const bool any_seen = __any_sync(0xffffffffu, seen_tgt);
+  if (lane == 0 && !any_seen) visit(tgt);
+}
+
+template <int D>
+static int launch_sparse_table_grad(const Table *t, const float *Q, const int64_t *targets, const float *lse,
+                                    const float *row_scale, int64_t M, const pcv_ce_mask *mask, uint32_t *T, float *dW,
+                                    cudaStream_t st) {
+  double qd = (1.0 - mask->keep_prob) * 4294967296.0;
+  const uint32_t q32 = qd <= 0.0 ? 0u : (qd >= 4294967295.0 ? 0xffffffffu : (uint32_t)(qd + 0.5));
+  PCV_CUDA(cudaMemsetAsync(dW, 0, (size_t)t->n_rows * D * sizeof(float), st));
+  ce_gap_table_kernel<<<1, 1, 0, st>>>(q32, T);
+  PCV_LAUNCH_CHECK();
+  ce_sparse_table_grad_kernel<D><<<(unsigned)((M + 7) / 8), 256, 0, st>>>(t->W, t->n_rows, Q, targets, lse, row_scale, M, T,
+                                                                         mask->seed, mask->offset, mask->offset_dev, dW);
+  PCV_LAUNCH_CHECK();
+  return PCV_OK;
+}
+
+// Candidate mode: one warp per row, lane = candidate column (as cand_ce_kernel); the logit is recomputed from lse, so
+// no [M, n_cand] buffer is kept.  Column c adds g (p_c - [c = target_pos]) q_i to dW[cand[i, c]] (duplicates once per
+// occurrence) with vector float atomics.
+template <int D>
+__global__ void __launch_bounds__(256)
+cand_ce_table_grad_kernel(const float *__restrict__ W, const float *__restrict__ Q, const int64_t *__restrict__ cand,
+                          const int64_t *__restrict__ tgt_pos, int64_t M, int nC, const float *__restrict__ lse,
+                          const float *__restrict__ row_scale, float *__restrict__ dW) {
+  const int lane = threadIdx.x & 31;
+  const int64_t row = (int64_t)blockIdx.x * (blockDim.x >> 5) + (threadIdx.x >> 5);
+  if (row >= M) return;
+  const float g = row_scale[row];
+  if (g == 0.f) return;
+  float q[D];
+#pragma unroll
+  for (int c = 0; c < D / 4; ++c) {
+    const float4 v = __ldg(reinterpret_cast<const float4 *>(Q + row * D) + c);
+    q[4 * c] = v.x; q[4 * c + 1] = v.y; q[4 * c + 2] = v.z; q[4 * c + 3] = v.w;
+  }
+  const float l_row = lse[row];
+  const int64_t tp = tgt_pos[row];
+  const int64_t *cr = cand + row * nC;
+  for (int c = lane; c < nC; c += 32) {
+    const int64_t j = __ldg(cr + c);
+    float w[D];
+#pragma unroll
+    for (int v4 = 0; v4 < D / 4; ++v4) {
+      const float4 v = __ldg(reinterpret_cast<const float4 *>(W + j * D) + v4);
+      w[4 * v4] = v.x; w[4 * v4 + 1] = v.y; w[4 * v4 + 2] = v.z; w[4 * v4 + 3] = v.w;
+    }
+    float s = 0.f;
+#pragma unroll
+    for (int k = 0; k < D; ++k) s = fmaf(w[k], q[k], s);   // the forward's chain (cand_ce_kernel)
+    const float p = __expf(s - l_row);
+    const float coef = g * (c == tp ? p - 1.f : p);
+    float4 *dst = reinterpret_cast<float4 *>(dW + j * D);
+#pragma unroll
+    for (int v4 = 0; v4 < D / 4; ++v4)
+      atomicAdd(dst + v4, make_float4(coef * q[4 * v4], coef * q[4 * v4 + 1], coef * q[4 * v4 + 2], coef * q[4 * v4 + 3]));
+  }
+}
+
 // tensor-core engine (ce_tc2.cu)
 bool ce_tc_supported(const Table *t);
 size_t ce_tc_workspace(const Table *t, int64_t M);
 int ce_tc_launch(const Table *t, const float *Q, const int64_t *targets, int64_t M, float *part, size_t ws_bytes, cudaStream_t st);
+int ce_tc_table_grad(const Table *t, const float *Q, const int64_t *targets, const float *lse, const float *row_scale,
+                     int64_t M, float *dW, cudaStream_t st);
 
 }  // namespace pcv
 
@@ -731,6 +1037,97 @@ int pcv_ce_partials(const pcv_table *th, const float *Q, const int64_t *targets,
                     pcv_stream_t stream) {
   PCV_CHECK_ARG(rec_out != nullptr, "rec_out is NULL");
   return ce_run(th, Q, targets, M, mask, nullptr, nullptr, nullptr, rec_out, workspace, workspace_bytes, stream);
+}
+
+int pcv_ce_table_grad_workspace_bytes(const pcv_table *th, int64_t M, const pcv_ce_mask *mask, size_t *bytes_host) {
+  PCV_CHECK_ARG(th && mask && bytes_host, "NULL pointer");
+  PCV_CHECK_ARG(M > 0, "M must be > 0");
+  const Table *t = reinterpret_cast<const Table *>(th);
+  if (!ce_rows_for(t->dim)) {
+    set_error("ce_table_grad: dim %d unsupported", t->dim);
+    return PCV_ERR_UNSUPPORTED;
+  }
+  size_t b = (CE_GB_HOST + 1) * sizeof(uint32_t);   // gap table of the Philox path
+  if (mask->bitmask || mask->keep_prob >= 1.0) {
+    TGPlan p;
+    tg_plan(t, M, &p);
+    if (p.ws_bytes > b) b = p.ws_bytes;
+  }
+  *bytes_host = (b + 255) & ~(size_t)255;
+  return PCV_OK;
+}
+
+int pcv_ce_table_grad(const pcv_table *th, const float *Q, const int64_t *targets, int64_t M, const pcv_ce_mask *mask,
+                      const float *lse, const float *row_scale, float *dW, void *workspace, size_t workspace_bytes,
+                      pcv_stream_t stream) {
+  PCV_CHECK_ARG(th && Q && targets && mask && lse && row_scale && dW, "NULL pointer");
+  PCV_CHECK_ARG(M > 0, "M must be > 0");
+  const Table *t = reinterpret_cast<const Table *>(th);
+  PCV_CHECK_ARG(t->row_offset == 0, "the table gradient needs the whole table (row_offset 0)");
+  PCV_CHECK_ARG(t->n_rows < 0x7fffffffLL, "table larger than 2^31-1 rows");
+  PCV_CHECK_ARG(mask->keep_prob > 0.0, "keep_prob must be > 0");
+  if (!ce_rows_for(t->dim)) {
+    set_error("ce_table_grad: dim %d unsupported (use 4, 8, 16, 32, 64 or 128)", t->dim);
+    return PCV_ERR_UNSUPPORTED;
+  }
+  const bool dense = mask->bitmask == nullptr && mask->keep_prob >= 1.0;
+  if (dense && mask->engine == PCV_CE_ENGINE_TF32 && t->dim < 8) {
+    set_error("ce_table_grad: the tf32 engine serves dims 8, 16, 32, 64 and 128 (this table has dim %d)", t->dim);
+    return PCV_ERR_UNSUPPORTED;
+  }
+  int rc = check_arch();
+  if (rc != PCV_OK) return rc;
+  size_t need = 0;
+  rc = pcv_ce_table_grad_workspace_bytes(th, M, mask, &need);
+  if (rc != PCV_OK) return rc;
+  if (!workspace || workspace_bytes < need) {
+    set_error("ce_table_grad: workspace too small (%zu < %zu)", workspace_bytes, need);
+    return PCV_ERR_WORKSPACE;
+  }
+  cudaStream_t st = (cudaStream_t)stream;
+  if (dense && mask->engine == PCV_CE_ENGINE_TF32) return ce_tc_table_grad(t, Q, targets, lse, row_scale, M, dW, st);
+  if (mask->bitmask || dense) {
+    TGPlan p;
+    tg_plan(t, M, &p);
+    float *part = reinterpret_cast<float *>(workspace);
+    return mask->bitmask ? table_grad_dispatch<CE_BITMASK>(t, p, Q, targets, lse, row_scale, M, mask->bitmask, dW, part, st)
+                         : table_grad_dispatch<CE_DENSE>(t, p, Q, targets, lse, row_scale, M, nullptr, dW, part, st);
+  }
+  uint32_t *T = reinterpret_cast<uint32_t *>(workspace);
+  switch (t->dim) {
+    case 4: return launch_sparse_table_grad<4>(t, Q, targets, lse, row_scale, M, mask, T, dW, st);
+    case 8: return launch_sparse_table_grad<8>(t, Q, targets, lse, row_scale, M, mask, T, dW, st);
+    case 16: return launch_sparse_table_grad<16>(t, Q, targets, lse, row_scale, M, mask, T, dW, st);
+    case 32: return launch_sparse_table_grad<32>(t, Q, targets, lse, row_scale, M, mask, T, dW, st);
+    case 64: return launch_sparse_table_grad<64>(t, Q, targets, lse, row_scale, M, mask, T, dW, st);
+    case 128: return launch_sparse_table_grad<128>(t, Q, targets, lse, row_scale, M, mask, T, dW, st);
+  }
+  return PCV_ERR_UNSUPPORTED;
+}
+
+int pcv_cand_ce_table_grad(const pcv_table *th, const float *Q, const int64_t *candidates, const int64_t *target_pos,
+                           int64_t M, int n_cand, const float *lse, const float *row_scale, float *dW, pcv_stream_t stream) {
+  PCV_CHECK_ARG(th && Q && candidates && target_pos && lse && row_scale && dW, "NULL pointer");
+  PCV_CHECK_ARG(M > 0 && n_cand > 0, "bad shape");
+  const Table *t = reinterpret_cast<const Table *>(th);
+  PCV_CHECK_ARG(t->row_offset == 0, "candidate CE needs the whole table (row_offset 0)");
+  int rc = check_arch();
+  if (rc != PCV_OK) return rc;
+  cudaStream_t st = (cudaStream_t)stream;
+  const unsigned blocks = (unsigned)((M + 7) / 8);
+  switch (t->dim) {
+    case 4: cand_ce_table_grad_kernel<4><<<blocks, 256, 0, st>>>(t->W, Q, candidates, target_pos, M, n_cand, lse, row_scale, dW); break;
+    case 8: cand_ce_table_grad_kernel<8><<<blocks, 256, 0, st>>>(t->W, Q, candidates, target_pos, M, n_cand, lse, row_scale, dW); break;
+    case 16: cand_ce_table_grad_kernel<16><<<blocks, 256, 0, st>>>(t->W, Q, candidates, target_pos, M, n_cand, lse, row_scale, dW); break;
+    case 32: cand_ce_table_grad_kernel<32><<<blocks, 256, 0, st>>>(t->W, Q, candidates, target_pos, M, n_cand, lse, row_scale, dW); break;
+    case 64: cand_ce_table_grad_kernel<64><<<blocks, 256, 0, st>>>(t->W, Q, candidates, target_pos, M, n_cand, lse, row_scale, dW); break;
+    case 128: cand_ce_table_grad_kernel<128><<<blocks, 256, 0, st>>>(t->W, Q, candidates, target_pos, M, n_cand, lse, row_scale, dW); break;
+    default:
+      set_error("cand_ce_table_grad: dim %d unsupported", t->dim);
+      return PCV_ERR_UNSUPPORTED;
+  }
+  PCV_LAUNCH_CHECK();
+  return PCV_OK;
 }
 
 int pcv_ce_vp_merge(const float *recs, int G, const float *W_full, int dim, const float *Q, const int64_t *targets,

@@ -551,6 +551,197 @@ ce_tc2_kernel(const float *__restrict__ Wsw, const float *__restrict__ Wt, int64
   }
 }
 
+// ---------------------------------------------------------------------------
+// Table gradient on the tensor cores (pcv_ce_table_grad, engine TF32, dense mask): ce_tc2_kernel with the roles of Q
+// and W swapped.  A CTA owns a slab of 128 items (the TMEM lanes) and sweeps every query row, BN at a time:
+//
+//   S^T[128 items x BN rows] = W_slab . Q_tile^T        KA accumulating tcgen05.mma kind::tf32, A = the slab and B
+//                                                       the query tile, both K-major SWIZZLE_32B images in smem
+//   P^T = g_i (exp(S^T - lse_i) - [t_i = j])            4 epilogue warps, thread = item: TMEM -> registers -> TMEM
+//   dW_slab[128 x NG] += P^T . Qt_tile^T                BN / 8 MMAs, A = P^T from TENSOR MEMORY, B = the transposed
+//                                                       query tile [NG dims x BN rows] (the layout of ce_tc2's Wt)
+//
+// dW stays in TMEM for the whole sweep and is written once: no atomics, no split, reproducible bit for bit.  lse is
+// known, so no reference exponent is needed.  The CTA builds its slab and each query tile's two images itself from
+// the fp32 arrays (they are small: BN x D floats per image); the steps of a tile run back to back (load, score MMA,
+// epilogue, gradient MMA), and the overlap comes from the other CTAs of the SM.
+//   D     BN   slab + Q tile + Qt tile (smem)   TMEM columns (S^T + dW, allocated)
+//   8    128      4 +  4 +  8 KB                  128 + 16  (256)
+//   16   128      8 +  8 +  8 KB                  128 + 16  (256)
+//   32   128     16 + 16 + 16 KB                  128 + 32  (256)
+//   64    64     32 + 16 + 16 KB                   64 + 64  (128)
+//   128   64     64 + 32 + 32 KB                   64 + 128 (256)
+// Error: the tf32 logit is within 2^-9 |q_i| |w_j| of the exact one (both operands truncated to 10 mantissa bits), and
+// the gradient MMA truncates P^T and Q again (2^-9 relative per term).
+template <int D>
+struct TgCfg {
+  static constexpr int KA = D / 8;
+  static constexpr int BN = D <= 32 ? 128 : 64;
+  static constexpr int NG = D < 16 ? 16 : D;
+  static constexpr int DW_COL = BN;
+  static constexpr int TCOLS = (BN + NG) <= 128 ? 128 : 256;
+  static constexpr int GW = D < 32 ? D : 32;
+};
+
+template <int D>
+struct __align__(1024) TgSmem {
+  using C = TgCfg<D>;
+  float wa[TC_BM * D];             // item slab: KA k-atoms of [128 rows x 32 B]
+  float qw[C::BN * D];             // query tile: KA k-atoms of [BN rows x 32 B]
+  float qt[(C::BN / 8) * C::NG * 8];   // transposed query tile: BN / 8 k-atoms of [NG rows x 32 B]
+  float lse[C::BN], rs[C::BN];
+  int64_t tg[C::BN];
+  unsigned long long sdone, gdone;
+  uint32_t tmem_base;
+};
+
+template <int D>
+__global__ void __launch_bounds__(TC_BM)
+ce_tc_table_grad_kernel(const float *__restrict__ W, int64_t n_rows, const float *__restrict__ Q,
+                        const int64_t *__restrict__ targets, const float *__restrict__ lse,
+                        const float *__restrict__ row_scale, int64_t M, float *__restrict__ dW) {
+  using C = TgCfg<D>;
+  constexpr int BN = C::BN, KA = C::KA, NG = C::NG, GW = C::GW;
+  constexpr uint32_t IDESC_S = C2_IDESC<BN>, IDESC_G = C2_IDESC<NG>;
+  extern __shared__ unsigned char smem_raw[];
+  TgSmem<D> &S = *reinterpret_cast<TgSmem<D> *>((reinterpret_cast<uintptr_t>(smem_raw) + 1023) & ~(uintptr_t)1023);
+  const int tid = threadIdx.x, warp = tid >> 5, lane = tid & 31;
+  const int64_t j0 = (int64_t)blockIdx.x * TC_BM;
+
+  // item slab, SWIZZLE_32B: row t at byte t*32 of its atom, 16-byte chunk c at ((c ^ bit2(t)) * 16); rows past the
+  // table end are zero
+  {
+    const int64_t j = j0 + tid;
+    const int sw = (tid >> 2) & 1;
+#pragma unroll
+    for (int a = 0; a < KA; ++a) {
+      float4 w0 = make_float4(0.f, 0.f, 0.f, 0.f), w1 = w0;
+      if (j < n_rows) {
+        w0 = __ldg(reinterpret_cast<const float4 *>(W + j * D + a * 8));
+        w1 = __ldg(reinterpret_cast<const float4 *>(W + j * D + a * 8) + 1);
+      }
+      float4 *dst = reinterpret_cast<float4 *>(S.wa + a * (TC_BM * 8) + tid * 8);
+      dst[0 ^ sw] = w0;
+      dst[1 ^ sw] = w1;
+    }
+  }
+  // the padding rows D..NG-1 of the transposed image stay zero for the whole sweep
+  for (int f = tid; f < (BN / 8) * NG * 8; f += TC_BM) S.qt[f] = 0.f;
+  if (tid == 0) {
+    mbar_init(&S.sdone, 1);
+    mbar_init(&S.gdone, 1);
+    asm volatile("fence.mbarrier_init.release.cluster;" ::: "memory");
+  }
+  if (warp == 0) {
+    asm volatile("tcgen05.alloc.cta_group::1.sync.aligned.shared::cta.b32 [%0], %1;" ::"r"(smem_u32(&S.tmem_base)),
+                 "r"(C::TCOLS));
+    asm volatile("tcgen05.relinquish_alloc_permit.cta_group::1.sync.aligned;");
+  }
+  asm volatile("tcgen05.fence::before_thread_sync;" ::: "memory");
+  __syncthreads();
+  asm volatile("tcgen05.fence::after_thread_sync;" ::: "memory");
+  const uint32_t tmem = S.tmem_base;
+  const uint32_t lane_base = tmem + ((uint32_t)(warp * 32) << 16);
+  const int64_t j = j0 + tid;            // this thread's item = its TMEM lane
+  const int n_tiles = (int)((M + BN - 1) / BN);
+
+  for (int t = 0; t < n_tiles; ++t) {
+    const int64_t i0 = (int64_t)t * BN;
+    // ---- query tile images + its lse / scale / target (rows past M: zero query, zero scale)
+    for (int f = tid; f < BN * KA; f += TC_BM) {
+      const int r = f / KA, a = f % KA;
+      const int64_t i = i0 + r;
+      float4 q0 = make_float4(0.f, 0.f, 0.f, 0.f), q1 = q0;
+      if (i < M) {
+        q0 = __ldg(reinterpret_cast<const float4 *>(Q + i * D + a * 8));
+        q1 = __ldg(reinterpret_cast<const float4 *>(Q + i * D + a * 8) + 1);
+      }
+      const int sw = (r >> 2) & 1;
+      float4 *dst = reinterpret_cast<float4 *>(S.qw + a * (BN * 8) + r * 8);
+      dst[0 ^ sw] = q0;
+      dst[1 ^ sw] = q1;
+      // transposed image: element (dim k, row r) of k-atom r / 8 at row k, chunk (r >> 2) & 1 swizzled by bit 2 of k
+      const float v[8] = {q0.x, q0.y, q0.z, q0.w, q1.x, q1.y, q1.z, q1.w};
+      const int ra = r >> 3, c = (r >> 2) & 1, e = r & 3;
+#pragma unroll
+      for (int kk = 0; kk < 8; ++kk) {
+        const int k = a * 8 + kk;
+        S.qt[(ra * NG + k) * 8 + ((c ^ ((k >> 2) & 1)) << 2) + e] = v[kk];
+      }
+    }
+    for (int r = tid; r < BN; r += TC_BM) {
+      const int64_t i = i0 + r;
+      const bool ok = i < M;
+      S.lse[r] = ok ? lse[i] : 0.f;
+      S.rs[r] = ok ? row_scale[i] : 0.f;
+      S.tg[r] = ok ? targets[i] : -1;
+    }
+    asm volatile("fence.proxy.async.shared::cta;" ::: "memory");
+    asm volatile("tcgen05.fence::before_thread_sync;" ::: "memory");
+    __syncthreads();
+    asm volatile("tcgen05.fence::after_thread_sync;" ::: "memory");
+    // ---- scores S^T = W_slab . Q_tile^T
+    if (warp == 0) {
+      const uint64_t adesc = umma_desc_sw32(S.wa), bdesc = umma_desc_sw32(S.qw);
+#pragma unroll
+      for (int a = 0; a < KA; ++a)
+        umma_tf32_elect(tmem, adesc + (uint64_t)(a * ((TC_BM * 32) >> 4)), bdesc + (uint64_t)(a * ((BN * 32) >> 4)),
+                        IDESC_S, a != 0);
+      umma_commit_elect(&S.sdone);
+    }
+    mbar_wait(&S.sdone, t & 1);
+    asm volatile("tcgen05.fence::after_thread_sync;" ::: "memory");
+    // ---- P^T = g (exp(S^T - lse) - onehot), in place, 32 columns at a time
+#pragma unroll 1
+    for (int c0 = 0; c0 < BN; c0 += 32) {
+      uint32_t v[32];
+      TC_LD32(v, lane_base + (uint32_t)c0);
+      TC_WAIT_LD(v);
+#pragma unroll
+      for (int c = 0; c < 32; ++c) {
+        const float p = __expf(__uint_as_float(v[c]) - S.lse[c0 + c]);
+        v[c] = __float_as_uint(S.rs[c0 + c] * (S.tg[c0 + c] == j ? p - 1.f : p));
+      }
+      C2_ST32(lane_base + (uint32_t)c0, v);
+    }
+    asm volatile("tcgen05.wait::st.sync.aligned;" ::: "memory");
+    asm volatile("tcgen05.fence::before_thread_sync;" ::: "memory");
+    __syncthreads();
+    asm volatile("tcgen05.fence::after_thread_sync;" ::: "memory");
+    // ---- dW_slab += P^T . Qt_tile^T
+    if (warp == 0) {
+      const uint64_t bd0 = umma_desc_sw32(S.qt);
+#pragma unroll
+      for (int a = 0; a < BN / 8; ++a)
+        umma_tf32_ts_elect(tmem + C::DW_COL, tmem + a * 8, bd0 + (uint64_t)(a * ((NG * 32) >> 4)), IDESC_G,
+                           (t == 0 && a == 0) ? 0u : 1u);
+      umma_commit_elect(&S.gdone);
+    }
+    mbar_wait(&S.gdone, t & 1);          // the MMAs have read the tiles and P^T: both may be overwritten
+    asm volatile("tcgen05.fence::after_thread_sync;" ::: "memory");
+  }
+
+  // ---- dW rows of this slab, once
+#pragma unroll 1
+  for (int k0 = 0; k0 < D; k0 += GW) {
+    uint32_t g[GW];
+    c2_ld<GW>(g, lane_base + (uint32_t)(C::DW_COL + k0));
+    c2_wait_ld<GW>(g);
+    if (j < n_rows && n_tiles > 0) {
+#pragma unroll
+      for (int k = 0; k < GW; k += 4)
+        *reinterpret_cast<float4 *>(dW + j * D + k0 + k) =
+            make_float4(__uint_as_float(g[k]), __uint_as_float(g[k + 1]), __uint_as_float(g[k + 2]), __uint_as_float(g[k + 3]));
+    }
+  }
+  asm volatile("tcgen05.fence::before_thread_sync;" ::: "memory");
+  __syncthreads();
+  if (warp == 0) {
+    asm volatile("tcgen05.fence::after_thread_sync;" ::: "memory");
+    asm volatile("tcgen05.dealloc.cta_group::1.sync.aligned.b32 %0, %1;" ::"r"(tmem), "r"(C::TCOLS));
+  }
+}
+
 // ------------------------------------------------------------------ host side
 struct Ce2Plan {
   int n_split;
@@ -687,6 +878,36 @@ int ce_tc_launch(const Table *tc, const float *Q, const int64_t *targets, int64_
     case 128: return ce_tc_launch_d<128>(t, p, Q, targets, M, part, st);
   }
   set_error("ce(tf32): dim %d unsupported (use 8, 16, 32, 64 or 128)", t->dim);
+  return PCV_ERR_UNSUPPORTED;
+}
+
+template <int D>
+static int ce_tc_table_grad_d(const Table *t, const float *Q, const int64_t *targets, const float *lse,
+                              const float *row_scale, int64_t M, float *dW, cudaStream_t st) {
+  static_assert(sizeof(TgSmem<D>) + 1024 <= 227 * 1024, "shared memory of one CTA");
+  const size_t smem = sizeof(TgSmem<D>) + 1024;
+  static bool attr_set[64] = {false};
+  if (!attr_set[t->device & 63]) {
+    PCV_CUDA(cudaFuncSetAttribute(ce_tc_table_grad_kernel<D>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
+    attr_set[t->device & 63] = true;
+  }
+  const unsigned grid = (unsigned)((t->n_rows + TC_BM - 1) / TC_BM);
+  ce_tc_table_grad_kernel<D><<<grid, TC_BM, smem, st>>>(t->W, t->n_rows, Q, targets, lse, row_scale, M, dW);
+  PCV_LAUNCH_CHECK();
+  return PCV_OK;
+}
+
+// tensor-core table gradient (dense mask, dims 8..128): see ce_tc_table_grad_kernel
+int ce_tc_table_grad(const Table *t, const float *Q, const int64_t *targets, const float *lse, const float *row_scale,
+                     int64_t M, float *dW, cudaStream_t st) {
+  switch (t->dim) {
+    case 8: return ce_tc_table_grad_d<8>(t, Q, targets, lse, row_scale, M, dW, st);
+    case 16: return ce_tc_table_grad_d<16>(t, Q, targets, lse, row_scale, M, dW, st);
+    case 32: return ce_tc_table_grad_d<32>(t, Q, targets, lse, row_scale, M, dW, st);
+    case 64: return ce_tc_table_grad_d<64>(t, Q, targets, lse, row_scale, M, dW, st);
+    case 128: return ce_tc_table_grad_d<128>(t, Q, targets, lse, row_scale, M, dW, st);
+  }
+  set_error("ce_table_grad(tf32): dim %d unsupported (use 8, 16, 32, 64 or 128)", t->dim);
   return PCV_ERR_UNSUPPORTED;
 }
 

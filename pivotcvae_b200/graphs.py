@@ -74,7 +74,12 @@ class GraphedTrainStep:
     capturable=True.  Philox masks / eps stay fresh per replay (device-side counter)."""
 
     def __init__(self, model, optimizer, batch, beta, n_neg, warmup=3):
+        from . import _lib
         from .train_generative import get_gen_loss
+        if any(getattr(model, k).weight.requires_grad for k in ("docEmbed", "userEmbed") if hasattr(model, k)):
+            raise _lib.PcvError("GraphedTrainStep: the embedding tables are trainable (fine_tune=True); a captured step "
+                                "would keep reading the table handle (and its packed images) of the capture, which every "
+                                "optimizer step replaces.  Train with fine_tune eagerly.")
         dev = model.docEmbed.weight.device
         L = model.slate_size
         self.model, self.opt = model, optimizer

@@ -47,7 +47,8 @@ class BaseCVAE(nn.Module):
         self.noUser = no_user
         self.device = device
         dev = _require_cuda(device)
-        # frozen, row-L2-normalised copies of the pretrained tables (cvae.py:27-41)
+        # row-L2-normalised copies of the pretrained tables (cvae.py:27-41); fine_tune=True trains both with the rest of
+        # the model (the CE's table gradient is pcv_ce_table_grad, the MLP gathers scatter theirs)
         with torch.no_grad():
             src = embeddings.weight.detach().to(dev, torch.float32)
             self.docEmbed = nn.Embedding(src.shape[0], src.shape[1], device=dev)
@@ -58,9 +59,6 @@ class BaseCVAE(nn.Module):
                 self.userEmbed = nn.Embedding(usrc.shape[0], usrc.shape[1], device=dev)
                 self.userEmbed.weight.data.copy_(ops.normalize_rows(usrc))
                 self.userEmbed.weight.requires_grad = fine_tune
-        if fine_tune:
-            raise L.PcvError("fine_tune=True is not supported: the fused kernels treat the tables as frozen "
-                             "(every reference subclass hard-codes fine_tune=False)")
         self.noise = NoiseSource()
         self.select_engine = "auto"
         self.ce_engine = "exact"   # "tf32": full-catalog CE logits and gradient on the tensor cores, D = 8..128 (reduced-precision tolerance)
@@ -90,11 +88,19 @@ class BaseCVAE(nn.Module):
         queries are all-gathered before every sharded scoring step (a few hundred KB over NVLink)."""
         import torch.distributed as dist
         from ..parallel import shard_bounds
+        if self.trainable_tables():
+            raise L.PcvError("enable_vocab_parallel: the embedding tables are trainable (fine_tune=True); the sharded "
+                             "catalog cross-entropy has no table gradient")
         world, rank = dist.get_world_size(group), dist.get_rank(group)
         lo, hi = shard_bounds(self.docEmbed.weight.shape[0], world, rank)
         self._vp = (group, lo, hi)
         self._vp_rows = bool(shard_rows)
         self._table = None
+
+    def trainable_tables(self):
+        """The embedding tables that require grad (fine_tune=True)."""
+        tabs = [self.docEmbed.weight] + ([] if self.noUser else [self.userEmbed.weight])
+        return [w for w in tabs if w.requires_grad]
 
     def _vp_row_slice(self, B):
         """(world, first row, rows per rank) when recommend() may shard its MLP rows over the vocab-parallel group:
@@ -189,11 +195,12 @@ class BaseCVAE(nn.Module):
 
     def _run_block(self, segs, layers, B, dense=(), **kw):
         """One fused MLP block; differentiable when grad mode is on."""
-        spec = MlpSpec(segs, [a for (_, _, a) in layers], save=torch.is_grad_enabled(), **kw)
+        spec = MlpSpec(segs, [a for (_, _, a) in layers], save=torch.is_grad_enabled(), train_tables=True, **kw)
         flat = []
         for (W, b, _) in layers:
             flat += [W, b]
-        return FusedMLPFn.apply(spec, B, len(dense), *dense, *flat)
+        tables = [segs[i][1] for i in spec.train_segs]          # fine_tune: gather tables that get a gradient
+        return FusedMLPFn.apply(spec, B, len(dense), *dense, *flat, *tables)
 
     def _user_seg(self, u):
         return ("gather", self.userEmbed.weight, u.reshape(-1, 1))
@@ -364,5 +371,5 @@ class BaseCVAE(nn.Module):
         from ..autograd import CandidateLogitsFn, LogitsFn
         if self.candidateFlag:
             cand = candidates.to(self._dev(), torch.int64).reshape(rx_flat.shape[0], -1)
-            return CandidateLogitsFn.apply(rx_flat, self.item_table(), cand)
-        return LogitsFn.apply(rx_flat, self.item_table())
+            return CandidateLogitsFn.apply(rx_flat, self.item_table(), cand, self.docEmbed.weight)
+        return LogitsFn.apply(rx_flat, self.item_table(), self.docEmbed.weight)

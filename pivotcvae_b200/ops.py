@@ -130,6 +130,8 @@ class Table:
             lib = L.load()
             fns = {"select": [lib.pcv_score_select_workspace_bytes], "ce": [lib.pcv_ce_workspace_bytes],
                    "topk": [lib.pcv_score_topk_workspace_bytes],
+                   # table gradient: the dense-mask query, the largest of the mask modes (row-split partials >= gap table)
+                   "ce_tgrad": [lambda h, m, out: lib.pcv_ce_table_grad_workspace_bytes(h, m, ctypes.byref(L.CeMask(1.0)), out)],
                    # no-repeat select: the top-1 workspace followed by the top-k one (include/pcv_b200.h)
                    "select_nr": [lib.pcv_score_select_workspace_bytes, lib.pcv_score_topk_workspace_bytes]}[kind]
             total = 0
@@ -602,11 +604,7 @@ def kl_fwd_bwd(mu, logvar, pmu, plogvar, grads=True):
     return out, g
 
 
-def ce_fwd_bwd(table, Q, targets, keep_prob=1.0, bitmask=None, seed=0, offset=0, want_dq=True, offset_dev=None,
-               engine="exact"):
-    """-> (loss_rows[M], lse[M], dq[M, D] or None); see include/pcv_b200.h."""
-    Q, targets = _f32(Q, "Q"), _i64(targets, "targets").reshape(-1)
-    M, D = Q.shape
+def _ce_mask(table, M, keep_prob, bitmask, seed, offset, offset_dev, engine):
     mask = L.CeMask()
     mask.keep_prob = float(keep_prob)
     if bitmask is not None:
@@ -619,6 +617,15 @@ def ce_fwd_bwd(table, Q, targets, keep_prob=1.0, bitmask=None, seed=0, offset=0,
     mask.seed, mask.offset = int(seed), int(offset)
     mask.offset_dev = offset_dev.data_ptr() if offset_dev is not None else None
     mask.engine = 1 if engine == "tf32" else 0
+    return mask, bitmask
+
+
+def ce_fwd_bwd(table, Q, targets, keep_prob=1.0, bitmask=None, seed=0, offset=0, want_dq=True, offset_dev=None,
+               engine="exact"):
+    """-> (loss_rows[M], lse[M], dq[M, D] or None); see include/pcv_b200.h."""
+    Q, targets = _f32(Q, "Q"), _i64(targets, "targets").reshape(-1)
+    M, D = Q.shape
+    mask, bitmask = _ce_mask(table, M, keep_prob, bitmask, seed, offset, offset_dev, engine)
     loss = torch.empty(M, dtype=torch.float32, device=Q.device)
     lse = torch.empty(M, dtype=torch.float32, device=Q.device)
     dq = torch.empty(M, D, dtype=torch.float32, device=Q.device) if want_dq else None
@@ -627,6 +634,38 @@ def ce_fwd_bwd(table, Q, targets, keep_prob=1.0, bitmask=None, seed=0, offset=0,
         L.check(L.load().pcv_ce_fwd_bwd(table.handle, _ptr(Q), _ptr(targets), M, ctypes.byref(mask), _ptr(loss),
                                         _ptr(lse), _ptr(dq), _ptr(ws), ws.numel(), _stream()), "pcv_ce_fwd_bwd")
     return loss, lse, dq
+
+
+def ce_table_grad(table, Q, targets, lse, row_scale, keep_prob=1.0, bitmask=None, seed=0, offset=0, offset_dev=None,
+                  engine="exact"):
+    """dW [n_rows, D] = d (sum_i row_scale[i] loss_rows[i]) / d table for the mask of the matching ce_fwd_bwd call;
+    see include/pcv_b200.h pcv_ce_table_grad."""
+    Q, targets = _f32(Q, "Q"), _i64(targets, "targets").reshape(-1)
+    lse, row_scale = _f32(lse, "lse"), _f32(row_scale, "row_scale")
+    M = Q.shape[0]
+    mask, bitmask = _ce_mask(table, M, keep_prob, bitmask, seed, offset, offset_dev, engine)
+    dW = torch.empty(table.n_rows, table.dim, dtype=torch.float32, device=Q.device)
+    ws = table.workspace("ce_tgrad", M)
+    with torch.cuda.device(Q.device), _timed("ce_table_grad"):
+        L.check(L.load().pcv_ce_table_grad(table.handle, _ptr(Q), _ptr(targets), M, ctypes.byref(mask), _ptr(lse),
+                                           _ptr(row_scale), _ptr(dW), _ptr(ws), ws.numel(), _stream()), "pcv_ce_table_grad")
+    return dW
+
+
+def cand_ce_table_grad(table, Q, candidates, target_pos, lse, row_scale):
+    """dW [n_rows, D] (zero-filled here) += the candidate-mode CE gradient w.r.t. the table rows each row's candidate
+    list names; see include/pcv_b200.h pcv_cand_ce_table_grad."""
+    Q = _f32(Q, "Q")
+    M = Q.shape[0]
+    candidates = _i64(candidates, "candidates").reshape(M, -1)
+    target_pos = _i64(target_pos, "target_pos").reshape(-1)
+    lse, row_scale = _f32(lse, "lse"), _f32(row_scale, "row_scale")
+    dW = torch.zeros(table.n_rows, table.dim, dtype=torch.float32, device=Q.device)
+    with torch.cuda.device(Q.device), _timed("cand_ce_table_grad"):
+        L.check(L.load().pcv_cand_ce_table_grad(table.handle, _ptr(Q), _ptr(candidates), _ptr(target_pos), M,
+                                                candidates.shape[1], _ptr(lse), _ptr(row_scale), _ptr(dW), _stream()),
+                "pcv_cand_ce_table_grad")
+    return dW
 
 
 def ce_partials(shard, Q, targets, engine="exact"):

@@ -9,6 +9,7 @@ reference's semantics (CE mean over B*L rows, KL summed, Adam without decay).
 import numpy as np
 import torch
 
+from ._lib import PcvError
 from .autograd import CatalogCEFn, KLFn  # noqa: F401
 from .env.response_model import sample_users
 from .models.listcvae import UserListCVAEWithPrior
@@ -46,11 +47,14 @@ def get_gen_loss(batch_data, model, lossFun, beta, n_neg=1000):
         M = slates.numel()
         cand = _as_tensor(batch_data["sample_candidates"], torch.int64, dev).reshape(M, -1)
         tpos = _as_tensor(batch_data["sample_targets"], torch.int64, dev).reshape(-1)
-        recLoss = CandidateCEFn.apply(rx.reshape(M, -1), model.item_table(), cand, tpos)
+        recLoss = CandidateCEFn.apply(rx.reshape(M, -1), model.item_table(), cand, tpos, model.docEmbed.weight)
         KLD = KLFn.apply(mu, logvar, pMu, pLogvar)
         model.noise.flush_eager()
         return recLoss + beta * KLD, recLoss, KLD
     vp = getattr(model, "_vp", None)
+    if vp is not None and model.docEmbed.weight.requires_grad:
+        raise PcvError("get_gen_loss: vocab-parallel training needs frozen tables (fine_tune=False): the sharded "
+                       "catalog cross-entropy has no table gradient")
     table = model.full_table() if vp is not None else model.item_table()
     N = table.n_rows
     if n_neg > N:
@@ -69,7 +73,8 @@ def get_gen_loss(batch_data, model, lossFun, beta, n_neg=1000):
                                                 slates.reshape(-1), vp[0], getattr(model, "ce_engine", "exact"))
     else:
         recLoss, _, _ = CatalogCEFn.apply(rx.reshape(M, -1), table, slates.reshape(-1), keep, bitmask, kw["seed"],
-                                          kw["offset"], kw.get("offset_dev"), getattr(model, "ce_engine", "exact"))
+                                          kw["offset"], kw.get("offset_dev"), getattr(model, "ce_engine", "exact"),
+                                          model.docEmbed.weight)
     KLD = KLFn.apply(mu, logvar, pMu, pLogvar)
     loss = recLoss + beta * KLD
     model.noise.flush_eager()
