@@ -16,7 +16,8 @@
  *    *_workspace_bytes() queries.  The one exception is pcv_table_create, a
  *    one-off constructor: it synchronises the device and allocates the handle's
  *    packed table copies (freed by pcv_table_destroy); a failure there is an
- *    error, never a silent downgrade to a slower engine;
+ *    error, never a silent downgrade to a slower engine.  pcv_table_refresh
+ *    brings those copies up to date on a stream without either;
  *  - float = IEEE binary32, indices = int64 (torch.long), row-major tensors.
  *  - there is no CPU fallback: a non-sm_100 device yields PCV_ERR_ARCH.
  */
@@ -52,7 +53,7 @@ int64_t pcv_launch_count(void);
 int pcv_counter_add(uint64_t *counter, uint64_t inc, pcv_stream_t stream);
 
 /* ------------------------------------------------------------------ */
-/* Item table (the frozen, row-L2-normalised catalog; cvae.py:27-33)   */
+/* Item table (the row-L2-normalised catalog; cvae.py:27-33)           */
 /* ------------------------------------------------------------------ */
 typedef struct pcv_table pcv_table;
 
@@ -61,11 +62,20 @@ typedef struct pcv_table pcv_table;
  * pcv_score_select are global (= local + row_offset).  The table is borrowed,
  * not copied: it must outlive the handle.  dim must be a multiple of 4, <= 128.
  * The handle owns the packed images the tensor-core engines stream with TMA: dim 8/16/32/64/128 the pre-swizzled fp32
- * copy (dim * 4 bytes per row), dim 8 with row norms in (0, 1e4) also the f16 image of the f16 filter (32 bytes per
- * row); they are snapshots: re-create the handle after the table changes. */
+ * copy (dim * 4 bytes per row), dim 8 with row norms in (0, 1e4) at creation also the f16 image of the f16 filter (32
+ * bytes per row), and a device scalar holding max_j |w_j|_2 that the kernels read.  They are derived from W's values:
+ * after W changes in place, call pcv_table_refresh (or re-create the handle when W moves or changes shape). */
 int pcv_table_create(const float *W, int64_t n_rows, int dim, int64_t row_offset,
                      pcv_table **out);
 void pcv_table_destroy(pcv_table *t);
+/* W was updated in place (same pointer, n_rows and dim, e.g. by an optimizer step): re-derive on `stream` everything
+ * the handle derived from its values -- max|w|, the pre-swizzled image, the f16 image and the tf32 CE's transposed
+ * image when the handle has them (a transposed image not built yet stays lazy).  One pass over W plus a one-thread
+ * kernel; no allocation, no synchronisation, no host copy, so it may be captured in a CUDA graph.  Afterwards every
+ * entry point gives bit for bit the results of a handle freshly created on the same W.  Whether an f16 image exists
+ * stays as decided at creation: if max|w| leaves (0, 1e4) the f16 filter flags every stream for the exact re-scan
+ * (exact, slow). */
+int pcv_table_refresh(pcv_table *t, pcv_stream_t stream);
 /* F.normalize(W, p=2, dim=1, eps=1e-12) row-wise, out-of-place (cvae.py:31,39). */
 int pcv_normalize_rows(const float *W, int64_t n_rows, int dim, float *out,
                        pcv_stream_t stream);
@@ -324,11 +334,12 @@ typedef struct {
   const uint64_t *offset_dev; /* optional device counter added to `offset` (CUDA-graph replays) */
   int engine;              /* PCV_CE_ENGINE_*: EXACT (default) or TF32 (dense mask, dim 8, 16, 32, 64 or 128: logits
                               AND the gradient contraction on the tensor cores, loss ~1e-4 / dq ~1e-3 relative — the
-                              reduced-precision tolerance; other dims return PCV_ERR_UNSUPPORTED).  The first TF32
+                              reduced-precision tolerance, reproducible bit for bit; other dims return
+                              PCV_ERR_UNSUPPORTED).  The first TF32
                               call on a table handle builds its transposed tile image (one-off allocation + device
                               sync, like pcv_table_create): run it once outside any CUDA-graph capture.  The handle
-                              keeps that image until it is destroyed: n_rows * dim * 4 bytes (rounded up to whole
-                              tiles) at dim >= 16, twice that at dim 8 */
+                              keeps that image until it is destroyed (pcv_table_refresh keeps it current): n_rows *
+                              dim * 4 bytes (rounded up to whole tiles) at dim >= 16, twice that at dim 8 */
 } pcv_ce_mask;
 #define PCV_CE_ENGINE_EXACT 0
 #define PCV_CE_ENGINE_TF32 1

@@ -85,6 +85,7 @@ EXPORTS = {
     "pcv_counter_add": (c_int, [c_void_p, c_uint64, c_void_p]),
     "pcv_table_create": (c_int, [c_void_p, c_int64, c_int, c_int64, ctypes.POINTER(c_void_p)]),
     "pcv_table_destroy": (None, [c_void_p]),
+    "pcv_table_refresh": (c_int, [c_void_p, c_void_p]),
     "pcv_normalize_rows": (c_int, [c_void_p, c_int64, c_int, c_void_p, c_void_p]),
     "pcv_score_select_workspace_bytes": (c_int, [c_void_p, c_int64, ctypes.POINTER(c_size_t)]),
     "pcv_score_select": (c_int, [c_void_p, c_void_p, c_int64, ctypes.POINTER(SelectOpts), c_void_p,

@@ -27,7 +27,7 @@
 // ce_finalize_kernel (target logit re-derived with the exact fp32 FMA chain).
 #include <mutex>
 
-#include "tc_common.cuh"
+#include "table_images.cuh"
 
 namespace pcv {
 
@@ -47,8 +47,8 @@ constexpr int C2_THREADS = 64 + 32 * C2_EPI_WARPS;
 template <int D>
 struct Ce2Cfg {
   static constexpr int KA = D / 8;                                 // k-atoms (8 fp32 = 32 B) of an embedding row
-  static constexpr int BN = D <= 32 ? 128 : D == 64 ? 64 : 32;     // items per tile (= TMEM columns of one S/P buffer)
-  static constexpr int NG = D < 16 ? 16 : D;                       // N of the gradient MMA
+  static constexpr int BN = WtGeom<D>::BN;                         // items per tile (= TMEM columns of one S/P buffer)
+  static constexpr int NG = WtGeom<D>::NG;                         // N of the gradient MMA
   static constexpr int STAGES = D == 8 ? 12 : D == 16 ? 10 : D == 32 ? 5 : 4;
   static constexpr int A_BUFS = D <= 64 ? 2 : 1;
   // N = 16 gradient MMAs are 8 cycles of work each: four independent accumulators keep the tensor pipe from waiting on
@@ -76,7 +76,7 @@ struct __align__(1024) Ce2Smem {
   float a[C::A_BUFS][C::A_FLOATS];
   unsigned long long full[C::STAGES], empty[C::STAGES], tfull[C2_BUFS], pfull[C2_BUFS], tempty[C2_BUFS];
   unsigned long long afull[C::A_BUFS], aempty[C::A_BUFS], dqfull, dqempty;
-  float lsum[2][TC_BM];      // per-row sum of l over the column slices 1..3 of a work item (double-buffered by item parity)
+  float lsum[2][3][TC_BM];   // per-row l of the column slices 1..3 of a work item (double-buffered by item parity)
   uint32_t tmem_base;
 };
 
@@ -186,7 +186,8 @@ __device__ __forceinline__ float c2_dot(const float *__restrict__ q, const float
 // ---- per-row reference exponent + safety flag (see the header)
 template <int D>
 __global__ void __launch_bounds__(256)
-ce_ref_kernel(const float *__restrict__ W, int64_t n_rows, int64_t row_offset, float max_row_norm, const float *__restrict__ Q,
+ce_ref_kernel(const float *__restrict__ W, int64_t n_rows, int64_t row_offset, const float *__restrict__ max_row_norm,
+              const float *__restrict__ Q,
               const int64_t *__restrict__ targets, int64_t M, float *__restrict__ cref, unsigned char *__restrict__ unsafe) {
   const int lane = threadIdx.x & 31;
   const int64_t row = (int64_t)blockIdx.x * (blockDim.x >> 5) + (threadIdx.x >> 5);
@@ -198,7 +199,7 @@ ce_ref_kernel(const float *__restrict__ W, int64_t n_rows, int64_t row_offset, f
   lb = warp_max(lb);
   if (lane == 0) {
     const float ss = c2_dot<D>(q, q);
-    const float ub = sqrtf(ss) * max_row_norm * 1.01f + 1e-30f;   // >= every tf32 logit (truncation only shrinks |s|)
+    const float ub = sqrtf(ss) * __ldg(max_row_norm) * 1.01f + 1e-30f;   // >= every tf32 logit (truncation only shrinks |s|)
     lb -= 0.01f * ub;                                              // the tf32 logit of that item may sit a little lower
     const bool ok = lb >= ub - 140.f && ub < 1.0e30f;
     cref[row] = ok ? fmaxf(lb, ub - 60.f) : 0.f;
@@ -259,20 +260,13 @@ ce_rowfix_kernel(const float *__restrict__ W, int64_t n_rows, const float *__res
   }
 }
 
-// Transposed, pre-swizzled image of the table for the gradient MMA's B operand: per BN-item tile, BN / 8 k-atoms (8
-// items each) of [NG rows x 32 B]: row r < D = embedding dimension r (rows D..15 zero at D = 8); the two 16-byte chunks
-// of a row are swapped when bit 2 of r is set (SWIZZLE_32B).  The buffer is zero-filled first (padding rows, tail of
-// the last tile).  One thread per table element.
+// Transposed, pre-swizzled image of the table for the gradient MMA's B operand (layout: wt_index).  The buffer is
+// zero-filled first (padding rows, tail of the last tile).  One thread per table element.
 template <int D>
 __global__ void pack_wt_kernel(const float *__restrict__ W, int64_t n_rows, float *__restrict__ out) {
-  using C = Ce2Cfg<D>;
   const int64_t f = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
   if (f >= n_rows * D) return;
-  const int64_t j = f / D;
-  const int r = (int)(f % D);
-  const int64_t tile = j / C::BN;
-  const int i = (int)(j % C::BN), a = i >> 3, c = (i >> 2) & 1, e = i & 3;
-  out[((tile * (C::BN / 8) + a) * C::NG + r) * 8 + ((c ^ ((r >> 2) & 1)) << 2) + e] = W[f];
+  out[wt_index<D>(f / D, (int)(f % D))] = W[f];
 }
 
 // 18 warps on the 4 SM sub-partitions (16 K registers each, five warps on two of them) allow 96 registers a thread
@@ -293,7 +287,6 @@ ce_tc2_kernel(const float *__restrict__ Wsw, const float *__restrict__ Wt, int64
   const int hw_warp = threadIdx.x >> 5;
   const int warp = hw_warp >= C2_EPI_WARPS ? hw_warp - C2_EPI_WARPS : hw_warp + 2;
 
-  if (threadIdx.x < 2 * TC_BM) (&S.lsum[0][0])[threadIdx.x] = 0.f;
   if (threadIdx.x == 0) {
     for (int s = 0; s < STAGES; ++s) { mbar_init(&S.full[s], 1); mbar_init(&S.empty[s], 1); }
     for (int b = 0; b < C2_BUFS; ++b) {
@@ -525,14 +518,15 @@ ce_tc2_kernel(const float *__restrict__ Wsw, const float *__restrict__ Wt, int64
         __syncwarp();
         if (lane == 0) mbar_arrive(&S.dqempty);
       }
-      // ONE record per (split, row): the other three column slices add their l into shared memory, a named barrier
-      // over the four warps of this TMEM lane quarter orders it, the slice-0 warp writes the record
-      float *ls = &S.lsum[it & 1][trow];
-      if (slice != 0) atomicAdd(ls, l);
+      // ONE record per (split, row): the other three column slices store their l in shared memory, a named barrier
+      // over the four warps of this TMEM lane quarter orders it, the slice-0 warp adds them in slice order (a fixed
+      // order: the records, and with them loss and lse, are reproducible bit for bit) and writes the record.  Each
+      // buffer is written again two items later, behind the next item's barrier
+      float (&ls)[3][TC_BM] = S.lsum[it & 1];
+      if (slice != 0) ls[slice - 1][trow] = l;
       asm volatile("bar.sync %0, 128;" ::"r"(1 + quarter) : "memory");
       if (slice == 0) {
-        l += *ls;
-        *ls = 0.f;             // this buffer is used again two items later, behind the next item's barrier
+        l += (ls[0][trow] + ls[1][trow]) + ls[2][trow];
         if (row < M) {
           rec[0] = __ldg(cref + row);
           rec[1] = l;
@@ -841,7 +835,7 @@ static int ce_tc_launch_d(Table *t, const Ce2Plan &p, const float *Q, const int6
   float *cref = reinterpret_cast<float *>(reinterpret_cast<char *>(part) + p.rec_bytes);
   unsigned char *unsafe = reinterpret_cast<unsigned char *>(cref) + (((size_t)M * 4 + 255) & ~(size_t)255);
   const int n_streams = p.n_split;
-  ce_ref_kernel<D><<<(unsigned)((M + 7) / 8), 256, 0, st>>>(t->W, t->n_rows, t->row_offset, t->max_row_norm, Q, targets, M,
+  ce_ref_kernel<D><<<(unsigned)((M + 7) / 8), 256, 0, st>>>(t->W, t->n_rows, t->row_offset, t->max_row_norm_dev(), Q, targets, M,
                                                             cref, unsafe);
   PCV_LAUNCH_CHECK();
   static_assert(sizeof(Ce2Smem<D>) + 1024 <= 227 * 1024, "shared memory of one CTA");

@@ -28,7 +28,11 @@ struct Table {
                      // the table at D >= 16 (twice at D = 8)
   void *packed_h;    // D = 8: f16 image (8 dims + constant dimension, SWIZZLE_32B) for the f16 filter (score_select_tc.cu)
   int tmap_valid;  // 1 when the tcgen05 engine can serve this table
-  float max_row_norm;  // max_j |w_j|_2 (error bound of the tf32 filter)
+  float max_row_norm;  // max_j |w_j|_2 (error bound of the tf32 filter) at creation: decides whether packed_h exists
+  // device words: [0] running max of |w_j|^2 (ordered uint bits, zero between refreshes), [1] max_j |w_j|_2 as a float,
+  // written by pcv_table_create and pcv_table_refresh; the kernels read max|w| from there, never from the host copy
+  unsigned int *norm_dev;
+  const float *max_row_norm_dev() const { return reinterpret_cast<const float *>(norm_dev + 1); }
   int tc_chunk_tiles;  // tcgen05 filter: tiles per column chunk once the table outgrows the L2
 };
 

@@ -46,7 +46,8 @@ __device__ __forceinline__ float chain_score(const float *__restrict__ q, const 
 
 template <int D>
 __global__ void __launch_bounds__(32)
-sigmoid_categorical_kernel(const float *__restrict__ W, int64_t n_rows, float max_row_norm, const float *__restrict__ Q,
+sigmoid_categorical_kernel(const float *__restrict__ W, int64_t n_rows, const float *__restrict__ max_row_norm,
+                           const float *__restrict__ Q,
                            int64_t M, uint64_t seed, uint64_t offset, const uint64_t *__restrict__ offset_dev,
                            int64_t *__restrict__ out_idx, int32_t *__restrict__ out_iters) {
   const int64_t row = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
@@ -61,7 +62,7 @@ sigmoid_categorical_kernel(const float *__restrict__ W, int64_t n_rows, float ma
   float ss = 0.f;
 #pragma unroll
   for (int k = 0; k < D; ++k) ss = fmaf(q[k], q[k], ss);
-  const float sigma_b = pcv_sigmoidf(sqrtf(ss) * max_row_norm * 1.0001f + 1e-6f);
+  const float sigma_b = pcv_sigmoidf(sqrtf(ss) * __ldg(max_row_norm) * 1.0001f + 1e-6f);
   const uint64_t r = (uint64_t)row + offset;
   const uint64_t N = (uint64_t)n_rows;
   const uint64_t lemire_t = (0ull - N) % N;     // 2^64 mod N
@@ -128,7 +129,7 @@ extern "C" int pcv_sigmoid_categorical(const pcv_table *th, const float *Q, int6
   const unsigned grid = (unsigned)((M + 31) / 32);   // one warp per CTA: rows finish independently, CTAs spread over the SMs
 #define PCV_SAMPLE_CASE(DD)                                                                                          \
   case DD:                                                                                                           \
-    sigmoid_categorical_kernel<DD><<<grid, 32, 0, st>>>(t->W, t->n_rows, t->max_row_norm, Q, M, seed, offset,       \
+    sigmoid_categorical_kernel<DD><<<grid, 32, 0, st>>>(t->W, t->n_rows, t->max_row_norm_dev(), Q, M, seed, offset, \
                                                          offset_dev, out_idx, out_iters);                            \
     break;
   switch (t->dim) {

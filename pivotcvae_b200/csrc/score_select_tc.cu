@@ -35,7 +35,7 @@
 #include <cstdlib>
 #include <cuda_fp16.h>
 
-#include "tc_common.cuh"
+#include "table_images.cuh"
 
 namespace pcv {
 
@@ -252,7 +252,7 @@ template <int KA, bool F16 = false>
 __global__ void __launch_bounds__(SEL_THREADS, 1)
 score_select_tc_kernel(const float *__restrict__ Wsw, const float *__restrict__ W, int64_t n_rows,
                        const float *__restrict__ Q, int64_t M, int T, int Tc, int row_tiles, int slots_max,
-                       float band_scale /* F16: max|w| * 1.003 */, float *__restrict__ out_r, int32_t *__restrict__ out_cnt,
+                       const float *__restrict__ max_row_norm /* the handle's device scalar */, float *__restrict__ out_r, int32_t *__restrict__ out_cnt,
                        unsigned long long *__restrict__ out_ent, unsigned long long *__restrict__ row_best,
                        unsigned long long *__restrict__ ovf_ent, int32_t *__restrict__ ovf_row, unsigned int ovf_cta_cap) {
   using C = TcCfg<KA>;
@@ -263,6 +263,10 @@ score_select_tc_kernel(const float *__restrict__ Wsw, const float *__restrict__ 
 
   const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
   if (threadIdx.x == 0) TC_TRACE(0);
+  const float wmax = __ldg(max_row_norm);
+  const float band_scale = tc_band_scale(F16, wmax);   // F16: max|w| * 1.003
+  // f16 filter on a table refreshed out of the f16 range: every stream is flagged, the refine scans them exactly
+  const bool flag_all = F16 && !tc_f16_in_range(wmax);
 
   if (threadIdx.x == 0) {
     S.ovf_n = 0u;
@@ -620,7 +624,7 @@ score_select_tc_kernel(const float *__restrict__ Wsw, const float *__restrict__ 
           }
         }
         out_r[stream * M + row] = r;
-        out_cnt[stream * M + row] = ovf ? -1 : min(k, TC_OUT);
+        out_cnt[stream * M + row] = (ovf || flag_all) ? -1 : min(k, TC_OUT);
       }
       if (threadIdx.x == 64) TC_TRACE(13);
     }
@@ -665,7 +669,8 @@ extern "C" int pcv_debug_tc_cta(long long *host4x256) {
 template <int D>
 __global__ void __launch_bounds__(256, D <= 16 ? 5 : 4)
 tc_refine_kernel(const float *__restrict__ W, int64_t n_rows, int64_t row_offset, const float *__restrict__ Q,
-                 int64_t M, int T, int Tc, int row_tiles, int slots_max, int G, float band_scale, float band_const,
+                 int64_t M, int T, int Tc, int row_tiles, int slots_max, int G, const float *__restrict__ max_row_norm,
+                 float band_const,
                  const float *__restrict__ out_r, const int32_t *__restrict__ out_cnt,
                  const unsigned long long *__restrict__ out_ent, unsigned long long *__restrict__ row_best,
                  unsigned int *__restrict__ ovf_count_reset, int64_t *__restrict__ out_idx,
@@ -725,7 +730,7 @@ tc_refine_kernel(const float *__restrict__ W, int64_t n_rows, int64_t row_offset
   }
   // (f16 filter: the running maxima and the recorded approximate maxima live in the scaled, shifted domain of that
   // filter, where the band is a constant)
-  const float band = band_const > 0.f ? band_const : band_scale * sqrtf(ss) * 1.0001f + 1e-37f;
+  const float band = band_const > 0.f ? band_const : tc_band_scale(false, __ldg(max_row_norm)) * sqrtf(ss) * 1.0001f + 1e-37f;
   R = warp_max(R);
   const float thr = R - band;
   float best = -INFINITY;
@@ -860,32 +865,22 @@ size_t score_select_tc_workspace(const Table *t, int64_t M) {
   return p.ws_bytes;
 }
 
-// Pre-swizzled image of the table.  Per 256-row tile and k-atom a (8 consecutive fp32 of a row) a [256][32 B] block in
-// which the two 16-byte chunks of a row are swapped when bit 2 of the row index is set (Swizzle<1,4,3>: address bit 4 ^=
-// bit 7); the ka atoms of a tile follow each other.  D = 8 (ka = 1): row j simply keeps its 32 bytes, chunks swapped.
+// Pre-swizzled image of the table (layout: sw32_chunk_index).  D = 8 (ka = 1): row j simply keeps its 32 bytes,
+// chunks swapped.
 __global__ void pack_sw32_kernel(const float4 *__restrict__ W, int64_t n_rows, int ka, float4 *__restrict__ out) {
   const int64_t f = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;  // 16-byte chunk index of W
   if (f >= n_rows * 2 * ka) return;
   const int64_t j = f / (2 * ka);
   const int a = (int)(f % (2 * ka)) >> 1;
   const int c = (int)(f & 1);
-  out[((j >> 8) * ka + a) * (TC_BN * 2) + (j & (TC_BN - 1)) * 2 + (c ^ (int)((j >> 2) & 1))] = W[f];
+  out[sw32_chunk_index(j, a, c, ka)] = W[f];
 }
 
-// f16 image of a D = 8 table for the f16 filter: row j = 16 f16 (8 dimensions, then the constant dimension 1 and zeros)
-// = 32 B, the two 16-byte halves swapped when bit 2 of the row index is set (the same SWIZZLE_32B rule)
+// f16 image of a D = 8 table for the f16 filter (layout: h16_store_row)
 __global__ void pack_h16_kernel(const float4 *__restrict__ W, int64_t n_rows, uint4 *__restrict__ out) {
   const int64_t j = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
   if (j >= n_rows) return;
-  const float4 w0 = W[2 * j], w1 = W[2 * j + 1];
-  const __half2 h0 = __floats2half2_rn(w0.x, w0.y), h1 = __floats2half2_rn(w0.z, w0.w);
-  const __half2 h2 = __floats2half2_rn(w1.x, w1.y), h3 = __floats2half2_rn(w1.z, w1.w);
-  const uint4 lo = make_uint4(*reinterpret_cast<const uint32_t *>(&h0), *reinterpret_cast<const uint32_t *>(&h1),
-                              *reinterpret_cast<const uint32_t *>(&h2), *reinterpret_cast<const uint32_t *>(&h3));
-  const uint4 hi = make_uint4(0x00003C00u, 0u, 0u, 0u);
-  const int sw = (int)((j >> 2) & 1);
-  out[2 * j + (0 ^ sw)] = lo;
-  out[2 * j + (1 ^ sw)] = hi;
+  h16_store_row(out, j, W[2 * j], W[2 * j + 1]);
 }
 
 int table_init_tc(Table *t) {
@@ -979,8 +974,9 @@ static int score_select_tc_impl(const Table *t, const float *Q, int64_t M, int64
     attr_set[t->device & 63] = true;
   }
   // |tf32 chain - fp32 chain| <= 1.25 * 2^-9 * |q| * max|w|; the band is twice that.  The f16 filter gets max|w| (+0.3 %)
-  // instead: it scales every query row into a fixed range, where its band is the constant TC_H_BAND
-  const float band_scale = F16 ? t->max_row_norm * 1.003f : 2.0f * 1.25f * 0.001953125f * t->max_row_norm;
+  // instead: it scales every query row into a fixed range, where its band is the constant TC_H_BAND.  Both kernels read
+  // max|w| from the handle's device scalar (tc_band_scale), so a refresh on the stream reaches a captured graph too
+  const float *wmax = t->max_row_norm_dev();
   const float *Wsw = F16 ? reinterpret_cast<const float *>(t->packed_h) : t->packed;
   for (int64_t r0 = 0; r0 < M; r0 += Mg) {   // row groups reuse the workspace back to back on the stream
     const int64_t m = (M - r0 < Mg) ? (M - r0) : Mg;
@@ -996,11 +992,11 @@ static int score_select_tc_impl(const Table *t, const float *Q, int64_t M, int64
     int32_t *cc = reinterpret_cast<int32_t *>(rr + n_sr);              // [n_sr]
     int32_t *ovf_row = cc + n_sr;                                      // [ovf_cap]
     score_select_tc_kernel<KA, F16><<<(unsigned)g.grid, SEL_THREADS, smem, st>>>(Wsw, t->W, t->n_rows, Qg, m, g.T, g.Tc, g.row_tiles,
-                                                                       g.slots, band_scale, rr, cc, ent, row_best, ovf_ent,
+                                                                       g.slots, wmax, rr, cc, ent, row_best, ovf_ent,
                                                                        ovf_row, g.ovf_cap / (unsigned)g.grid);
     PCV_LAUNCH_CHECK();
     tc_refine_kernel<D><<<(unsigned)((m + 7) / 8), 256, 0, st>>>(t->W, t->n_rows, t->row_offset, Qg, m, g.T, g.Tc, g.row_tiles,
-                                                             g.slots, g.grid, band_scale, F16 ? TC_H_BAND : 0.f, rr, cc, ent, row_best, ovf_count, out_idx + r0,
+                                                             g.slots, g.grid, wmax, F16 ? TC_H_BAND : 0.f, rr, cc, ent, row_best, ovf_count, out_idx + r0,
                                                              out_val ? out_val + r0 : nullptr);
     if (cudaPeekAtLastError() != cudaSuccess) {
       // the filter ran but the kernel that re-zeroes the head did not launch: heal the workspace here, so that a

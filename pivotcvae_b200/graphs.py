@@ -71,15 +71,21 @@ class GraphedSlateGenerator:
 class GraphedTrainStep:
     """One training step (get_gen_loss -> backward -> Adam.step, train_generative.py:124-134)
     captured as ONE CUDA graph over static batch buffers.  The optimizer must be built with
-    capturable=True.  Philox masks / eps stay fresh per replay (device-side counter)."""
+    capturable=True.  Philox masks / eps stay fresh per replay (device-side counter).
 
-    def __init__(self, model, optimizer, batch, beta, n_neg, warmup=3):
+    train_tables=True captures a fine_tune step too (trainable docEmbed / userEmbed): the step ends by refreshing the
+    item-table handle in place (pcv_table_refresh) after the optimizer has updated docEmbed, so the next replay's
+    cross-entropy reads packed images and a max|w| that match the table.  userEmbed has no handle: only the fused MLP
+    gathers read it."""
+
+    def __init__(self, model, optimizer, batch, beta, n_neg, warmup=3, train_tables=False):
         from . import _lib
         from .train_generative import get_gen_loss
-        if any(getattr(model, k).weight.requires_grad for k in ("docEmbed", "userEmbed") if hasattr(model, k)):
-            raise _lib.PcvError("GraphedTrainStep: the embedding tables are trainable (fine_tune=True); a captured step "
-                                "would keep reading the table handle (and its packed images) of the capture, which every "
-                                "optimizer step replaces.  Train with fine_tune eagerly.")
+        trainable = any(getattr(model, k).weight.requires_grad for k in ("docEmbed", "userEmbed") if hasattr(model, k))
+        if trainable and not train_tables:
+            raise _lib.PcvError("GraphedTrainStep: the embedding tables are trainable (fine_tune=True); pass "
+                                "train_tables=True to capture a step that refreshes the item-table handle after every "
+                                "optimizer step, or train with fine_tune eagerly.")
         dev = model.docEmbed.weight.device
         L = model.slate_size
         self.model, self.opt = model, optimizer
@@ -87,11 +93,17 @@ class GraphedTrainStep:
                        "users": torch.zeros(batch, 1, dtype=torch.int64, device=dev),
                        "responses": torch.zeros(batch, L, device=dev)}
 
+        # the one handle every replay reads (and refreshes); kept alive with the graph that baked its pointers in
+        self._table = model.item_table() if trainable else None
+
         def step():
             optimizer.zero_grad(set_to_none=True)
             loss, rec, kld = get_gen_loss(self.static, model, None, beta, n_neg=n_neg)
             loss.backward()
             optimizer.step()
+            if self._table is not None:     # docEmbed moved in place: bring the handle along, once per step
+                self._table.refresh()
+                self._mark_current()
             model.noise.end_graph_step()
             return loss.detach(), rec.detach(), kld.detach()
 
@@ -115,6 +127,9 @@ class GraphedTrainStep:
                     for k, v in optimizer.state.get(p, {}).items():
                         if torch.is_tensor(v):
                             v.copy_(ss[k]) if k in ss else v.zero_()   # state created by the warm-up starts at zero
+            if self._table is not None:     # the restore changed docEmbed in place: the first replay reads the handle
+                self._table.refresh()
+                self._mark_current()
         torch.cuda.current_stream(dev).wait_stream(side)
         torch.cuda.synchronize(dev)
         self.graph = torch.cuda.CUDAGraph()
@@ -125,7 +140,13 @@ class GraphedTrainStep:
         model.item_table().pin_workspaces()
         ops.pin_packed()
 
+    def _mark_current(self):
+        """The handle matches docEmbed as it is now: item_table() must not refresh it again."""
+        self._table.version = self.model.docEmbed.weight._version
+
     def __call__(self, batch):
+        if self._table is not None and self._table is not self.model.item_table():
+            raise RuntimeError("GraphedTrainStep: docEmbed was re-allocated or reshaped since the capture; build a new step")
         for k, v in self.static.items():
             v.copy_(batch[k].reshape(v.shape), non_blocking=True)
         self.graph.replay()
@@ -133,4 +154,6 @@ class GraphedTrainStep:
         # counters so every cache keyed on them (packed weights, concatenated heads) refreshes on next use
         for p in self._params:
             torch.autograd.graph.increment_version(p)
+        if self._table is not None:     # ... except the item-table handle: the replay's last node refreshed it
+            self._mark_current()
         return self.loss, self.rec, self.kld

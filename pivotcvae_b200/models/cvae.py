@@ -147,10 +147,13 @@ class BaseCVAE(nn.Module):
             return self.item_table()
         w = self.docEmbed.weight
         t = getattr(self, "_full", None)
-        if t is None or t.weight.data_ptr() != w.data_ptr() or t.n_rows != w.shape[0] or t.version != w._version:
+        if t is None or t.weight.data_ptr() != w.data_ptr() or t.weight.shape != w.shape:
             t = ops.Table(w.detach())
             t.version = w._version
             self._full = t
+        elif t.version != w._version:   # updated in place (an optimizer step): refresh the handle on the stream
+            t.refresh()
+            t.version = w._version
         return t
 
     def item_table(self):
@@ -159,15 +162,21 @@ class BaseCVAE(nn.Module):
         if self._vp is not None:
             _, lo, hi = self._vp
             if (t is None or t.row_offset != lo or t.n_rows != hi - lo or t.weight.data_ptr() != w[lo:hi].data_ptr()
-                    or t.version != w._version):
+                    or t.dim != w.shape[1]):
                 t = ops.Table(w.detach()[lo:hi], row_offset=lo)
                 t.version = w._version
                 self._table = t
+            elif t.version != w._version:
+                t.refresh()
+                t.version = w._version
             return t
-        if t is None or t.weight.data_ptr() != w.data_ptr() or t.n_rows != w.shape[0] or t.version != w._version:
+        if t is None or t.weight.data_ptr() != w.data_ptr() or t.weight.shape != w.shape:
             t = ops.Table(w.detach())
             t.version = w._version
             self._table = t
+        elif t.version != w._version:   # updated in place (an optimizer step): refresh the handle on the stream
+            t.refresh()
+            t.version = w._version
         return t
 
     # ---- helpers shared by the subclasses

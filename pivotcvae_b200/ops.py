@@ -93,7 +93,8 @@ def device_ok(device=None):
 # item table handle
 # ----------------------------------------------------------------------------
 class Table:
-    """Borrowed view of the frozen item table (cvae.py:30-32) + cached workspaces."""
+    """Borrowed view of the item table (cvae.py:30-32) + cached workspaces.  The handle derives packed images and
+    max|w| from the weight's values: after an in-place update call refresh(); re-create it when the weight moves."""
 
     def __init__(self, weight, row_offset=0):
         self.weight = _f32(weight, "item table")
@@ -119,6 +120,13 @@ class Table:
     @property
     def handle(self):
         return self._h
+
+    def refresh(self):
+        """Bring the handle up to date with an in-place update of the weight (same storage and shape), on the current
+        stream: no allocation and no host sync, so a CUDA graph may capture it.  The object, its workspaces and their
+        pins stay."""
+        with torch.cuda.device(self.weight.device):
+            L.check(L.load().pcv_table_refresh(self._h, _stream()), "pcv_table_refresh")
 
     def workspace(self, kind, M):
         key = (kind, int(M))
