@@ -379,7 +379,14 @@ int pcv_cand_ce_fwd_bwd(const pcv_table *t, const float *Q, const int64_t *candi
  *   dW[j] = sum_i row_scale[i] * m_ij * (e^{x_ij - lse_i} - [t_i = j]) * q_i
  * with the forward's mask m (masked-out logits are constant zeros: no gradient).  Q, targets, M and mask are those of
  * the pcv_ce_fwd_bwd call, lse [M] is what it returned, row_scale [M] = d loss / d loss_rows[i] (device).  dW [n_rows,
- * dim] is OVERWRITTEN.  Whole table only (row_offset 0), dims 4..128 as the forward.  Paths (the forward's routing):
+ * dim] is OVERWRITTEN.  Dims 4..128 as the forward.
+ * Row shard (vocab-parallel, pcv_table_create with row_offset > 0; row_offset must be a multiple of 128, else
+ * PCV_ERR_ARG): dW holds the shard's n_rows rows only, targets stay global indices (a one-hot term counts only when
+ * its target lies in [row_offset, row_offset + n_rows)), and lse must be the WHOLE catalog's (pcv_ce_fwd_bwd on the
+ * full table, or pcv_ce_vp_merge).  A bitmask is the shard's own columns: row i holds ceil(n_rows / 32) words, bit j
+ * is global column row_offset + j (columns [row_offset / 32, ceil((row_offset + n_rows) / 32)) of the forward's mask).
+ * Every row of a shard equals that row of the whole-table result: bit for bit on the tf32 path, and on the exact pass
+ * when both plans have one row split.  Paths (the forward's routing):
  *  - bitmask, or keep_prob >= 1 with engine EXACT: item-major exact pass — a CTA owns 128 items and streams every
  *    query row, logits re-derived with the forward's fp32 FMA chain, rows summed in a fixed order (+ a fixed-order
  *    reduce of row splits when the catalog is small).  REPRODUCIBLE bit for bit;
@@ -388,7 +395,8 @@ int pcv_cand_ce_fwd_bwd(const pcv_table *t, const float *Q, const int64_t *candi
  *    stays in TMEM for the whole sweep).  Reduced precision like the tf32 forward (tf32 logits, within 2^-9 |q| |w|;
  *    tf32 products in the contraction), REPRODUCIBLE bit for bit; needs no workspace beyond the query;
  *  - Philox (keep_prob < 1, no bitmask): regenerates exactly the forward's gap-process mask from seed, offset and
- *    *offset_dev, O(M * n_neg) work, float atomics: NOT reproducible bit for bit (last-bit differences run to run).
+ *    *offset_dev, O(M * n_neg) work (a shard walks only the 1024-column blocks it overlaps: O(M * n_neg * n_rows / N)),
+ *    float atomics: NOT reproducible bit for bit (last-bit differences run to run).
  * Workspace: pcv_ce_table_grad_workspace_bytes for the same table, M and mask (no zero-fill needed).  No allocation,
  * no host sync. */
 int pcv_ce_table_grad_workspace_bytes(const pcv_table *t, int64_t M, const pcv_ce_mask *mask, size_t *bytes_host);
@@ -397,7 +405,9 @@ int pcv_ce_table_grad(const pcv_table *t, const float *Q, const int64_t *targets
                       float *dW, void *workspace, size_t workspace_bytes, pcv_stream_t stream);
 /* Candidate mode: dW[candidates[i, c]] += row_scale[i] * (softmax_c(p[i, :]) - [c = target_pos[i]]) * q_i for every
  * column c (a duplicate candidate once per occurrence), logits re-derived from lse (of pcv_cand_ce_fwd_bwd).  ADDS
- * into dW: the caller zero-fills it.  Float atomics: not reproducible bit for bit. */
+ * into dW: the caller zero-fills it.  Float atomics: not reproducible bit for bit.  A row shard (row_offset a multiple
+ * of 128, else PCV_ERR_ARG) takes the whole catalog's lse and global candidate ids; it skips candidates outside it and
+ * adds into dW[j - row_offset] ([n_rows, dim]). */
 int pcv_cand_ce_table_grad(const pcv_table *t, const float *Q, const int64_t *candidates, const int64_t *target_pos,
                            int64_t M, int n_cand, const float *lse, const float *row_scale, float *dW, pcv_stream_t stream);
 

@@ -230,9 +230,11 @@ class CatalogCEFn(torch.autograd.Function):
     (train_generative.py:36-42, 59) without materialising logits."""
 
     @staticmethod
-    def forward(ctx, q, table, targets, keep_prob, bitmask, seed, offset, offset_dev=None, engine="exact", weight=None):
+    def forward(ctx, q, table, targets, keep_prob, bitmask, seed, offset, offset_dev=None, engine="exact", weight=None,
+                grad_table=None):
         """weight: the tensor `table` views (docEmbed.weight); when it requires grad, backward returns d loss / d weight
-        (pcv_ce_table_grad over the same mask)."""
+        (pcv_ce_table_grad over the same mask).  grad_table: a row shard of `table` (vocab-parallel); the table
+        gradient is then computed for its rows only and is zero elsewhere."""
         ctx.set_materialize_grads(False)
         loss_rows, lse, dq = ops.ce_fwd_bwd(table, q, targets, keep_prob, bitmask, seed, offset,
                                             want_dq=q.requires_grad, offset_dev=offset_dev, engine=engine)
@@ -246,6 +248,7 @@ class CatalogCEFn(torch.autograd.Function):
             # forward read, so that the backward regenerates the forward's mask
             snap = offset_dev.clone() if offset_dev is not None else None
             ctx.table, ctx.mask_args = table, (keep_prob, bitmask, seed, offset, snap, engine)
+            ctx.grad_table = grad_table
         ctx.save_for_backward(*saved)
         ctx.mark_non_differentiable(lse)
         return loss_rows.mean(), loss_rows, lse
@@ -261,8 +264,26 @@ class CatalogCEFn(torch.autograd.Function):
                 d = dq * g_rows.unsqueeze(1) if d is None else d + dq * g_rows.unsqueeze(1)
         if ctx.want_dw and (g_mean is not None or g_rows is not None):
             q, targets, lse = saved[-3:]
-            dW = ops.ce_table_grad(ctx.table, q, targets, lse, _row_scale(g_mean, g_rows, ctx.M), *ctx.mask_args)
-        return d, None, None, None, None, None, None, None, None, dW
+            rs = _row_scale(g_mean, g_rows, ctx.M)
+            shard = ctx.grad_table
+            if shard is None:
+                dW = ops.ce_table_grad(ctx.table, q, targets, lse, rs, *ctx.mask_args)
+            else:
+                keep, bitmask, seed, offset, snap, engine = ctx.mask_args
+                if bitmask is not None:     # the shard's own columns (its row_offset is a multiple of 32)
+                    bitmask = bitmask[:, shard.row_offset // 32:-(-(shard.row_offset + shard.n_rows) // 32)]
+                dW = _shard_grad(ctx.table.n_rows, shard, lambda out: ops.ce_shard_table_grad(
+                    shard, q, targets, lse, rs, keep, bitmask, seed, offset, snap, engine, out=out))
+        return d, None, None, None, None, None, None, None, None, dW, None
+
+
+def _shard_grad(n_items, shard, fill):
+    """[n_items, D] gradient of a table of which `shard` covers some rows: zero outside them, fill(out) writes the
+    shard's rows into `out`, their view.  Vocab-parallel: each rank computes its own rows, and the row exchange
+    (parallel.exchange_owned_rows) assembles the full gradient on every rank."""
+    dW = torch.zeros(n_items, shard.dim, dtype=torch.float32, device=shard.weight.device)
+    fill(dW[shard.row_offset:shard.row_offset + shard.n_rows])
+    return dW
 
 
 def _row_scale(g_mean, g_rows, M):
@@ -276,10 +297,13 @@ def _row_scale(g_mean, g_rows, M):
 class VocabParallelCEFn(torch.autograd.Function):
     """The same mean CE with the catalog sharded over the ranks of `group` (SURVEY §8e): local partial records over
     this rank's row shard, ONE all-gather of [M, 2 + D] floats, merge.  Every rank gets the full loss and the full
-    d loss / d q, so the replicated MLPs see identical gradients without any further collective."""
+    d loss / d q, so the replicated MLPs see identical gradients without any further collective.
+
+    weight: the tensor `full_weight` is a detached view of (docEmbed.weight); when it requires grad, backward returns
+    its gradient for the shard's rows (pcv_ce_table_grad on the shard with the merged lse), zero elsewhere."""
 
     @staticmethod
-    def forward(ctx, q, shard, full_weight, targets, group, engine="exact"):
+    def forward(ctx, q, shard, full_weight, targets, group, engine="exact", weight=None):
         import torch.distributed as dist
         ctx.set_materialize_grads(False)
         rec = ops.ce_partials(shard, q, targets, engine=engine)
@@ -289,18 +313,31 @@ class VocabParallelCEFn(torch.autograd.Function):
         recs = recs.view(world, rec.shape[0], rec.shape[1])
         loss_rows, lse, dq = ops.ce_vp_merge(recs, full_weight, q, targets, want_dq=q.requires_grad)
         ctx.M = q.shape[0]
-        if dq is not None:
-            ctx.save_for_backward(dq)
+        ctx.want_dq = dq is not None
+        ctx.want_dw = weight is not None and weight.requires_grad
+        saved = [dq] if dq is not None else []
+        if ctx.want_dw:
+            saved += [q.detach(), targets, lse]
+            ctx.shard, ctx.engine, ctx.n_items = shard, engine, full_weight.shape[0]
+        ctx.save_for_backward(*saved)
         ctx.mark_non_differentiable(lse)
         return loss_rows.mean(), loss_rows, lse
 
     @staticmethod
     def backward(ctx, g_mean, g_rows, _g_lse):
-        (dq,) = ctx.saved_tensors
-        d = dq * (g_mean / ctx.M) if g_mean is not None else None
-        if g_rows is not None:
-            d = dq * g_rows.unsqueeze(1) if d is None else d + dq * g_rows.unsqueeze(1)
-        return d, None, None, None, None, None
+        saved = ctx.saved_tensors
+        d = dW = None
+        if ctx.want_dq:
+            dq = saved[0]
+            d = dq * (g_mean / ctx.M) if g_mean is not None else None
+            if g_rows is not None:
+                d = dq * g_rows.unsqueeze(1) if d is None else d + dq * g_rows.unsqueeze(1)
+        if ctx.want_dw and (g_mean is not None or g_rows is not None):
+            q, targets, lse = saved[-3:]
+            rs = _row_scale(g_mean, g_rows, ctx.M)
+            dW = _shard_grad(ctx.n_items, ctx.shard, lambda out: ops.ce_shard_table_grad(
+                ctx.shard, q, targets, lse, rs, 1.0, engine=ctx.engine, out=out))
+        return d, None, None, None, None, None, dW
 
 
 class GatherNormFn(torch.autograd.Function):
@@ -373,9 +410,10 @@ class CandidateCEFn(torch.autograd.Function):
     """mean CE over per-row candidate lists (train_generative.py:52-56)."""
 
     @staticmethod
-    def forward(ctx, q, table, candidates, target_pos, weight=None):
+    def forward(ctx, q, table, candidates, target_pos, weight=None, grad_table=None):
         """weight: the tensor `table` views; when it requires grad, backward returns d loss / d weight
-        (pcv_cand_ce_table_grad)."""
+        (pcv_cand_ce_table_grad).  grad_table: a row shard of `table` (vocab-parallel); the table gradient is then
+        computed for its rows only and is zero elsewhere."""
         loss_rows, lse, dq, _ = ops.cand_ce_fwd_bwd(table, q, candidates, target_pos, want_dq=q.requires_grad)
         ctx.M = q.shape[0]
         ctx.want_dq = dq is not None
@@ -383,7 +421,7 @@ class CandidateCEFn(torch.autograd.Function):
         saved = [dq] if dq is not None else []
         if ctx.want_dw:
             saved += [q.detach(), candidates, target_pos, lse]
-            ctx.table = table
+            ctx.table, ctx.grad_table = table, grad_table
         ctx.save_for_backward(*saved)
         return loss_rows.mean()
 
@@ -394,8 +432,13 @@ class CandidateCEFn(torch.autograd.Function):
         dW = None
         if ctx.want_dw:
             q, cand, tpos, lse = saved[-4:]
-            dW = ops.cand_ce_table_grad(ctx.table, q, cand, tpos, lse, _row_scale(g, None, ctx.M))
-        return d, None, None, None, dW
+            rs, shard = _row_scale(g, None, ctx.M), ctx.grad_table
+            if shard is None:
+                dW = ops.cand_ce_table_grad(ctx.table, q, cand, tpos, lse, rs)
+            else:
+                dW = _shard_grad(ctx.table.n_rows, shard,
+                                 lambda out: ops.cand_ce_table_grad(shard, q, cand, tpos, lse, rs, out=out))
+        return d, None, None, None, dW, None
 
 
 class CandidateLogitsFn(torch.autograd.Function):

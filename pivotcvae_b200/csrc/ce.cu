@@ -613,6 +613,8 @@ static int ce_dispatch(const Table *t, const CEPlan &p, const float *Q, const in
 // streams query rows through shared memory, TG_ROWS at a time; every logit is recomputed with the forward's exact
 // fp32 FMA chain.  Rows are summed in ascending order; when the catalog gives too few CTAs the rows are cut into
 // n_split ranges whose partial rows ce_tg_reduce_kernel adds in split order.  No atomics: reproducible bit for bit.
+// A row shard (row_offset > 0, a multiple of TG_ITEMS) owns the items [row_offset, row_offset + n_rows) of the catalog:
+// targets are global, lse is the whole catalog's, so each item's arithmetic is the whole table's.
 // ---------------------------------------------------------------------------
 constexpr int TG_ITEMS = 128;   // items per CTA = threads
 constexpr int TG_ROWS = 32;     // query rows per shared-memory tile
@@ -647,7 +649,7 @@ static void tg_plan(const Table *t, int64_t M, TGPlan *p) {
 
 template <int D, int MODE>
 __global__ void __launch_bounds__(TG_ITEMS, D <= 16 ? 8 : 1)
-ce_table_grad_kernel(const float *__restrict__ W, int64_t n_rows, const float *__restrict__ Q,
+ce_table_grad_kernel(const float *__restrict__ W, int64_t n_rows, int64_t row_offset, const float *__restrict__ Q,
                      const int64_t *__restrict__ targets, const float *__restrict__ lse,
                      const float *__restrict__ row_scale, int64_t M, int64_t rows_per_split,
                      const uint32_t *__restrict__ bitmask, int64_t mask_words, float *__restrict__ out) {
@@ -689,7 +691,7 @@ ce_table_grad_kernel(const float *__restrict__ W, int64_t n_rows, const float *_
     if (tid < nr) {
       ls[tid] = lse[i0 + tid];
       gs[tid] = row_scale[i0 + tid];
-      ts[tid] = targets[i0 + tid];
+      ts[tid] = targets[i0 + tid] - row_offset;   // local item index; outside the shard it matches no item
     }
     __syncthreads();
 #pragma unroll(Cfg::UNROLL)
@@ -759,8 +761,8 @@ static int launch_table_grad(const Table *t, const TGPlan &p, const float *Q, co
   }
   const int64_t mask_words = (t->n_rows + 31) / 32;
   dim3 grid((unsigned)p.item_ctas, (unsigned)p.n_split);
-  kern<<<grid, TG_ITEMS, Cfg::SMEM, st>>>(t->W, t->n_rows, Q, targets, lse, row_scale, M, p.rows_per_split, bitmask,
-                                           mask_words, p.n_split > 1 ? part : dW);
+  kern<<<grid, TG_ITEMS, Cfg::SMEM, st>>>(t->W, t->n_rows, t->row_offset, Q, targets, lse, row_scale, M, p.rows_per_split, bitmask,
+                                            mask_words, p.n_split > 1 ? part : dW);
   PCV_LAUNCH_CHECK();
   if (p.n_split > 1) {
     const int64_t n4 = t->n_rows * D / 4;
@@ -791,9 +793,11 @@ static int table_grad_dispatch(const Table *t, const TGPlan &p, const float *Q, 
 // block, Philox keyed on (block, row + offset) — regenerates exactly the forward's kept columns, O(n_neg) per row.
 // Each kept column adds g (p - [j = t]) q_i to its dW row with vector float atomics: NOT reproducible bit for bit
 // (the summation order over rows follows the schedule).  The caller's dW is zeroed by the entry point first.
+// A row shard [lo, lo + n_rows) walks only the blocks that overlap it: blocks keep their global ids (the Philox key),
+// so the kept columns inside the shard are exactly the forward's, and the work per row is O(n_neg * n_rows / N).
 template <int D>
 __global__ void __launch_bounds__(256)
-ce_sparse_table_grad_kernel(const float *__restrict__ W, int64_t n_rows, const float *__restrict__ Q,
+ce_sparse_table_grad_kernel(const float *__restrict__ W, int64_t n_rows, int64_t lo, const float *__restrict__ Q,
                             const int64_t *__restrict__ targets, const float *__restrict__ lse,
                             const float *__restrict__ row_scale, int64_t M, const uint32_t *__restrict__ T,
                             uint64_t seed, uint64_t offset, const uint64_t *__restrict__ offset_dev,
@@ -814,23 +818,24 @@ ce_sparse_table_grad_kernel(const float *__restrict__ W, int64_t n_rows, const f
   const int64_t tgt = targets[row];
   const float l_row = lse[row];
   bool seen_tgt = false;
-  auto visit = [&](int64_t j) {
+  auto visit = [&](int64_t j) {   // j global, in the shard
     float s = 0.f;
 #pragma unroll
     for (int c = 0; c < D / 4; ++c) {
-      const float4 v = __ldg(reinterpret_cast<const float4 *>(W + j * D) + c);
+      const float4 v = __ldg(reinterpret_cast<const float4 *>(W + (j - lo) * D) + c);
       s = fmaf(q[4 * c], v.x, s); s = fmaf(q[4 * c + 1], v.y, s);
       s = fmaf(q[4 * c + 2], v.z, s); s = fmaf(q[4 * c + 3], v.w, s);
     }
     const float p = __expf(s - l_row);
     const float coef = g * (j == tgt ? p - 1.f : p);
-    float4 *dst = reinterpret_cast<float4 *>(dW + j * D);
+    float4 *dst = reinterpret_cast<float4 *>(dW + (j - lo) * D);
 #pragma unroll
     for (int c = 0; c < D / 4; ++c)
       atomicAdd(dst + c, make_float4(coef * q[4 * c], coef * q[4 * c + 1], coef * q[4 * c + 2], coef * q[4 * c + 3]));
   };
-  const int64_t n_blocks = (n_rows + CE_GB - 1) / CE_GB;
-  for (int64_t b = lane; b < n_blocks; b += 32) {
+  const int64_t hi = lo + n_rows;
+  const int64_t b_end = (hi + CE_GB - 1) / CE_GB;
+  for (int64_t b = lo / CE_GB + lane; b < b_end; b += 32) {
     int c = -1;
     Philox4 ph = {0, 0, 0, 0};
     for (int k = 0;; ++k) {
@@ -841,14 +846,16 @@ ce_sparse_table_grad_kernel(const float *__restrict__ W, int64_t n_rows, const f
       c += 1 + gap_from_u(T, u);
       if (c >= CE_GB) break;
       const int64_t j = b * CE_GB + c;
-      if (j >= n_rows) break;
+      if (j >= hi) break;
+      if (j < lo) continue;
       if (j == tgt) seen_tgt = true;
       visit(j);
     }
   }
-  // the target column is always part of the mask (train_generative.py:38)
+  // the target column is always part of the mask (train_generative.py:38); a target inside the shard was seen iff the
+  // forward's walk drew it
   const bool any_seen = __any_sync(0xffffffffu, seen_tgt);
-  if (lane == 0 && !any_seen) visit(tgt);
+  if (lane == 0 && !any_seen && tgt >= lo && tgt < hi) visit(tgt);
 }
 
 template <int D>
@@ -860,18 +867,21 @@ static int launch_sparse_table_grad(const Table *t, const float *Q, const int64_
   PCV_CUDA(cudaMemsetAsync(dW, 0, (size_t)t->n_rows * D * sizeof(float), st));
   ce_gap_table_kernel<<<1, 1, 0, st>>>(q32, T);
   PCV_LAUNCH_CHECK();
-  ce_sparse_table_grad_kernel<D><<<(unsigned)((M + 7) / 8), 256, 0, st>>>(t->W, t->n_rows, Q, targets, lse, row_scale, M, T,
-                                                                         mask->seed, mask->offset, mask->offset_dev, dW);
+  ce_sparse_table_grad_kernel<D><<<(unsigned)((M + 7) / 8), 256, 0, st>>>(t->W, t->n_rows, t->row_offset, Q, targets, lse,
+                                                                         row_scale, M, T, mask->seed, mask->offset,
+                                                                         mask->offset_dev, dW);
   PCV_LAUNCH_CHECK();
   return PCV_OK;
 }
 
 // Candidate mode: one warp per row, lane = candidate column (as cand_ce_kernel); the logit is recomputed from lse, so
 // no [M, n_cand] buffer is kept.  Column c adds g (p_c - [c = target_pos]) q_i to dW[cand[i, c]] (duplicates once per
-// occurrence) with vector float atomics.
+// occurrence) with vector float atomics.  A row shard [lo, lo + n_rows) skips the candidates outside it and writes row
+// j - lo.
 template <int D>
 __global__ void __launch_bounds__(256)
-cand_ce_table_grad_kernel(const float *__restrict__ W, const float *__restrict__ Q, const int64_t *__restrict__ cand,
+cand_ce_table_grad_kernel(const float *__restrict__ W, int64_t n_rows, int64_t lo, const float *__restrict__ Q,
+                          const int64_t *__restrict__ cand,
                           const int64_t *__restrict__ tgt_pos, int64_t M, int nC, const float *__restrict__ lse,
                           const float *__restrict__ row_scale, float *__restrict__ dW) {
   const int lane = threadIdx.x & 31;
@@ -889,7 +899,8 @@ cand_ce_table_grad_kernel(const float *__restrict__ W, const float *__restrict__
   const int64_t tp = tgt_pos[row];
   const int64_t *cr = cand + row * nC;
   for (int c = lane; c < nC; c += 32) {
-    const int64_t j = __ldg(cr + c);
+    const int64_t j = __ldg(cr + c) - lo;
+    if (j < 0 || j >= n_rows) continue;
     float w[D];
 #pragma unroll
     for (int v4 = 0; v4 < D / 4; ++v4) {
@@ -1063,7 +1074,7 @@ int pcv_ce_table_grad(const pcv_table *th, const float *Q, const int64_t *target
   PCV_CHECK_ARG(th && Q && targets && mask && lse && row_scale && dW, "NULL pointer");
   PCV_CHECK_ARG(M > 0, "M must be > 0");
   const Table *t = reinterpret_cast<const Table *>(th);
-  PCV_CHECK_ARG(t->row_offset == 0, "the table gradient needs the whole table (row_offset 0)");
+  PCV_CHECK_ARG(t->row_offset % 128 == 0, "a table shard's row_offset must be a multiple of 128");
   PCV_CHECK_ARG(t->n_rows < 0x7fffffffLL, "table larger than 2^31-1 rows");
   PCV_CHECK_ARG(mask->keep_prob > 0.0, "keep_prob must be > 0");
   if (!ce_rows_for(t->dim)) {
@@ -1110,18 +1121,18 @@ int pcv_cand_ce_table_grad(const pcv_table *th, const float *Q, const int64_t *c
   PCV_CHECK_ARG(th && Q && candidates && target_pos && lse && row_scale && dW, "NULL pointer");
   PCV_CHECK_ARG(M > 0 && n_cand > 0, "bad shape");
   const Table *t = reinterpret_cast<const Table *>(th);
-  PCV_CHECK_ARG(t->row_offset == 0, "candidate CE needs the whole table (row_offset 0)");
+  PCV_CHECK_ARG(t->row_offset % 128 == 0, "a table shard's row_offset must be a multiple of 128");
   int rc = check_arch();
   if (rc != PCV_OK) return rc;
   cudaStream_t st = (cudaStream_t)stream;
   const unsigned blocks = (unsigned)((M + 7) / 8);
   switch (t->dim) {
-    case 4: cand_ce_table_grad_kernel<4><<<blocks, 256, 0, st>>>(t->W, Q, candidates, target_pos, M, n_cand, lse, row_scale, dW); break;
-    case 8: cand_ce_table_grad_kernel<8><<<blocks, 256, 0, st>>>(t->W, Q, candidates, target_pos, M, n_cand, lse, row_scale, dW); break;
-    case 16: cand_ce_table_grad_kernel<16><<<blocks, 256, 0, st>>>(t->W, Q, candidates, target_pos, M, n_cand, lse, row_scale, dW); break;
-    case 32: cand_ce_table_grad_kernel<32><<<blocks, 256, 0, st>>>(t->W, Q, candidates, target_pos, M, n_cand, lse, row_scale, dW); break;
-    case 64: cand_ce_table_grad_kernel<64><<<blocks, 256, 0, st>>>(t->W, Q, candidates, target_pos, M, n_cand, lse, row_scale, dW); break;
-    case 128: cand_ce_table_grad_kernel<128><<<blocks, 256, 0, st>>>(t->W, Q, candidates, target_pos, M, n_cand, lse, row_scale, dW); break;
+    case 4: cand_ce_table_grad_kernel<4><<<blocks, 256, 0, st>>>(t->W, t->n_rows, t->row_offset, Q, candidates, target_pos, M, n_cand, lse, row_scale, dW); break;
+    case 8: cand_ce_table_grad_kernel<8><<<blocks, 256, 0, st>>>(t->W, t->n_rows, t->row_offset, Q, candidates, target_pos, M, n_cand, lse, row_scale, dW); break;
+    case 16: cand_ce_table_grad_kernel<16><<<blocks, 256, 0, st>>>(t->W, t->n_rows, t->row_offset, Q, candidates, target_pos, M, n_cand, lse, row_scale, dW); break;
+    case 32: cand_ce_table_grad_kernel<32><<<blocks, 256, 0, st>>>(t->W, t->n_rows, t->row_offset, Q, candidates, target_pos, M, n_cand, lse, row_scale, dW); break;
+    case 64: cand_ce_table_grad_kernel<64><<<blocks, 256, 0, st>>>(t->W, t->n_rows, t->row_offset, Q, candidates, target_pos, M, n_cand, lse, row_scale, dW); break;
+    case 128: cand_ce_table_grad_kernel<128><<<blocks, 256, 0, st>>>(t->W, t->n_rows, t->row_offset, Q, candidates, target_pos, M, n_cand, lse, row_scale, dW); break;
     default:
       set_error("cand_ce_table_grad: dim %d unsupported", t->dim);
       return PCV_ERR_UNSUPPORTED;

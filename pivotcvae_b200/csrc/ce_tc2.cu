@@ -567,6 +567,8 @@ ce_tc2_kernel(const float *__restrict__ Wsw, const float *__restrict__ Wt, int64
 //   128   64     64 + 32 + 32 KB                   64 + 128 (256)
 // Error: the tf32 logit is within 2^-9 |q_i| |w_j| of the exact one (both operands truncated to 10 mantissa bits), and
 // the gradient MMA truncates P^T and Q again (2^-9 relative per term).
+// A row shard (row_offset a multiple of 128) has the whole table's slabs from row_offset / 128 on: targets are global
+// and lse is the whole catalog's, so every item's result is the whole table's, bit for bit.
 template <int D>
 struct TgCfg {
   static constexpr int KA = D / 8;
@@ -591,7 +593,7 @@ struct __align__(1024) TgSmem {
 
 template <int D>
 __global__ void __launch_bounds__(TC_BM)
-ce_tc_table_grad_kernel(const float *__restrict__ W, int64_t n_rows, const float *__restrict__ Q,
+ce_tc_table_grad_kernel(const float *__restrict__ W, int64_t n_rows, int64_t row_offset, const float *__restrict__ Q,
                         const int64_t *__restrict__ targets, const float *__restrict__ lse,
                         const float *__restrict__ row_scale, int64_t M, float *__restrict__ dW) {
   using C = TgCfg<D>;
@@ -668,7 +670,7 @@ ce_tc_table_grad_kernel(const float *__restrict__ W, int64_t n_rows, const float
       const bool ok = i < M;
       S.lse[r] = ok ? lse[i] : 0.f;
       S.rs[r] = ok ? row_scale[i] : 0.f;
-      S.tg[r] = ok ? targets[i] : -1;
+      S.tg[r] = ok ? targets[i] - row_offset : -1;   // local item index; outside the shard it matches no item
     }
     asm volatile("fence.proxy.async.shared::cta;" ::: "memory");
     asm volatile("tcgen05.fence::before_thread_sync;" ::: "memory");
@@ -886,7 +888,7 @@ static int ce_tc_table_grad_d(const Table *t, const float *Q, const int64_t *tar
     attr_set[t->device & 63] = true;
   }
   const unsigned grid = (unsigned)((t->n_rows + TC_BM - 1) / TC_BM);
-  ce_tc_table_grad_kernel<D><<<grid, TC_BM, smem, st>>>(t->W, t->n_rows, Q, targets, lse, row_scale, M, dW);
+  ce_tc_table_grad_kernel<D><<<grid, TC_BM, smem, st>>>(t->W, t->n_rows, t->row_offset, Q, targets, lse, row_scale, M, dW);
   PCV_LAUNCH_CHECK();
   return PCV_OK;
 }

@@ -76,7 +76,9 @@ class GraphedTrainStep:
     train_tables=True captures a fine_tune step too (trainable docEmbed / userEmbed): the step ends by refreshing the
     item-table handle in place (pcv_table_refresh) after the optimizer has updated docEmbed, so the next replay's
     cross-entropy reads packed images and a max|w| that match the table.  userEmbed has no handle: only the fused MLP
-    gathers read it."""
+    gathers read it.  On a vocab-parallel model (enable_vocab_parallel(train_tables=True)) that handle is this rank's
+    shard, and the full-catalog handle is refreshed too when the step reads it (masked mode); the row exchange of the
+    table gradients runs inside the graph."""
 
     def __init__(self, model, optimizer, batch, beta, n_neg, warmup=3, train_tables=False):
         from . import _lib
@@ -93,17 +95,20 @@ class GraphedTrainStep:
                        "users": torch.zeros(batch, 1, dtype=torch.int64, device=dev),
                        "responses": torch.zeros(batch, L, device=dev)}
 
-        # the one handle every replay reads (and refreshes); kept alive with the graph that baked its pointers in
+        # the handles every replay reads (and refreshes); kept alive with the graph that baked their pointers in
         self._table = model.item_table() if trainable else None
+        # vocab-parallel: a masked step (n_neg < N) also reads the full-catalog handle (the static batch carries no
+        # candidate lists, so candidate mode is never captured)
+        vp = getattr(model, "_vp", None) is not None
+        self._full = model.full_table() if (trainable and vp and n_neg < model.docEmbed.weight.shape[0]) else None
 
         def step():
             optimizer.zero_grad(set_to_none=True)
             loss, rec, kld = get_gen_loss(self.static, model, None, beta, n_neg=n_neg)
             loss.backward()
             optimizer.step()
-            if self._table is not None:     # docEmbed moved in place: bring the handle along, once per step
-                self._table.refresh()
-                self._mark_current()
+            if self._table is not None:     # docEmbed moved in place: bring the handles along, once per step
+                self._refresh()
             model.noise.end_graph_step()
             return loss.detach(), rec.detach(), kld.detach()
 
@@ -128,8 +133,7 @@ class GraphedTrainStep:
                         if torch.is_tensor(v):
                             v.copy_(ss[k]) if k in ss else v.zero_()   # state created by the warm-up starts at zero
             if self._table is not None:     # the restore changed docEmbed in place: the first replay reads the handle
-                self._table.refresh()
-                self._mark_current()
+                self._refresh()
         torch.cuda.current_stream(dev).wait_stream(side)
         torch.cuda.synchronize(dev)
         self.graph = torch.cuda.CUDAGraph()
@@ -138,14 +142,25 @@ class GraphedTrainStep:
             self.loss, self.rec, self.kld = step()
         self.launches_per_step = ops.launch_count() - l0
         model.item_table().pin_workspaces()
+        if self._full is not None:
+            self._full.pin_workspaces()
         ops.pin_packed()
 
+    def _refresh(self):
+        for t in (self._table, self._full):
+            if t is not None:
+                t.refresh()
+        self._mark_current()
+
     def _mark_current(self):
-        """The handle matches docEmbed as it is now: item_table() must not refresh it again."""
-        self._table.version = self.model.docEmbed.weight._version
+        """The handles match docEmbed as it is now: item_table() / full_table() must not refresh them again."""
+        for t in (self._table, self._full):
+            if t is not None:
+                t.version = self.model.docEmbed.weight._version
 
     def __call__(self, batch):
-        if self._table is not None and self._table is not self.model.item_table():
+        if ((self._table is not None and self._table is not self.model.item_table())
+                or (self._full is not None and self._full is not self.model.full_table())):
             raise RuntimeError("GraphedTrainStep: docEmbed was re-allocated or reshaped since the capture; build a new step")
         for k, v in self.static.items():
             v.copy_(batch[k].reshape(v.shape), non_blocking=True)

@@ -69,6 +69,8 @@ class BaseCVAE(nn.Module):
         self._table = None
         self._full = None    # full-catalog handle while vocab-parallel (the sampler draws over every row)
         self._vp = None      # vocab-parallel state: (group, lo, hi) once enable_vocab_parallel() is called
+        self._vp_train = False   # enable_vocab_parallel(train_tables=True): the tables train on the sharded catalog
+        self._vp_hooks = []      # their row-exchange hooks (removable handles)
 
     # ---- extension state is rebuilt lazily (whole-model pickling, train_generative.py:199)
     def __getstate__(self):
@@ -76,26 +78,42 @@ class BaseCVAE(nn.Module):
         st["_table"] = None
         st["_full"] = None
         st["_vp"] = None
+        st["_vp_train"] = False
+        st["_vp_hooks"] = []
         st.pop("_rows", None)
         st.pop("_head_cache", None)
         return st
 
     # ---- vocab-parallel scoring (SURVEY §8e): every rank keeps the full fp32 table (<= 320 MB) for the
     # gathers, but scores only its own 128-aligned row shard; one all-gather of (val, idx) per scoring step
-    def enable_vocab_parallel(self, group=None, shard_rows=True):
+    def enable_vocab_parallel(self, group=None, shard_rows=True, train_tables=False):
         """Score against this rank's row shard of the catalog only.  shard_rows (default): in recommend() the MLP
         blocks run on this rank's 1/world slice of the batch instead of redundantly on all of it, and the
-        queries are all-gathered before every sharded scoring step (a few hundred KB over NVLink)."""
+        queries are all-gathered before every sharded scoring step (a few hundred KB over NVLink).
+
+        train_tables: required when the tables are trainable (fine_tune=True).  The catalog cross-entropy's table
+        gradient is then computed for this rank's rows only, and after every backward a hook on each trainable table
+        all-gathers each rank's own rows of its .grad (parallel.exchange_owned_rows: N * D * 4 bytes per table), so
+        that every rank holds the same full gradient and the replicated tables take identical optimizer steps."""
         import torch.distributed as dist
-        from ..parallel import shard_bounds
-        if self.trainable_tables():
-            raise L.PcvError("enable_vocab_parallel: the embedding tables are trainable (fine_tune=True); the sharded "
-                             "catalog cross-entropy has no table gradient")
+        from ..parallel import exchange_owned_rows, shard_bounds
+        tabs = self.trainable_tables()
+        if tabs and not train_tables:
+            raise L.PcvError("enable_vocab_parallel: the embedding tables are trainable (fine_tune=True); pass "
+                             "train_tables=True to train them on the sharded catalog")
         world, rank = dist.get_world_size(group), dist.get_rank(group)
         lo, hi = shard_bounds(self.docEmbed.weight.shape[0], world, rank)
         self._vp = (group, lo, hi)
         self._vp_rows = bool(shard_rows)
+        self._vp_train = bool(train_tables)
         self._table = None
+        for h in getattr(self, "_vp_hooks", ()):     # a second call replaces the hooks of the first
+            h.remove()
+        self._vp_hooks = []
+        if train_tables:
+            for w in tabs:
+                self._vp_hooks.append(w.register_post_accumulate_grad_hook(
+                    lambda p: exchange_owned_rows(p.grad, group)))
 
     def trainable_tables(self):
         """The embedding tables that require grad (fine_tune=True)."""

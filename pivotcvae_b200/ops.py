@@ -644,15 +644,39 @@ def ce_fwd_bwd(table, Q, targets, keep_prob=1.0, bitmask=None, seed=0, offset=0,
     return loss, lse, dq
 
 
+def _grad_out(out, table, Q):
+    if out is None:
+        return torch.empty(table.n_rows, table.dim, dtype=torch.float32, device=Q.device)
+    if (out.dtype != torch.float32 or tuple(out.shape) != (table.n_rows, table.dim) or not out.is_contiguous()
+            or out.device != Q.device):
+        raise L.PcvError("out must be a contiguous float32 [n_rows, dim] tensor on the queries' device")
+    return out
+
+
 def ce_table_grad(table, Q, targets, lse, row_scale, keep_prob=1.0, bitmask=None, seed=0, offset=0, offset_dev=None,
                   engine="exact"):
     """dW [n_rows, D] = d (sum_i row_scale[i] loss_rows[i]) / d table for the mask of the matching ce_fwd_bwd call;
-    see include/pcv_b200.h pcv_ce_table_grad."""
+    see include/pcv_b200.h pcv_ce_table_grad.  The whole table only: a row shard goes through ce_shard_table_grad."""
+    if table.row_offset != 0:
+        raise L.PcvError("ce_table_grad: the table is a row shard (row_offset %d); use ce_shard_table_grad, which takes "
+                         "the whole catalog's lse and writes the shard's rows" % table.row_offset)
+    return _ce_table_grad(table, Q, targets, lse, row_scale, keep_prob, bitmask, seed, offset, offset_dev, engine, None)
+
+
+def ce_shard_table_grad(shard, Q, targets, lse, row_scale, keep_prob=1.0, bitmask=None, seed=0, offset=0,
+                        offset_dev=None, engine="exact", out=None):
+    """The table gradient of ce_table_grad for one row shard (vocab-parallel): targets stay global, lse is the WHOLE
+    catalog's (ce_fwd_bwd on the full table, or ce_vp_merge), a bitmask is the shard's own columns
+    ([M, ceil(n_rows / 32)]).  -> the shard's rows [n_rows, D]; out: a contiguous [n_rows, D] tensor to write into."""
+    return _ce_table_grad(shard, Q, targets, lse, row_scale, keep_prob, bitmask, seed, offset, offset_dev, engine, out)
+
+
+def _ce_table_grad(table, Q, targets, lse, row_scale, keep_prob, bitmask, seed, offset, offset_dev, engine, out):
     Q, targets = _f32(Q, "Q"), _i64(targets, "targets").reshape(-1)
     lse, row_scale = _f32(lse, "lse"), _f32(row_scale, "row_scale")
     M = Q.shape[0]
     mask, bitmask = _ce_mask(table, M, keep_prob, bitmask, seed, offset, offset_dev, engine)
-    dW = torch.empty(table.n_rows, table.dim, dtype=torch.float32, device=Q.device)
+    dW = _grad_out(out, table, Q)
     ws = table.workspace("ce_tgrad", M)
     with torch.cuda.device(Q.device), _timed("ce_table_grad"):
         L.check(L.load().pcv_ce_table_grad(table.handle, _ptr(Q), _ptr(targets), M, ctypes.byref(mask), _ptr(lse),
@@ -660,15 +684,17 @@ def ce_table_grad(table, Q, targets, lse, row_scale, keep_prob=1.0, bitmask=None
     return dW
 
 
-def cand_ce_table_grad(table, Q, candidates, target_pos, lse, row_scale):
+def cand_ce_table_grad(table, Q, candidates, target_pos, lse, row_scale, out=None):
     """dW [n_rows, D] (zero-filled here) += the candidate-mode CE gradient w.r.t. the table rows each row's candidate
-    list names; see include/pcv_b200.h pcv_cand_ce_table_grad."""
+    list names; see include/pcv_b200.h pcv_cand_ce_table_grad.  A row shard (vocab-parallel) takes global candidate ids
+    and the whole catalog's lse and adds into its own rows.  out: a zero-filled contiguous [n_rows, D] tensor to add
+    into instead."""
     Q = _f32(Q, "Q")
     M = Q.shape[0]
     candidates = _i64(candidates, "candidates").reshape(M, -1)
     target_pos = _i64(target_pos, "target_pos").reshape(-1)
     lse, row_scale = _f32(lse, "lse"), _f32(row_scale, "row_scale")
-    dW = torch.zeros(table.n_rows, table.dim, dtype=torch.float32, device=Q.device)
+    dW = torch.zeros(table.n_rows, table.dim, dtype=torch.float32, device=Q.device) if out is None else _grad_out(out, table, Q)
     with torch.cuda.device(Q.device), _timed("cand_ce_table_grad"):
         L.check(L.load().pcv_cand_ce_table_grad(table.handle, _ptr(Q), _ptr(candidates), _ptr(target_pos), M,
                                                 candidates.shape[1], _ptr(lse), _ptr(row_scale), _ptr(dW), _stream()),

@@ -23,10 +23,15 @@ import torch.distributed as dist
 SHARD_ALIGN = 128  # the tensor-core select's TMA tiles stay aligned across shards
 
 
+def shard_stride(n_rows, world, align=SHARD_ALIGN):
+    """Rows per shard of shard_bounds (the last shard may be shorter, or empty)."""
+    per = -(-n_rows // world)
+    return -(-per // align) * align
+
+
 def shard_bounds(n_rows, world, rank, align=SHARD_ALIGN):
     """Contiguous [lo, hi) row range of `rank`; every boundary but the last is a multiple of align."""
-    per = -(-n_rows // world)
-    per = -(-per // align) * align
+    per = shard_stride(n_rows, world, align)
     lo = min(rank * per, n_rows)
     hi = min(lo + per, n_rows)
     return lo, hi
@@ -52,6 +57,26 @@ def all_gather_rows(t, group=None):
     out = torch.empty((world * t.shape[0],) + tuple(t.shape[1:]), dtype=t.dtype, device=t.device)
     dist.all_gather_into_tensor(out, t, group=group)
     return out
+
+
+def exchange_owned_rows(t, group=None):
+    """In place on `t` ([N, C], the same shape on every rank): rows shard_bounds(N, world, rank) of each rank replace
+    every other rank's copy of them, so that `t` ends byte-identical on every rank.  ONE all-gather through a padded
+    [world * stride, C] buffer (the last shard may be short or empty); capturable in a CUDA graph with NCCL, and it
+    runs over gloo too.
+
+    Vocab-parallel table training: a rank's table gradient is exact on the rows it owns only (the catalog
+    cross-entropy's term is computed there alone), and the MLP gathers' scatter-add runs with atomics, so the
+    replicas' Adam steps stay identical only after this exchange."""
+    world, rank = dist.get_world_size(group), dist.get_rank(group)
+    n = t.shape[0]
+    per = shard_stride(n, world)
+    lo, hi = shard_bounds(n, world, rank)
+    send = t.new_zeros((per,) + tuple(t.shape[1:]))
+    send[:hi - lo] = t[lo:hi]
+    out = t.new_empty((world * per,) + tuple(t.shape[1:]))
+    dist.all_gather_into_tensor(out, send, group=group)
+    t.copy_(out[:n])
 
 
 def merge_ce_partials(recs, W_full, Q, targets):

@@ -39,6 +39,14 @@ def get_gen_loss(batch_data, model, lossFun, beta, n_neg=1000):
     slates = _as_tensor(batch_data["slates"], torch.int64, dev)
     users = _as_tensor(batch_data["users"], torch.int64, dev)
     targets = _as_tensor(batch_data["responses"], torch.float32, dev)
+    vp = getattr(model, "_vp", None)
+    train_vp = vp is not None and model.docEmbed.weight.requires_grad
+    if train_vp and not getattr(model, "_vp_train", False):
+        raise PcvError("get_gen_loss: vocab-parallel training with trainable tables (fine_tune=True) needs "
+                       "enable_vocab_parallel(train_tables=True)")
+    # vocab-parallel: the masked and candidate forwards touch O(n_neg) columns per row and run on the whole catalog;
+    # with train_tables their table gradient is computed for this rank's shard only (grad_table)
+    grad_table = model.item_table() if train_vp else None
     pMu, pLogvar = model.get_prior(targets, users)
     rx, z, mu, logvar, _ = model.forward_latent(slates, targets, users)
     if model.candidateFlag:
@@ -47,16 +55,12 @@ def get_gen_loss(batch_data, model, lossFun, beta, n_neg=1000):
         M = slates.numel()
         cand = _as_tensor(batch_data["sample_candidates"], torch.int64, dev).reshape(M, -1)
         tpos = _as_tensor(batch_data["sample_targets"], torch.int64, dev).reshape(-1)
-        recLoss = CandidateCEFn.apply(rx.reshape(M, -1), model.item_table(), cand, tpos, model.docEmbed.weight)
+        recLoss = CandidateCEFn.apply(rx.reshape(M, -1), model.full_table(), cand, tpos, model.docEmbed.weight,
+                                      grad_table)
         KLD = KLFn.apply(mu, logvar, pMu, pLogvar)
         model.noise.flush_eager()
         return recLoss + beta * KLD, recLoss, KLD
-    vp = getattr(model, "_vp", None)
-    if vp is not None and model.docEmbed.weight.requires_grad:
-        raise PcvError("get_gen_loss: vocab-parallel training needs frozen tables (fine_tune=False): the sharded "
-                       "catalog cross-entropy has no table gradient")
-    table = model.full_table() if vp is not None else model.item_table()
-    N = table.n_rows
+    N = model.docEmbed.weight.shape[0]
     if n_neg > N:
         raise RuntimeError("n_neg (%d) > number of items (%d): torch.bernoulli would reject p > 1" % (n_neg, N))
     keep = float(n_neg) / float(N)
@@ -70,11 +74,12 @@ def get_gen_loss(batch_data, model, lossFun, beta, n_neg=1000):
         # (SURVEY §8e).  Masked training (keep < 1) touches O(n_neg) columns per row and stays unsharded below.
         from .autograd import VocabParallelCEFn
         recLoss, _, _ = VocabParallelCEFn.apply(rx.reshape(M, -1), model.item_table(), model.docEmbed.weight.detach(),
-                                                slates.reshape(-1), vp[0], getattr(model, "ce_engine", "exact"))
+                                                slates.reshape(-1), vp[0], getattr(model, "ce_engine", "exact"),
+                                                model.docEmbed.weight)
     else:
-        recLoss, _, _ = CatalogCEFn.apply(rx.reshape(M, -1), table, slates.reshape(-1), keep, bitmask, kw["seed"],
+        recLoss, _, _ = CatalogCEFn.apply(rx.reshape(M, -1), model.full_table(), slates.reshape(-1), keep, bitmask, kw["seed"],
                                           kw["offset"], kw.get("offset_dev"), getattr(model, "ce_engine", "exact"),
-                                          model.docEmbed.weight)
+                                          model.docEmbed.weight, grad_table)
     KLD = KLFn.apply(mu, logvar, pMu, pLogvar)
     loss = recLoss + beta * KLD
     model.noise.flush_eager()
