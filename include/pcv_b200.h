@@ -113,7 +113,12 @@ typedef struct {
  * calls with the same table and M, one call at a time. */
 int pcv_score_select_workspace_bytes(const pcv_table *t, int64_t M, size_t *bytes_host);
 /* Q: [M, dim].  out_idx: [M] int64 (global index).  out_val: [M] fp32 (the
- * winning score; for exprace the winning key) or NULL. */
+ * winning score; for exprace the winning key) or NULL.
+ * Non-finite scores (DESIGN.md section 2), every engine alike: +-inf order as numbers and equal ones tie by index,
+ * as in torch.max; a NaN score never wins (it counts as -inf; torch.max would return it), and a row with no score
+ * above -inf returns its first index (row_offset) with value -inf.  An index is therefore always inside the table.
+ * The exponential race keys NaN scores like the oracle's exp does (the clamp maps exp(NaN) to exp(-86)).
+ * Workspace: any engine may follow any other on one workspace. */
 int pcv_score_select(const pcv_table *t, const float *Q, int64_t M,
                      const pcv_select_opts *opts, int64_t *out_idx, float *out_val,
                      void *workspace, size_t workspace_bytes, pcv_stream_t stream);
@@ -134,7 +139,9 @@ int pcv_sigmoid_categorical(const pcv_table *t, const float *Q, int64_t M, uint6
 /* Exact top-k over the catalog (torch.topk of the score row; models/deterministic.py:119 in the reference, and the
  * building block of the no-repeat selection): out_idx/out_val [M, k], k <= 16, sorted by score descending, equal
  * scores by ascending index; same fp32 sequential-k FMA chain as pcv_score_select; entries beyond the catalog size
- * are -1 / -inf.  Indices are global (+ row_offset). */
+ * are -1 / -inf.  Indices are global (+ row_offset).  Only scores above -inf are listed (a NaN counts as -inf): the
+ * rest of the window is -1 / -inf as past the end of a short catalog.  pcv_slate_no_repeat: a slot with no untaken
+ * item above -inf keeps its top-1 pick (it may repeat, and it takes nothing from the later slots). */
 int pcv_score_topk_workspace_bytes(const pcv_table *t, int64_t M, size_t *bytes_host);
 int pcv_score_topk(const pcv_table *t, const float *Q, int64_t M, int k, int64_t *out_idx, float *out_val,
                    void *workspace, size_t workspace_bytes, pcv_stream_t stream);

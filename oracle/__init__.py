@@ -136,7 +136,8 @@ def reparam(mu, logvar, eps):
 
 
 def score_select(W, Q, mode="greedy", noise=None):
-    """argmax_j <q_i, w_j> (greedy) or the sigmoid exponential race. -> (idx int64[M], val f32[M])."""
+    """argmax_j <q_i, w_j> (greedy) or the sigmoid exponential race. -> (idx int64[M], val f32[M]).  Greedy: a NaN
+    score never wins (it counts as -inf); a row with no score above -inf returns index 0 and value -inf."""
     W, Q = _f32(W), _f32(Q)
     N, D = W.shape
     M = Q.shape[0]
@@ -171,27 +172,39 @@ def score_logits(W, Q):
 
 def score_topk(W, Q, k):
     """torch.topk of every score row, restated: score descending, equal scores by ascending index (the order a
-    first-index arg-max repeated k times gives).  -> (idx int64[M, k], val f32[M, k])."""
+    first-index arg-max repeated k times gives).  Non-finite rule (include/pcv_b200.h): a NaN score counts as -inf, and
+    only scores above -inf are listed; the slots after them hold index -1 and value -inf, as past the end of a short
+    catalog.  -> (idx int64[M, k], val f32[M, k])."""
     p = score_logits(W, Q)
-    order = np.lexsort((np.broadcast_to(np.arange(p.shape[1]), p.shape), -p.astype(np.float64)), axis=1)[:, :k]
-    return order.astype(np.int64), np.take_along_axis(p, order, 1)
+    key = np.where(np.isnan(p), -np.inf, p).astype(np.float64)
+    order = np.lexsort((np.broadcast_to(np.arange(p.shape[1]), p.shape), -key), axis=1)[:, :k]
+    val = np.take_along_axis(key, order, 1).astype(np.float32)
+    idx = np.where(val > -np.inf, order, -1).astype(np.int64)
+    return idx, val
 
 
 def slate_no_repeat(W, Q, L):
     """Opt-in no-repeat selection (NOT reference behaviour, SURVEY F1): rows of Q are the L slots of M/L slates;
-    slot l takes arg-max_j <q, w_j> (ties -> lowest j) over the items slots 0..l-1 of its slate have not taken."""
+    slot l takes arg-max_j <q, w_j> (ties -> lowest j) over the items slots 0..l-1 of its slate have taken, among the
+    scores above -inf (a NaN score counts as -inf).  A slot with no such item keeps its plain arg-max
+    (score_select's result), which may repeat an earlier slot's item; it does not count as taken."""
     p = score_logits(W, Q)
+    p = np.where(np.isnan(p), np.float32(-np.inf), p)
     M = p.shape[0]
     items = np.empty(M, dtype=np.int64)
     vals = np.empty(M, dtype=np.float32)
     for b in range(M // L):
         taken = []
         for l in range(L):
-            row = p[b * L + l].copy()
-            row[taken] = -np.inf
-            j = int(np.argmax(row))            # numpy arg-max returns the first maximal index
+            row = p[b * L + l]
+            free = row.copy()
+            free[taken] = -np.inf
+            if free.max() > -np.inf:
+                j = int(np.argmax(free))          # numpy arg-max returns the first maximal index
+                taken.append(j)
+            else:
+                j = int(np.argmax(row))           # all -inf: index 0, as score_select
             items[b * L + l], vals[b * L + l] = j, row[j]
-            taken.append(j)
     return items, vals
 
 

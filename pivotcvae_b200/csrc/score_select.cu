@@ -58,6 +58,10 @@ static int tile_for(int D) {
   return t < 128 ? 128 : t;
 }
 
+// The partial winners sit behind the head of the workspace that the tcgen05 engine needs zero on entry (its overflow
+// counter and per-row overflow winners: score_select_tc.cu), so that the engines can share one workspace in any order.
+static size_t ss_ws_head(int64_t M) { return 256 + (((size_t)M * 8 + 255) & ~(size_t)255); }
+
 static int make_plan(const Table *t, int64_t M, SSPlan *p) {
   p->rows_per_cta = rows_per_cta_for(t->dim);
   if (p->rows_per_cta == 0) return PCV_ERR_UNSUPPORTED;
@@ -73,7 +77,7 @@ static int make_plan(const Table *t, int64_t M, SSPlan *p) {
   ns = (n_tiles + tiles_per_split - 1) / tiles_per_split;
   p->n_split = (int)ns;
   p->items_per_split = tiles_per_split * p->tile;
-  p->ws_bytes = (size_t)ns * (size_t)M * (sizeof(float) + sizeof(int32_t));
+  p->ws_bytes = ss_ws_head(M) + (size_t)ns * (size_t)M * (sizeof(float) + sizeof(int32_t));
   return PCV_OK;
 }
 
@@ -216,6 +220,7 @@ __global__ void select_finalize_kernel(const float *__restrict__ part_val,
     int32_t oi = part_idx[(int64_t)s * M + i];
     if (ov > v || (ov == v && oi < ix)) { v = ov; ix = oi; }
   }
+  if (ix == 0x7fffffff) ix = 0;   // no score above -inf (NaN never wins): the first index, value -inf (pcv_b200.h)
   out_idx[i] = (int64_t)ix + row_offset;
   if (out_val) out_val[i] = v;
 }
@@ -362,7 +367,7 @@ int pcv_score_select(const pcv_table *th, const float *Q, int64_t M,
     set_error("score_select: workspace too small (%zu < %zu)", workspace_bytes, p.ws_bytes);
     return PCV_ERR_WORKSPACE;
   }
-  float *pv = reinterpret_cast<float *>(workspace);
+  float *pv = reinterpret_cast<float *>(static_cast<char *>(workspace) + ss_ws_head(M));
   int32_t *pi = reinterpret_cast<int32_t *>(pv + (size_t)p.n_split * M);
 
   rc = opts->mode == PCV_SELECT_GREEDY ? dispatch_dim<SS_GREEDY>(t, p, Q, M, nullptr, pv, pi, nullptr, st)

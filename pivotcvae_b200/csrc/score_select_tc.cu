@@ -113,6 +113,24 @@ __device__ __forceinline__ float tc_norm2(const float *__restrict__ q) {
   return ss;
 }
 
+// |q| for the tf32 filter's band, from ss = tc_norm2.  Where |q|^2 under- or overflows (|q| outside ~[1e-15, 1e15])
+// the chain is re-summed on q scaled by 2^+-64, which is exact, so that the band still follows |q|: a band collapsed
+// to 1e-37 would let the refine drop the chunk of the true arg-max of a tiny row.  Filter and refine both call this.
+template <int D>
+__device__ __noinline__ float tc_norm_rescaled(const float *__restrict__ q, float s) {
+  float ss = 0.f;
+#pragma unroll
+  for (int k = 0; k < D; ++k) {
+    const float v = __ldg(q + k) * s;
+    ss = fmaf(v, v, ss);
+  }
+  return sqrtf(ss) / s;
+}
+template <int D>
+__device__ __forceinline__ float tc_norm(const float *__restrict__ q, float ss) {
+  return (ss >= 0x1p-100f && ss <= 0x1p100f) ? sqrtf(ss) : tc_norm_rescaled<D>(q, ss < 1.f ? 0x1p64f : 0x1p-64f);
+}
+
 // max of 32 accumulator values; g[0..10] are the maxima of the 3-element groups
 // (g[10] covers elements 30, 31) so the rare slow path can skip whole groups.
 __device__ __forceinline__ float chunk_max(const uint32_t (&v)[32], float (&g)[11]) {
@@ -133,7 +151,8 @@ __device__ __forceinline__ float chunk_max(const uint32_t (&v)[32], float (&g)[1
 //     a~ = sum_k f16(q'_k) f16(w_k) + 1   in (0, 2),   |a~ - (s' + 1)| <= 2^-10 (operands, RN) + 2^-10 (result) = 2^-9.
 // Scaling a row by 2^-e does not move its arg-max, so the filter runs entirely in that scaled, shifted domain with the
 // CONSTANT band 2 * 1.25 * 2^-9; the refine re-scores the surviving chunks with the exact fp32 chain as before.
-// (The scale is 0.99 / (|q| max|w| 1.003), not a power of two: see tc_h_scale.)
+// (The scale is 0.99 / (|q| max|w| 1.003), not a power of two: see tc_h_scale.)  Rows the scale cannot serve get q' = 0
+// instead: every approximate score is then the constant 1, their streams overflow and are scanned exactly.
 constexpr float TC_H_BAND = 2.0f * 1.25f * 0.001953125f;
 constexpr uint32_t TC_IDESC_F16 = (0u << 4) | (0u << 7) | (0u << 10) | ((uint32_t)(TC_BN >> 3) << 17) | ((uint32_t)(TC_BM >> 4) << 24);
 
@@ -172,9 +191,11 @@ __device__ __forceinline__ void chunk_max_u16x2(const uint32_t *v, uint32_t &b0,
 // domain, so relative to |q| it is 1 / (|q'| max|w|) times wider — at 0.5 twice the tf32 filter's, and with it the
 // number of chunks a stream hands over (measured at 10 M items: streams overflowing their four hand-over slots and
 // being re-scanned exactly made the refine 200x slower).
+// ss below 2^-100 (|q| < ~1e-15) may be a subnormal that has lost most of its bits: a scale from it could put
+// |q'| max|w| above 1 and a~ below 0, whose f16 sign bit wins the unsigned maxima.  Such rows get q' = 0 as well.
 __device__ __forceinline__ float tc_h_scale(float ss, float wmax_s) {
   const float t = sqrtf(ss) * wmax_s;
-  if (!(t > 1.0e-30f) || !(t < 1.0e30f)) return 1.f;      // zero / non-finite row: every approximate score is the constant
+  if (!(ss >= 0x1p-100f) || !(t > 1.0e-30f) || !(t < 1.0e30f)) return 0.f;   // zero, tiny, huge or non-finite row: q' = 0
   return 0.99f / t;
 }
 
@@ -221,6 +242,7 @@ __device__ __noinline__ void tc_rescore_overflow(const float *__restrict__ W, in
       best = tc_exact_score<D>(Q + row * D, W + j * D);
       bidx = (int32_t)j;
     }
+    if (!(best > -INFINITY)) { best = -INFINITY; bidx = 0x7fffffff; }   // a NaN never wins (nor poisons the merge)
 #pragma unroll
     for (int o = 16; o > 0; o >>= 1) {
       const float ov = __shfl_xor_sync(0xffffffffu, best, o);
@@ -339,6 +361,7 @@ score_select_tc_kernel(const float *__restrict__ Wsw, const float *__restrict__ 
               ss = fmaf(q0.x, q0.x, ss); ss = fmaf(q0.y, q0.y, ss); ss = fmaf(q0.z, q0.z, ss); ss = fmaf(q0.w, q0.w, ss);
               ss = fmaf(q1.x, q1.x, ss); ss = fmaf(q1.y, q1.y, ss); ss = fmaf(q1.z, q1.z, ss); ss = fmaf(q1.w, q1.w, ss);
               const float sc = tc_h_scale(ss, band_scale);
+              if (sc == 0.f) { q0 = make_float4(0.f, 0.f, 0.f, 0.f); q1 = q0; }   // (inf * 0 would be NaN)
               const __half2 h0 = __floats2half2_rn(q0.x * sc, q0.y * sc), h1 = __floats2half2_rn(q0.z * sc, q0.w * sc);
               const __half2 h2 = __floats2half2_rn(q1.x * sc, q1.y * sc), h3 = __floats2half2_rn(q1.z * sc, q1.w * sc);
               q0 = make_float4(__uint_as_float(*reinterpret_cast<const uint32_t *>(&h0)), __uint_as_float(*reinterpret_cast<const uint32_t *>(&h1)),
@@ -456,9 +479,9 @@ score_select_tc_kernel(const float *__restrict__ Wsw, const float *__restrict__ 
         if constexpr (F16) {
           band = TC_H_BAND;     // constant in the scaled, shifted domain of the approximate scores
         } else {
-          float ss = 0.f;
-          if (live) ss = tc_norm2<D>(Q + row * D);
-          band = band_scale * sqrtf(ss) * 1.0001f + 1e-37f;
+          float nq = 0.f;
+          if (live) nq = tc_norm<D>(Q + row * D, tc_norm2<D>(Q + row * D));
+          band = band_scale * nq * 1.0001f + 1e-37f;
         }
         // running max of the approximate scores; finite start so that masked (-inf) columns
         // never pass, +inf for dummy rows so that nothing ever passes
@@ -730,9 +753,11 @@ tc_refine_kernel(const float *__restrict__ W, int64_t n_rows, int64_t row_offset
   }
   // (f16 filter: the running maxima and the recorded approximate maxima live in the scaled, shifted domain of that
   // filter, where the band is a constant)
-  const float band = band_const > 0.f ? band_const : tc_band_scale(false, __ldg(max_row_norm)) * sqrtf(ss) * 1.0001f + 1e-37f;
+  const float band = band_const > 0.f ? band_const : tc_band_scale(false, __ldg(max_row_norm)) * tc_norm<D>(Q + row * D, ss) * 1.0001f + 1e-37f;
   R = warp_max(R);
   const float thr = R - band;
+  // R = +inf (a score overflowed) or a NaN band: the band says nothing, every stream of the row is scanned exactly
+  const bool exact_row = !(thr < INFINITY);
   float best = -INFINITY;
   int32_t bidx = 0x7fffffff;
   auto score = [&](int64_t j) {
@@ -752,7 +777,7 @@ tc_refine_kernel(const float *__restrict__ W, int64_t n_rows, int64_t row_offset
     if (ch > 0) chunk_geom(ch, Tch, n_units, cfirst, n_streams, sbase);
     for (int base = 0; base < n_streams; base += 32) {
       if (base > 0 || ch > 0) load_group(sbase, n_streams, base, cnt, ents);
-      unsigned flagged = __ballot_sync(0xffffffffu, cnt < 0);
+      unsigned flagged = __ballot_sync(0xffffffffu, (cnt < 0 || exact_row) && base + lane < n_streams);
       while (flagged) {  // exact scan of a flagged stream's whole column range
         const int fs = base + __ffs(flagged) - 1;
         flagged &= flagged - 1;
@@ -794,6 +819,7 @@ tc_refine_kernel(const float *__restrict__ W, int64_t n_rows, int64_t row_offset
       unpack_best(pb, &ov, &oi);
       if (ov > best || (ov == best && oi < bidx)) { best = ov; bidx = oi; }
     }
+    if (bidx == 0x7fffffff) bidx = 0;   // no score above -inf (NaN never wins): the first index, value -inf
     out_idx[row] = (int64_t)bidx + row_offset;
     if (out_val) out_val[row] = best;
   }

@@ -18,7 +18,13 @@ __device__ __forceinline__ int64_t sw32_chunk_index(int64_t j, int a, int c, int
 
 // f16 image of a D = 8 table (the f16 select filter): row j = 16 f16 (8 dimensions, then the constant dimension 1 and
 // zeros) = 32 B, the two 16-byte halves swapped when bit 2 of the row index is set (the same SWIZZLE_32B rule).
+// A row holding a NaN is stored as zeros: an f16 NaN pattern would win the filter's unsigned 16-bit chunk maxima and
+// hide the real winner of its chunk; as zeros its approximate score is the constant 1, and the refine re-scores it.
 __device__ __forceinline__ void h16_store_row(uint4 *__restrict__ out, int64_t j, float4 w0, float4 w1) {
+  if (isnan(w0.x + w0.y + w0.z + w0.w + w1.x + w1.y + w1.z + w1.w)) {   // (inf - inf rows: out of the f16 range anyway)
+    w0 = make_float4(0.f, 0.f, 0.f, 0.f);
+    w1 = w0;
+  }
   const __half2 h0 = __floats2half2_rn(w0.x, w0.y), h1 = __floats2half2_rn(w0.z, w0.w);
   const __half2 h2 = __floats2half2_rn(w1.x, w1.y), h3 = __floats2half2_rn(w1.z, w1.w);
   const uint4 lo = make_uint4(*reinterpret_cast<const uint32_t *>(&h0), *reinterpret_cast<const uint32_t *>(&h1),
